@@ -5,7 +5,8 @@
 // src/functions.cpp / src/Camera.cpp, add include/ of this repo to the include path and link libsva_b200.so.  The signatures
 // are the reference's own (functions.h:22,26,34-38,45; Camera.h:12-13), so src/CameraStereoVision.cpp and the dlibFaceSelect
 // ROI path call them unchanged.  It compiles against real OpenCV (cv::Mat) — and, for this repo's tests, against the minimal
-// stand-in in oracle/cvshim.  No reference source is copied: the headers are included from the reference tree.
+// stand-in in oracle/cvshim.  No reference source is copied: the headers are the reference tree's own, or for this repo's tests
+// the stand-in declarations in adapter/refshim where no reference tree is given.
 //
 // Error behaviour: the reference surfaces failures as cv::Exception; a non-zero sva status is turned back into one.
 // Ownership: every function returns a freshly allocated Mat / vector, inputs are not mutated, no pointer is retained.

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the driver's measurement contract for the multi-camera depth hot path.
 
-  python bench.py --gpus N --steps K --warmup W [--config c1] [--win-half 20] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--config c1] [--win-half 20] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path (K1a AD volume -> K1b box/pack -> 8-path SGM -> WTA/LR/sub-pixel) over one synthetic
 frame per rank.  `value` = whole-job MDE/s with inputs resident in HBM (CUDA events on the library's stream, max over ranks);
@@ -213,6 +213,9 @@ def run_sva(args):
     R.barrier()
     launches = ctx.launches() - l0
     total_ms = R.max(total_ms)
+    if args.dump_outputs and rank == 0:
+        disp, sub = ctx.download_disparity()  # the maps the last timed step left on the device
+        dump_outputs(args.dump_outputs, {"disparity": disp, "subpixel": sub})
     # Per-kernel table: the default schedule runs the second horizontal SGM direction on a second stream NEXT TO the first row-sweeping
     # group (where the launches are not paced), so event times of those launches overlap and say little about each kernel.  The table,
     # the roofline of the dominant kernel and the ncu pairing therefore come from a second pass of the same frames with that one overlap
@@ -436,7 +439,7 @@ def run_c4_strong(args, R):
         for _ in range(3):
             ctx.run(abi.STAGE_ALL)
         ctx.synchronize()
-        steps = 2
+        steps = args.steps
         R.barrier()
         ms = ctx.time(abi.STAGE_ALL, steps * (fe - fb))
         R.barrier()
@@ -461,7 +464,7 @@ def run_c3(args, R, headline=False):
     sc = configs.scene(name, frame=0)
     mde = configs.mde_per_frame(name)
     world, rank = R.world, R.rank
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
     base = {"workload": "c3: " + cfg["desc"], "scaling": "strong", "n_gpus": world, "unit": "MDE/s", "steps": steps,
             "timing": "CUDA events on the library's streams, inputs resident, max over ranks"}
     if world == 1:
@@ -474,6 +477,9 @@ def run_c3(args, R, headline=False):
             l0 = ctx.launches()
             ms = ctx.time(abi.STAGE_ALL, steps) / steps
             launches = ctx.launches() - l0
+            if headline and args.dump_outputs:
+                disp, sub = ctx.download_disparity()  # the maps the last timed step left on the device
+                dump_outputs(args.dump_outputs, {"disparity": disp, "subpixel": sub})
         finally:
             ctx.close()
         res = dict(base, scheme="single GPU: the whole frame, no exchange", latency_ms=round(ms, 3), ms_per_frame=round(ms, 3), frames_per_s=round(1e3 / ms, 2),
@@ -504,11 +510,12 @@ def run_c3(args, R, headline=False):
                 ctxs[0].rows_download()  # checks the hand-off time-outs
             lat /= steps
             launches = (ctxs[0].launches() - l0) // steps
-            # frames back to back with P = 1, 2, 3 frames in flight per GPU (P contexts on one stream): phase 0 of frame f is enqueued before
-            # phase 1 of frame f - P + 1, so a rank spends the wait for the far end of its second sweep on the next frames' first halves
+            # frames back to back (`steps` frames per run) with P = 1, 2, 3 frames in flight per GPU (P contexts on one stream): phase 0 of
+            # frame f is enqueued before phase 1 of frame f - P + 1, so a rank spends the wait for the far end of its second sweep on the next
+            # frames' first halves
             by_in_flight = {}
             for in_flight in range(1, max_in_flight + 1):
-                frames = 12
+                frames = steps
                 use = ctxs[:in_flight]
                 R.barrier()
                 ctxs[0].timer_start()
@@ -523,7 +530,7 @@ def run_c3(args, R, headline=False):
             # three frames in flight in the three-part form (sva_rows_run_part): part 0 of frame f, part 1 of frame f - 1, part 2 of frame f - 2 —
             # every wait for a neighbour's state sits behind a later frame's cost volume, which needs no neighbour
             if max_in_flight >= 3:
-                frames = 12
+                frames = steps
                 use = ctxs[:3]
                 R.barrier()
                 ctxs[0].timer_start()
@@ -543,7 +550,8 @@ def run_c3(args, R, headline=False):
             # by chain position, iteration i of rank r runs the cost volume of frame i, its FIRST sweep of frame i - 1 - min(pd, pu) and its second
             # sweep + K3 of frame i - 1 - max(pd, pu) (pd = r, pu = G - 1 - r: hops from the start of the down / up chain): the state a sweep needs
             # was produced by the neighbour ONE ITERATION EARLIER, so no wait ever blocks.  Needs G + 1 contexts per GPU (frames in flight);
-            # reported as the steady-state slope between a 16- and a 48-frame run and as the 48-frame average (fill and drain included).
+            # reported as the steady-state slope between a `steps`- and a 3 x `steps`-frame run and as the average of the longer run (fill and
+            # drain included).
             skew = None
             try:
                 G = world
@@ -559,7 +567,8 @@ def run_c3(args, R, headline=False):
                 pd, pu = rank, G - 1 - rank
                 lag1, lag2 = 1 + min(pd, pu), 1 + max(pd, pu)
                 t_run = {}
-                for frames in (16, 48):
+                short, long = steps, 3 * steps
+                for frames in (short, long):
                     R.barrier()
                     ctxs[0].timer_start()
                     for i in range(frames + G):
@@ -572,9 +581,10 @@ def run_c3(args, R, headline=False):
                     t_run[frames] = R.max(ctxs[0].timer_stop())
                     for c in ctxs:
                         c.rows_download()
-                skew = {"contexts_per_gpu": P, "ms_per_frame_steady_state": round((t_run[48] - t_run[16]) / 32, 3), "ms_per_frame_48_frames": round(t_run[48] / 48, 3),
+                skew = {"contexts_per_gpu": P, "frames_per_run": [short, long], "ms_per_frame_steady_state": round((t_run[long] - t_run[short]) / (long - short), 3),
+                        "ms_per_frame_long_run": round(t_run[long] / long, 3),
                         "order": "iteration i of rank r: part 0 of frame i, part 1 of frame i - 1 - min(r, G-1-r), part 2 of frame i - 1 - max(r, G-1-r) (sva_rows_run_part)"}
-                by_in_flight["%d (skewed by chain position, 48 frames incl. fill and drain)" % P] = t_run[48] / 48
+                by_in_flight["%d (skewed by chain position, %d frames incl. fill and drain)" % (P, long)] = t_run[long] / long
             except Exception as e:  # noqa: BLE001 — the figures above stand on their own
                 skew = {"error": "%s: %s" % (type(e).__name__, str(e)[:200])}
             R.barrier()
@@ -682,13 +692,15 @@ def run_literal(args, R):
     L.sva_timer_start(hnd)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        improved = step()
     wall = time.perf_counter() - t0
     ms = C.c_float(); L.sva_timer_stop(hnd, C.byref(ms))
     R.barrier()
     clocks = sampler.stop() if sampler else None
     n1 = C.c_uint64(); L.sva_kernel_launches(hnd, C.byref(n1))
     dev_ms, wall_ms = R.max(ms.value), R.max(wall * 1e3)
+    if args.dump_outputs and R.rank == 0:
+        dump_outputs(args.dump_outputs, {"improved": improved})
     ev = literal_evals(w, h, stride=64) / 1e6
     if R.rank == 0:
         peak, peak_src = measured_peak()
@@ -806,6 +818,25 @@ def run_reference(args):
     emit(json.dumps(out))
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every map as <out_dir>/<name>.npy in float32 (u8 / u16 disparities are exact in float32).  Maps of more than
+    DUMP_BYTES in all (c3) keep a fixed sample of rows drawn with seed 0, the same rows of every map, listed in sample_rows.npy."""
+    arrays = {name: np.asarray(a, dtype=np.float32) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        h = next(iter(arrays.values())).shape[0]
+        keep = h * (DUMP_BYTES - 2**20) // total  # 1 MiB left for the row list and the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(h, keep, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 class StdoutToStderr:
     """NCCL / torchrun print banners on fd 1; the contract is ONE JSON line on stdout, so everything else goes to stderr"""
 
@@ -849,7 +880,14 @@ def main():
                          "'pairs' = north_star's pair sharding + NCCL reduce of the AD volume; 'slices' = disparity-slice / direction / row sharding (DESIGN.md §7)")
     ap.add_argument("--no-extras", action="store_true", help="skip the c4-strong and c3 runs that the default line carries as extra keys")
     ap.add_argument("--extras-timeout", type=int, default=420, help="seconds after which the line is printed without the extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the maps rank 0 received in the last timed step as DIR/<name>.npy "
+                                                          "(float32): disparity and subpixel, or improved for --config literal; c3 keeps a seeded sample of "
+                                                          "rows (sample_rows.npy) and is dumped on one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "sva" or (args.config == "c3" and dist_env()[2] > 1)):
+        ap.error("--dump-outputs covers --impl sva, and --config c3 on one GPU")
     args.warmup = max(args.warmup, 3) if args.impl == "sva" else args.warmup
     with StdoutToStderr():
         if args.impl == "reference":

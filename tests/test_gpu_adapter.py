@@ -1,4 +1,5 @@
-"""Drop-in check: adapter/sva_functions.cpp (the reference-side binding, compiled against the reference's OWN headers) driven like
+"""Drop-in check: adapter/sva_functions.cpp (the reference-side binding, compiled against the reference's headers, or the stand-ins in
+adapter/refshim when no reference tree is given) driven like
 the reference's main() — getCameraPairs / Camera / improveWithDisparity / getAbsDiff under their reference names, the loop nest as
 one svaMatchLiteral call — must reproduce what the reference's main() produced (tests/golden/main_*.npz)."""
 import ctypes as C
@@ -15,8 +16,7 @@ SO = os.path.join(ROOT, "adapter", "_build", "libsva_adapter_test.so")
 
 
 def test_adapter_reproduces_reference_driver():
-    if not os.path.exists(SO):
-        pytest.skip("adapter test library not built (needs /root/reference at build time)")
+    assert os.path.exists(SO), "adapter test library not built (__graft_entry__.build() builds it)"
     lib = C.CDLL(SO)
     lib.adapter_last_error.restype = C.c_char_p
     for name in ("main_120x160_s7", "main_100x176_s9"):
@@ -36,8 +36,7 @@ def test_adapter_reproduces_reference_driver():
 
 def test_adapter_depth_consumers():
     """shiftPerspective2 / DepthMapToPoints3D / Points3DToDepthMap / getGroups through the C++ binding == the reference's fixtures"""
-    if not os.path.exists(SO):
-        pytest.skip("adapter test library not built (needs /root/reference at build time)")
+    assert os.path.exists(SO), "adapter test library not built (__graft_entry__.build() builds it)"
     lib = C.CDLL(SO)
     lib.adapter_last_error.restype = C.c_char_p
     lib.adapter_depth_consumers.restype = C.c_longlong
@@ -71,8 +70,7 @@ def adapter_multi_gpu(lib, device, uid, rank, world, p, ref, others):
 
 def test_adapter_reaches_the_multi_gpu_entry_points(oracle):
     """world of one: the same C++ calls a multi-process host makes (tools/check_sharded.py runs them over several GPUs)"""
-    if not os.path.exists(SO):
-        pytest.skip("adapter test library not built (needs /root/reference at build time)")
+    assert os.path.exists(SO), "adapter test library not built (__graft_entry__.build() builds it)"
     from stereovisionarray_b200 import abi
     from stereovisionarray_b200._lib import lib as load
     load()  # maps torch's NCCL before the adapter's library binds one (see _lib._preload_nccl)
