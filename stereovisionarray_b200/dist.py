@@ -288,12 +288,17 @@ def rows_direct_connect(ctx, p, rank, world, group=None):
 def rows_direct_depth(ctx, p, ref, others, mask, rank, world, group=None):
     """One frame through the peer-direct row-block pipeline (sva_rows_*; rows_direct_connect first): the path-line state is stored by the
     neighbour's march kernel straight into this GPU's memory and sequenced by device flags.  Returns (disp, subpix) on rank 0, None elsewhere."""
-    import torch
-    import torch.distributed as dist
-    from . import abi
     ctx.upload(p, ref, others, mask)
     ctx.rows_run()
     d, s = ctx.rows_download()
+    return gather_rows(d, s, p, rank, world, group)
+
+
+def gather_rows(d, s, p, rank, world, group=None):
+    """this rank's block of the maps (DepthContext.rows_download) -> the whole maps (disp, subpix) on rank 0, None elsewhere.  Collective."""
+    import torch
+    import torch.distributed as dist
+    from . import abi
     if world == 1:
         return d, s
     rows_per = row_blocks(p.height, world)[0]
@@ -335,17 +340,40 @@ def rows_skewed_order(rank, world, frames):
     return order
 
 
-def rows_direct_stream(ctxs, rank, world, frames, upload=None):
-    """Drives `frames` frames through world + 1 contexts of this rank (all on ONE stream, each connected with rows_direct_connect) in the
-    skewed order.  upload(ctx, frame) is called before a frame's part 0 where the frames differ; results stay in the contexts (rows_download)."""
+def rows_direct_stream_steps(ctxs, rank, world, frames, upload=None, download=None):
+    """Generator form of rows_direct_stream: each next() enqueues one iteration of rows_skewed_order(rank, world, frames) on this rank, and the
+    next() after the last iteration downloads the frames still in the contexts and stops.  One process per GPU simply exhausts it; a process
+    that plays several ranks advances one generator per rank round-robin, one iteration each, and runs the same code as production.
+
+    upload(ctx, f) is called right before part 0 of frame f.  download(ctx, f) is called exactly once per frame: at the start of the iteration
+    that reuses frame f's context (before upload and part 0 of frame f + world + 1), and for the last min(world + 1, frames) frames after the
+    loop, in frame order.  A download may synchronise the device: in the skewed order every wait enqueued on any rank depends only on work
+    its neighbour enqueued in an EARLIER iteration (the sweep's state one iteration before, the ack of the context's previous frame at least
+    world iterations before), so a host that blocks at the start of iteration i — every rank having enqueued iteration i - 1 — never blocks on
+    work that is not enqueued yet."""
     P = world + 1
     if len(ctxs) < P:
         raise ValueError("the skewed order keeps world + 1 = %d frames in flight: that many contexts per GPU" % P)
     for step in rows_skewed_order(rank, world, frames):
         for part, f in step:
-            if part == 0 and upload is not None:
-                upload(ctxs[f % P], f)
+            if part == 0:
+                if download is not None and f >= P:
+                    download(ctxs[(f - P) % P], f - P)
+                if upload is not None:
+                    upload(ctxs[f % P], f)
             ctxs[f % P].rows_run_part(part)
+        yield
+    if download is not None:
+        for f in range(max(0, frames - P), frames):
+            download(ctxs[f % P], f)
+
+
+def rows_direct_stream(ctxs, rank, world, frames, upload=None, download=None):
+    """Drives `frames` frames through world + 1 contexts of this rank (all on ONE stream, each connected with rows_direct_connect) in the
+    skewed order (rows_direct_stream_steps: where upload(ctx, f) and download(ctx, f) are called).  Without a download hook a frame's maps
+    stay in its context (rows_download) until frame f + world + 1 overwrites them."""
+    for _ in rows_direct_stream_steps(ctxs, rank, world, frames, upload, download):
+        pass
 
 
 def numpy_pack(a_u16):

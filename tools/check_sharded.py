@@ -3,9 +3,11 @@
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/check_sharded.py [--c3] [--time]
 
 Schemes: pairs (C: sva_depth_pair_sharded, NCCL reduce from the library), slices and rows (Python + torch.distributed), rows_direct
-(C: sva_rows_*, peer-direct hand-off over CUDA IPC).  Small frames are checked against a live oracle run; --c3 checks the full
-3840x2160x256 frame against the oracle digests in tests/golden/c3_full_oracle.json (tests/golden/make_c3_hash.py), and --time adds
-device-timed runs of the row pipelines at that size.  Exit code 1 on any mismatch."""
+(C: sva_rows_*, peer-direct hand-off over CUDA IPC), rows_stream (rows_direct over a stream of distinct frames in the order skewed by chain
+position, dist.rows_direct_stream, every frame checked).  Small frames are checked against a live oracle run; --c3 checks the full
+3840x2160x256 frame against the oracle digests in tests/golden/c3_full_oracle.json (tests/golden/make_c3_hash.py) and the stream on c3's
+width, D and pairs at 24 rows per rank (+ the border bands) against a live oracle run, and --time adds device-timed runs of the row pipelines at full size.
+Exit code 1 on any mismatch."""
 import argparse
 import hashlib
 import json
@@ -24,7 +26,7 @@ from stereovisionarray_b200.pipeline import DepthContext  # noqa: E402
 ap = argparse.ArgumentParser()
 ap.add_argument("--c3", action="store_true", help="the full c3 frame against the committed oracle digests")
 ap.add_argument("--time", action="store_true", help="with --c3: device-timed row pipelines")
-ap.add_argument("--schemes", default="pairs,slices,rows,rows_direct,adapter")
+ap.add_argument("--schemes", default="pairs,slices,rows,rows_direct,rows_stream,adapter")
 args = ap.parse_args()
 
 rank, local, world = int(os.environ["RANK"]), int(os.environ["LOCAL_RANK"]), int(os.environ["WORLD_SIZE"])
@@ -111,6 +113,63 @@ def run_schemes(p, sc, tag):
     return out
 
 
+def rows_stream(p, scenes):
+    """the frames `scenes` through rows_direct in the order skewed by chain position (dist.rows_direct_stream): world + 1 contexts on one
+    stream, each its own link; the download hook gathers every frame's rows on rank 0 before its context is reused.  -> [(frame, (disp,
+    subpix))] in download order on rank 0"""
+    P = world + 1
+    ctxs, got = [], []
+    try:
+        for j in range(P):
+            c = DepthContext(local)
+            ctxs.append(c)
+            if j:
+                c.set_stream(ctxs[0].get_stream())
+            sdist.rows_direct_connect(c, p, rank, world)
+        assert scenes[0]["mask"] is None and scenes[1]["mask"] is not None
+        for sc in scenes[:2]:  # every buffer, masked and unmasked, before the stream: a buffer that grew there would synchronise the device
+            for c in ctxs:
+                c.upload(p, sc["ref"], sc["others"], sc["mask"])
+                c.rows_run()
+                c.rows_download()
+
+        def upload(c, f):
+            c.upload(p, scenes[f]["ref"], scenes[f]["others"], scenes[f]["mask"])
+
+        def download(c, f):
+            d, s = c.rows_download()
+            got.append((f, sdist.gather_rows(d, s, p, rank, world)))
+        sdist.rows_direct_stream(ctxs, rank, world, len(scenes), upload, download)
+        dist.barrier()  # nobody unmaps a link a neighbour still writes into
+        for c in reversed(ctxs):  # the borrowers first: ctxs[0] owns the stream
+            c.rows_close()
+    finally:
+        for c in reversed(ctxs):
+            c.close()
+    return got
+
+
+def check_stream(p, scenes, tag):
+    global ok
+    got = rows_stream(p, scenes)
+    if rank != 0:
+        return
+    from oracle.oracle import Oracle
+    if [f for f, _ in got] != list(range(len(scenes))):
+        say("rows_stream %s over %d GPUs vs oracle: MISMATCH (frames downloaded: %s)" % (tag, world, [f for f, _ in got]))
+        ok = False
+    for f, (d, s) in got:
+        d0, s0 = Oracle().depth_from_array(p, scenes[f]["ref"], scenes[f]["others"], scenes[f]["mask"])
+        same = np.array_equal(d, d0) and np.array_equal(s, s0) and bool((d0 != 0xFFFF).any())  # a frame with no valid pixel checks nothing
+        say("rows_stream %s frame %d over %d GPUs vs oracle: %s (valid %.3f)" % (tag, f, world, "bit-exact" if same else "MISMATCH", float((d0 != 0xFFFF).mean())))
+        ok = ok and same
+
+
+def stream_scenes(h, w, D, off):
+    """3 (world + 1) distinct frames — every link of the skewed order carries three — the mask on odd frames"""
+    return [synth.make_scene(h, w, D, off, 7700 + f, face=f % 2 == 1) for f in range(3 * (world + 1))]
+
+
 if not args.c3:
     from oracle.oracle import Oracle  # test infrastructure: the checker
     for (h, w, D, off, k, face) in [(270, 480, 256, OFF15, 20, True), (203, 333, 128, OFF15[:8], 7, True), (131, 3840, 192, OFF15[:3], 4, False)]:
@@ -125,6 +184,8 @@ if not args.c3:
                 same = np.array_equal(o[0], dref) and np.array_equal(o[1], sref)
                 say("%s %dx%dx%d over %d GPUs vs oracle: %s (valid %.3f)" % (name, w, h, D, world, "bit-exact" if same else "MISMATCH", float((d0 != 0xFFFF).mean())))
                 ok = ok and same
+        if "rows_stream" in schemes:
+            check_stream(p, stream_scenes(h, w, D, off), "%dx%dx%d" % (w, h, D))
 else:
     with open(os.path.join(ROOT, "tests", "golden", "c3_full_oracle.json")) as f:
         gold = json.load(f)
@@ -142,6 +203,10 @@ else:
             say("%s c3 3840x2160x256, 15 pairs, %d GPUs vs oracle digests: integer map %s, sub-pixel map %s (valid pixels %d / %d)"
                 % (name, world, "bit-exact" if same_d else "MISMATCH", "bit-exact" if same_s else "MISMATCH", int((o[0] != 0xFFFF).sum()), gold["valid_pixels"]))
             ok = ok and same_d and same_s
+    if "rows_stream" in schemes:  # distinct full-size c3 frames would cost a minute of oracle time each: c3's width, D and pairs at a
+        ps = configs.params("c3")  # height of 24 rows per rank plus the two border bands of win_half rows, which hold no valid pixel
+        ps.height = 24 * world + 2 * ps.win_half
+        check_stream(ps, stream_scenes(ps.height, ps.width, ps.num_disp, configs.offsets("c3")), "c3 3840x%dx256" % ps.height)
     if args.time:
         ctx = DepthContext(local)
         stream = torch.cuda.current_stream()
