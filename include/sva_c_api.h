@@ -86,9 +86,10 @@ typedef enum sva_cost_mode { SVA_COST_SAD = 0, SVA_COST_CENSUS = 1 } sva_cost_mo
 typedef struct sva_ctx sva_ctx;
 
 /* ---- context ----------------------------------------------------------------------------------------------- */
-int sva_create(int device, sva_ctx** out);          /* one ctx per GPU; owns a stream and the HBM workspaces */
+int sva_create(int device, sva_ctx** out);          /* one ctx per GPU; owns a stream and the HBM workspaces.  SVA_ERR_BAD_ARG when an
+                                                        A/B switch (DESIGN §8a) holds a value outside its documented set */
 int sva_destroy(sva_ctx* ctx);
-const char* sva_last_error(const sva_ctx* ctx);      /* valid until the next call on ctx */
+const char* sva_last_error(const sva_ctx* ctx);      /* valid until the next call on ctx; NULL: why this thread's last sva_create failed */
 int sva_api_version(void);
 int sva_set_stream(sva_ctx* ctx, void* cuda_stream); /* run on a caller stream (e.g. torch's; NULL = the legacy default stream); the stream must
                                                        * stay alive until sva_use_own_stream / another sva_set_stream / sva_destroy */

@@ -170,6 +170,9 @@ struct LaunchScope {
 
 static inline int div_up(int a, int b) { return (a + b - 1) / b; }
 
+// an environment switch's value as a whole number in [lo, hi]; false for text, overflow or a value outside (sva_ctx.cu)
+bool sva_parse_env_int(const char* s, long long lo, long long hi, long long* out);
+
 #ifdef __CUDACC__
 // streaming (read-once) global loads: bypass L1 allocation
 __device__ __forceinline__ uint32_t ldg_stream_u32(const void* p) {

@@ -1,6 +1,9 @@
 // sva_ctx.cu — context lifetime, HBM workspaces, event-based kernel timing.
+#include <cerrno>
+#include <climits>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 
 #include "sva_common.cuh"
 
@@ -77,40 +80,80 @@ void sva_ctx::time_begin(const char* name) {
 
 void sva_ctx::time_end() { cudaEventRecord(ktimes.back().end, stream); }
 
+// why the last sva_create of this thread failed (sva_last_error(NULL))
+static thread_local std::string create_err;
+
+// A whole number in [lo, hi] (surrounding blanks allowed), or false: atoi would read a typo as 0 and run another variant without a word.
+bool sva_parse_env_int(const char* s, long long lo, long long hi, long long* out) {
+    if (!s) return false;
+    errno = 0;
+    char* end = nullptr;
+    const long long v = strtoll(s, &end, 10);
+    if (end == s || errno == ERANGE) return false;
+    while (*end == ' ' || *end == '\t') end++;
+    if (*end != '\0' || v < lo || v > hi) return false;
+    *out = v;
+    return true;
+}
+
+// One A/B switch of DESIGN §8a: unset keeps the default; a value outside [lo, hi], or equal to hole, is refused.
+static bool read_switch(const char* name, int& field, int lo, int hi, const char* allowed, int hole = INT_MIN) {
+    const char* e = getenv(name);
+    if (!e) return true;
+    long long v = 0;
+    if (!sva_parse_env_int(e, lo, hi, &v) || v == hole) {
+        create_err = std::string(name) + "=" + e + " is not valid (allowed: " + allowed + ")";
+        return false;
+    }
+    field = (int)v;
+    return true;
+}
+
+static bool read_switches(sva_ctx* c) {
+    bool ok = read_switch("SVA_SGM_SPLIT", c->tune_sgm_split, 0, 1, "0, 1")
+           && read_switch("SVA_SGM_PACE", c->tune_sgm_pace, -1, 1, "-1, 0, 1")
+           && read_switch("SVA_SGM_PACE_WINDOW", c->tune_sgm_pace_window, 1, 1 << 20, "1 or more")
+           && read_switch("SVA_SGM_HSTORE", c->tune_sgm_hstore, 0, 3, "0, 1, 2, 3")
+           && read_switch("SVA_SGM_BULK", c->tune_sgm_bulk, 0, 2, "0, 1, 2")
+           && read_switch("SVA_SGM_DIAG_SPLIT", c->tune_sgm_diag_split, 0, 2, "0, 1, 2")
+           && read_switch("SVA_STREAM_AD_AHEAD", c->tune_stream_ad_ahead, 0, 2, "0, 1, 2")
+           && read_switch("SVA_PREZERO", c->tune_prezero, 0, 1, "0, 1")
+           && read_switch("SVA_WTA_SEG", c->tune_wta_seg, -1, 1 << 16, "-1, 0, or a segment length up to 65536")
+           && read_switch("SVA_AD_GATHER", c->tune_ad_gather, 0, 1, "0, 1")
+           && read_switch("SVA_AD_SET", c->tune_ad_set, 0, 1, "0, 1")
+           && read_switch("SVA_AD_TH", c->tune_ad_th, 0, 1 << 16, "0, or rows per tile up to 65536")
+           && read_switch("SVA_BOX_SHFL", c->tune_box_shfl, 0, 1, "0, 1")
+           && read_switch("SVA_BOX_L2", c->tune_box_l2, 0, 1, "0, 1")
+           && read_switch("SVA_BOX_BANDS", c->tune_box_bands, 0, 1 << 20, "0, or a band count")
+           && read_switch("SVA_BOX_OCC", c->tune_box_occ, 0, 3, "0, 2, 3", 1);  // K1b exists for 2 and 3 CTAs per SM
+    // read where the SGM launches are planned (k_sgm.cu), by presence; "1" is the one documented value, anything else is a mistake
+    for (const char* name : {"SVA_SGM_NO_BLK", "SVA_SGM_NO_RANGED", "SVA_SGM_NO_COLSPLIT"}) {
+        const char* e = getenv(name);
+        if (ok && e && strcmp(e, "1") != 0) { create_err = std::string(name) + "=" + e + " is not valid (allowed: 1, or unset)"; ok = false; }
+    }
+    return ok;
+}
+
 extern "C" {
 
 int sva_api_version(void) { return SVA_API_VERSION; }
 
 int sva_create(int device, sva_ctx** out) {
+    create_err.clear();
     if (!out) return SVA_ERR_BAD_ARG;
     *out = nullptr;
     int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0 || device < 0 || device >= n) return SVA_ERR_NO_DEVICE;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0 || device < 0 || device >= n) { create_err = "no such CUDA device"; return SVA_ERR_NO_DEVICE; }
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return SVA_ERR_CUDA;
-    if (prop.major != 10) return SVA_ERR_NO_DEVICE;  // built for sm_100a only; there is no fallback path
-    if (cudaSetDevice(device) != cudaSuccess) return SVA_ERR_CUDA;
+    if (prop.major != 10) { create_err = "not an sm_100 GPU"; return SVA_ERR_NO_DEVICE; }  // built for sm_100a only; there is no fallback path
     sva_ctx* c = new sva_ctx();
+    if (!read_switches(c)) { delete c; return SVA_ERR_BAD_ARG; }
+    if (cudaSetDevice(device) != cudaSuccess) { delete c; return SVA_ERR_CUDA; }
     c->device = device;
     c->sm_count = prop.multiProcessorCount;
     if (cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return SVA_ERR_CUDA; }
     c->stream = c->own_stream;
-    if (const char* e = getenv("SVA_SGM_SPLIT")) c->tune_sgm_split = atoi(e);
-    if (const char* e = getenv("SVA_SGM_PACE")) c->tune_sgm_pace = atoi(e);
-    if (const char* e = getenv("SVA_SGM_HSTORE")) c->tune_sgm_hstore = atoi(e);
-    if (const char* e = getenv("SVA_STREAM_AD_AHEAD")) c->tune_stream_ad_ahead = atoi(e);
-    if (const char* e = getenv("SVA_SGM_BULK")) c->tune_sgm_bulk = atoi(e);
-    if (const char* e = getenv("SVA_PREZERO")) c->tune_prezero = atoi(e);
-    if (const char* e = getenv("SVA_SGM_DIAG_SPLIT")) c->tune_sgm_diag_split = atoi(e);
-    if (const char* e = getenv("SVA_WTA_SEG")) c->tune_wta_seg = atoi(e);
-    if (const char* e = getenv("SVA_AD_GATHER")) c->tune_ad_gather = atoi(e);
-    if (const char* e = getenv("SVA_AD_TH")) c->tune_ad_th = atoi(e);
-    if (const char* e = getenv("SVA_BOX_SHFL")) c->tune_box_shfl = atoi(e);
-    if (const char* e = getenv("SVA_BOX_L2")) c->tune_box_l2 = atoi(e);
-    if (const char* e = getenv("SVA_BOX_BANDS")) c->tune_box_bands = atoi(e);
-    if (const char* e = getenv("SVA_BOX_OCC")) c->tune_box_occ = atoi(e);
-    if (const char* e = getenv("SVA_AD_SET")) c->tune_ad_set = atoi(e);
-    if (const char* e = getenv("SVA_SGM_PACE_WINDOW")) c->tune_sgm_pace_window = atoi(e);
     *out = c;
     return SVA_OK;
 }
@@ -142,7 +185,7 @@ int sva_destroy(sva_ctx* c) {
     return SVA_OK;
 }
 
-const char* sva_last_error(const sva_ctx* c) { return c ? c->err.c_str() : "null context"; }
+const char* sva_last_error(const sva_ctx* c) { return c ? c->err.c_str() : !create_err.empty() ? create_err.c_str() : "null context"; }
 
 int sva_set_stream(sva_ctx* c, void* s) {  // NULL = the legacy default stream (what torch.cuda.current_stream() usually is)
     if (!c) return SVA_ERR_BAD_ARG;

@@ -232,13 +232,17 @@ int sva_rows_open(sva_ctx* c, const sva_params* p, int32_t rank, int32_t world) 
     if (p->n_paths != 8) return c->fail(SVA_ERR_BAD_ARG, "rows_open: the row-block pipeline aggregates 8 paths");
     const int rows_per = (p->height + world - 1) / world;
     if ((long long)rows_per * (world - 1) >= p->height) return c->fail(SVA_ERR_BAD_ARG, "rows_open: fewer image rows than the ranks need (every rank owns at least one row)");
+    long long timeout_ms = 0;
+    const char* te = getenv("SVA_ROWS_TIMEOUT_MS");
+    if (te && !sva_parse_env_int(te, 1, 1LL << 40, &timeout_ms))  // 0 or text would be a time-out that fires at once
+        return c->fail(SVA_ERR_BAD_ARG, std::string("rows_open: SVA_ROWS_TIMEOUT_MS=") + te + " is not valid (allowed: milliseconds, 1 or more)");
     SVA_TRY(sva_rows_close(c));
     SVA_CUDA_OK(c, cudaSetDevice(c->device));
     RowsLink* l = new RowsLink();
     l->rank = rank; l->world = world; l->W = p->width; l->H = p->height; l->D = p->num_disp;
     l->y0 = rank * rows_per; l->rows = std::min(p->height, (rank + 1) * rows_per) - l->y0;
     l->state_bytes = (((size_t)3 * p->width * p->num_disp * sizeof(uint16_t)) + 255) & ~(size_t)255;
-    if (const char* e = getenv("SVA_ROWS_TIMEOUT_MS")) l->timeout_ns = atoll(e) * 1000000LL;
+    if (te) l->timeout_ns = timeout_ms * 1000000LL;
     const size_t bytes = FLAGS_BYTES + 2 * l->state_bytes;
     cudaError_t e = cudaMalloc(&l->mem, bytes);
     if (e != cudaSuccess) { delete l; return c->fail(SVA_ERR_NOMEM, std::string("rows_open: cudaMalloc: ") + cudaGetErrorString(e)); }

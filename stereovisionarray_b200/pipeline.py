@@ -7,7 +7,7 @@ import ctypes as C
 import numpy as np
 
 from . import abi
-from ._lib import check, lib
+from ._lib import SvaError, check, lib
 
 
 def _p(a, t):
@@ -19,6 +19,8 @@ class DepthContext:
         self._L = lib()
         h = C.c_void_p()
         rc = self._L.sva_create(device, C.byref(h))
+        if rc == abi.SVA_ERR_BAD_ARG:  # an A/B switch (DESIGN §8a) outside its documented set
+            raise SvaError(rc, "sva_create: " + self._L.sva_last_error(None).decode())
         if rc != 0:
             raise RuntimeError("sva_create(device=%d) failed with %d — a B200 (sm_100) GPU is required; there is no CPU fallback" % (device, rc))
         self._h = h

@@ -19,6 +19,9 @@ WIDE = [
     # c3-wide rows: three directions x 3840 lines exceed one resident wave, so each row-sweeping group runs as ranged launches
     (48, 3840, 256, [(-1, 0), (1, 1)], dict(win_half=4, n_paths=8, lr_gx=-1)),
     (40, 3840, 192, [(-1, 0), (0, -1)], dict(win_half=3, n_paths=8, lr_gx=1)),
+    # more rows than one block of W / 16 = 240: each row-sweeping group is marched in two row blocks (240 + 20 rows, run_group_in_blocks),
+    # the path-line state handed across the boundary, each block cut by columns into its own set of ranged launches
+    (260, 3840, 64, [(-1, 0), (1, 0), (0, 1)], dict(win_half=4, n_paths=8, lr_gx=-1)),
 ]
 
 

@@ -199,12 +199,21 @@ def test_bad_arguments_fail_loudly(ctx):
     assert disp.shape == (32, 40)
 
 
-@pytest.mark.parametrize("h,w,D,blocks", [(67, 96, 64, [(0, 20), (20, 47), (47, 67)]), (90, 140, 128, [(0, 9), (9, 10), (10, 55), (55, 90)]),
-                                           (64, 70, 256, [(0, 33), (33, 64)]), (58, 3840, 192, [(0, 30), (30, 58)])])
+ROW_BLOCKS = [(67, 96, 64, [(0, 20), (20, 47), (47, 67)]), (90, 140, 128, [(0, 9), (9, 10), (10, 55), (55, 90)]),
+              (64, 70, 256, [(0, 33), (33, 64)]), (58, 3840, 192, [(0, 30), (30, 58)])]
+
+
+@pytest.mark.parametrize("h,w,D,blocks", ROW_BLOCKS)
 def test_row_block_pipeline_emulated_on_one_gpu(ctx, h, w, D, blocks):
     """the row-block scheme's building blocks (sva_frame_rows_begin / sva_frame_sgm_rows / sva_frame_wta_rows with the path-line state
     handed from block to block) reproduce the whole-frame aggregation and maps bit for bit; blocks as small as one row, diagonals that
     wrap at a block boundary, rows wide enough for ranged launches"""
+    check_row_block_pipeline(ctx, h, w, D, blocks)
+
+
+def check_row_block_pipeline(ctx, h, w, D, blocks, oracle=None):
+    """the row-block pipeline on a second, guarded context against the whole-frame run on ctx (and, given the oracle, that run against
+    the oracle: cost volume, aggregation and maps); test_gpu_switches runs it under the A/B switches"""
     import torch
     sc = synth.make_scene(h, w, D, OFF8[:3] if w > 1000 else OFF8, 900 + D, face=True)
     offs = OFF8[:3] if w > 1000 else OFF8
@@ -217,6 +226,12 @@ def test_row_block_pipeline_emulated_on_one_gpu(ctx, h, w, D, blocks):
     S_full = ctx.download_sgm()
     d_full, s_full = ctx.download_disparity()
     C_full = ctx.download_cost()
+    if oracle is not None:
+        C_o = oracle.box_cost(p, oracle.ad_volume(p, sc["ref"], sc["others"]))
+        S_o = oracle.sgm_aggregate(p, C_o)
+        d_o, s_o = oracle.wta(p, S_o, sc["mask"])
+        assert np.array_equal(C_full, C_o) and np.array_equal(S_full, S_o), "whole frame: cost volume / aggregation"
+        assert np.array_equal(d_full, d_o) and np.array_equal(s_full, s_o), "whole frame: maps"
     state = [torch.empty(3 * w * D, dtype=torch.int16, device="cuda") for _ in range(2)]
     torch.cuda.synchronize()
     # the cost volume block by block on a second, poisoned context (bottom block first: a block must not lean on its neighbours' rows)
