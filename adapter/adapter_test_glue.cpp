@@ -8,6 +8,7 @@
 #include "dlibFaceSelect.h"
 
 #include "sva_c_api.h"
+#include "sva_rows_stream.h"
 
 cv::Mat svaMatchLiteral(std::vector<cv::Mat>&, std::vector<Camera>&, std::vector<std::array<int, 2>>&, cv::Mat&, int, double, double);
 void svaSelectDevice(int device);
@@ -98,6 +99,35 @@ extern "C" int adapter_multi_gpu(int device, const uint8_t* id128, int rank, int
         std::vector<uint16_t> dr = svaDepthRowsSharded(*p, r, o, nullptr, rank, world, out_y0, out_rows, &sub);
         std::memcpy(out_rows_disp, dr.data(), dr.size() * 2);
         std::memcpy(out_rows_sub, sub.data(), sub.size() * 4);
+        return 0;
+    } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
+// a C++ host streaming frames through the row-block pipeline (SvaRowsStream) as rank `rank` of `world`: n frames, frame f = refs[f], the
+// n_pairs views others[f * n_pairs ...] and masks[f] (null: no mask); this rank's rows of frame f land at out_disp / out_sub + f * rows * width.
+// All frames are submitted, then flushed and waited for in reverse order.
+extern "C" int adapter_rows_stream(int device, const uint8_t* id128, int rank, int world, const sva_params* p, int n, const uint8_t* const* refs,
+                                   const uint8_t* const* others, const uint8_t* const* masks, uint16_t* out_disp, float* out_sub, int* out_y0, int* out_rows) {
+    try {
+        const int w = p->width, h = p->height;
+        auto mat = [&](const uint8_t* src) { cv::Mat m(h, w, CV_8UC1); std::memcpy(m.data, src, (size_t)w * h); return m; };
+        std::array<uint8_t, SVA_COMM_ID_BYTES> id{};
+        if (id128) std::memcpy(id.data(), id128, id.size());
+        SvaRowsStream s(device, *p, rank, world, id128 ? &id : nullptr);
+        std::vector<cv::Mat> ref, msk;
+        std::vector<std::vector<cv::Mat>> oth(n);
+        for (int f = 0; f < n; f++) {
+            ref.push_back(mat(refs[f]));
+            msk.push_back(masks[f] ? mat(masks[f]) : cv::Mat());
+            for (int i = 0; i < p->n_pairs; i++) oth[f].push_back(mat(others[(size_t)f * p->n_pairs + i]));
+        }
+        const size_t px = (size_t)s.rows() * w;
+        std::vector<int64_t> tickets;
+        for (int f = 0; f < n; f++) tickets.push_back(s.submit(ref[f], oth[f], masks[f] ? &msk[f] : nullptr, out_disp + f * px, out_sub + f * px));
+        s.flush();
+        for (int f = n - 1; f >= 0; f--) s.wait(tickets[f]);
+        *out_y0 = s.y0();
+        *out_rows = s.rows();
         return 0;
     } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }

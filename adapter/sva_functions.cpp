@@ -18,6 +18,7 @@
 #include "functions.h"
 #include "dlibFaceSelect.h"
 #include "sva_c_api.h"
+#include "sva_rows_stream.h"
 
 namespace {
 
@@ -215,3 +216,64 @@ std::vector<uint16_t> svaDepthRowsSharded(const sva_params& p, cv::Mat& ref, std
     if (subpix) *subpix = sub;
     return disp;
 }
+
+// ---- a stream of frames through the row-block pipeline in the order skewed by chain position (sva_rows_stream_*): one call per frame ----
+namespace {
+void check_ctx(sva_ctx* c, int rc, const char* what) {
+    if (rc < 0) throw cv::Exception(std::string(what) + ": " + sva_last_error(c));
+}
+}  // namespace
+
+SvaRowsStream::SvaRowsStream(int device, const sva_params& p, int rank, int world, const std::array<uint8_t, SVA_COMM_ID_BYTES>* comm_id) {
+    try {
+        for (int j = 0; j <= world; j++) {
+            sva_ctx* c = nullptr;
+            const int rc = sva_create(device, &c);
+            if (rc != SVA_OK) throw cv::Exception(std::string("sva_create failed (status ") + std::to_string(rc) + "): " + sva_last_error(nullptr));
+            ctxs_.push_back(c);
+            if (j) {  // one stream for all of them: frames interleave by enqueue order, never as concurrent kernels
+                void* s = nullptr;
+                check_ctx(ctxs_[0], sva_get_stream(ctxs_[0], &s), "sva_get_stream");
+                check_ctx(c, sva_set_stream(c, s), "sva_set_stream");
+            }
+            check_ctx(c, sva_rows_open(c, &p, rank, world), "sva_rows_open");
+        }
+        if (world > 1) {
+            if (!comm_id) throw cv::Exception("SvaRowsStream: several ranks need the communicator id of svaCommUniqueId");
+            check_ctx(ctxs_[0], sva_comm_init(ctxs_[0], comm_id->data(), rank, world), "sva_comm_init");
+        }
+        check_ctx(ctxs_[0], sva_rows_stream_create(ctxs_.data(), (int32_t)ctxs_.size(), &p, &stream_), "sva_rows_stream_create");
+        check_ctx(ctxs_[0], sva_rows_stream_connect_comm(stream_), "sva_rows_stream_connect_comm");
+        int32_t y0 = 0, rows = 0;
+        check_ctx(ctxs_[0], sva_rows_block(ctxs_[0], &y0, &rows), "sva_rows_block");
+        y0_ = y0; rows_ = rows;
+    } catch (...) {
+        release();
+        throw;
+    }
+}
+
+SvaRowsStream::~SvaRowsStream() {
+    if (stream_) sva_rows_stream_flush(stream_);  // the neighbours' frames wait for this rank's parts of them
+    release();
+}
+
+void SvaRowsStream::release() {
+    if (stream_) sva_rows_stream_destroy(stream_);
+    stream_ = nullptr;
+    for (auto it = ctxs_.rbegin(); it != ctxs_.rend(); ++it) sva_destroy(*it);  // the borrowers first: ctxs_[0] owns the stream
+    ctxs_.clear();
+}
+
+int64_t SvaRowsStream::submit(const cv::Mat& ref, const std::vector<cv::Mat>& others, const cv::Mat* mask, uint16_t* disp_rows, float* subpix_rows) {
+    std::vector<sva_image_u8> o;
+    for (auto& m : others) o.push_back(view(m));
+    sva_image_u8 r = view(ref), mk = mask ? view(*mask) : sva_image_u8{};
+    int64_t ticket = -1;
+    check_ctx(ctxs_[0], sva_rows_stream_submit(stream_, &r, o.data(), mask ? &mk : nullptr, disp_rows, subpix_rows, &ticket), "sva_rows_stream_submit");
+    return ticket;
+}
+
+void SvaRowsStream::flush() { check_ctx(ctxs_[0], sva_rows_stream_flush(stream_), "sva_rows_stream_flush"); }
+
+void SvaRowsStream::wait(int64_t ticket) { check_ctx(ctxs_[0], sva_rows_stream_wait(stream_, ticket), "sva_rows_stream_wait"); }

@@ -300,6 +300,41 @@ int sva_rows_close(sva_ctx* ctx);
 int sva_depth_rows_sharded(sva_ctx* ctx, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
                            uint16_t* out_disp_rows, float* out_subpix_rows);
 
+/* ---- a STREAM of frames through the row-block pipeline, one call per frame and rank (DESIGN.md §7) --------------------------------------
+ * The order skewed by chain position behind one call.  The stream borrows world + 1 contexts of this rank: each has been through
+ * sva_rows_open(p, rank, world) with the same rank, world and geometry, all run on ONE stream (sva_get_stream), and context j of every rank forms
+ * one chain.  Their links are connected before the first submit: with sva_rows_connect / sva_rows_connect_local before or after create, or with
+ * sva_rows_stream_connect_comm (collective: one all-gather of all world + 1 handles per rank over ctxs[0]'s communicator; nothing to do for a
+ * world of one).  Errors are reported through sva_last_error(ctxs[0]); a refused call enqueues nothing.  The stream does not own the contexts:
+ * flush, wait and destroy it before them.
+ *
+ * Submit number i (its ticket) is iteration i of the skewed order: part 0 of frame i, part 1 of frame i - 1 - min(r, G-1-r) and part 2 of frame
+ * i - 1 - max(r, G-1-r) (sva_rows_run_part), frame f on context f mod (world + 1).  flush enqueues the remaining iterations, after which every
+ * submitted frame completes; a submit after a flush starts a new fill, tickets continuing.  Every rank makes the same sequence of submit and
+ * flush calls.
+ *
+ * The images are uploaded on a copy stream of the object once the cost volume of the context's previous frame has read its own, the mask once
+ * that frame's K3 has; the block's rows come back on a second copy stream, through pinned staging owned by the object: a ring of world + 2
+ * slots, one per ticket.  The maps reach out_disp_rows / out_subpix_rows (rows x width of sva_rows_block;
+ * out_subpix_rows may be NULL) in sva_rows_stream_wait(ticket) or when the ticket's slot is reused, whichever comes first: the ticket is then
+ * retired, and until then the caller's input images and output buffers must stay valid and untouched.
+ * With pinned inputs, submit never waits for device work of the current or the previous iteration: it waits only when it reuses a slot, for
+ * the download of a frame at least two iterations old.  With pageable inputs cudaMemcpy2DAsync may hold the host until the context's previous
+ * frame has finished — safe in the skewed order, but the upload then no longer overlaps the iteration: pin the images for real overlap.
+ * Nothing is allocated on the device after create (which warms every context up for the geometry, masked and unmasked).
+ *
+ * sva_rows_stream_wait: SVA_ERR_STATE while the ticket's last part is not enqueued yet (submit more frames, or flush); SVA_ERR_COMM if a
+ * hand-off of the frame's context timed out (SVA_ROWS_TIMEOUT_MS) up to that frame — the maps are then not valid; SVA_ERR_BAD_ARG for a ticket
+ * never issued.  A retired ticket returns at once. */
+typedef struct sva_rows_stream sva_rows_stream;
+int sva_rows_stream_create(sva_ctx* const* ctxs, int32_t n_ctxs, const sva_params* p, sva_rows_stream** out);
+int sva_rows_stream_connect_comm(sva_rows_stream* s);
+int sva_rows_stream_submit(sva_rows_stream* s, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
+                           uint16_t* out_disp_rows, float* out_subpix_rows, int64_t* out_ticket);
+int sva_rows_stream_flush(sva_rows_stream* s);
+int sva_rows_stream_wait(sva_rows_stream* s, int64_t ticket);
+int sva_rows_stream_destroy(sva_rows_stream* s);  /* waits for the work in flight; tickets not yet retired are dropped */
+
 #ifdef __cplusplus
 }
 #endif

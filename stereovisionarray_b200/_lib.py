@@ -26,6 +26,8 @@ EXPORTS = [
     "sva_comm_get_unique_id", "sva_comm_init", "sva_comm_destroy", "sva_comm_barrier", "sva_frame_reduce_ad", "sva_depth_pair_sharded",
     "sva_rows_open", "sva_rows_export", "sva_rows_connect", "sva_rows_connect_comm", "sva_rows_connect_local", "sva_rows_block", "sva_rows_run", "sva_rows_run_phase", "sva_rows_run_part", "sva_get_stream",
     "sva_rows_download", "sva_rows_close", "sva_depth_rows_sharded",
+    "sva_rows_stream_create", "sva_rows_stream_connect_comm", "sva_rows_stream_submit", "sva_rows_stream_flush", "sva_rows_stream_wait",
+    "sva_rows_stream_destroy",
 ]
 
 _lib = None
@@ -67,6 +69,11 @@ def lib():
         L.sva_rows_connect.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         for n in ("sva_rows_open", "sva_comm_init"):
             getattr(L, n).argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]
+        L.sva_rows_stream_create.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.POINTER(C.c_void_p)]
+        L.sva_rows_stream_submit.argtypes = [C.c_void_p] * 7
+        L.sva_rows_stream_wait.argtypes = [C.c_void_p, C.c_int64]
+        for n in ("sva_rows_stream_connect_comm", "sva_rows_stream_flush", "sva_rows_stream_destroy"):
+            getattr(L, n).argtypes = [C.c_void_p]
         missing = [n for n in EXPORTS if not hasattr(L, n)]
         if missing:
             raise ImportError("libsva_b200.so does not export %s — rebuild it" % missing)

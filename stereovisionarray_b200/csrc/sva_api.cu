@@ -61,7 +61,8 @@ static void merge_rows(int& a0, int& a1, int b0, int b1) {
     a0 = std::min(a0, b0); a1 = std::max(a1, b1);
 }
 
-static int check_frame_args(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask) {
+// (also used by sva_rows_stream_submit, sva_dist.cu: a frame is refused before anything of it is enqueued)
+int check_frame_args(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask) {
     SVA_TRY(check_params(c, p));
     const int W = p->width, H = p->height;
     SVA_TRY(check_image(c, ref, W, H, "ref"));

@@ -457,3 +457,285 @@ int sva_depth_rows_sharded(sva_ctx* c, const sva_params* p, const sva_image_u8* 
 }
 
 }  // extern "C"
+
+// ---- a stream of frames in the order skewed by chain position (sva_rows_stream_*) ------------------------------------------------------
+// Iteration i of rank r enqueues part 0 of frame i, part 1 of frame i - lag1 and part 2 of frame i - lag2 (lag1 = 1 + min(r, G-1-r),
+// lag2 = 1 + max(r, G-1-r) <= G), frame f on context f mod (G + 1) — dist.rows_skewed_order.  Every wait for a neighbour then depends on work
+// the neighbour enqueued in an EARLIER iteration, so a host that blocks only on work at least two iterations old never blocks on work that is
+// not enqueued yet, and the device never runs dry while the host enqueues.
+//
+// Three streams per rank: the contexts' compute stream, an upload stream and a download stream.  Per context:
+//   images of frame f      uploaded after part 0 of the context's previous frame (K1a is their last reader);
+//   mask of frame f        uploaded after part 2 of the context's previous frame (K3 is its only reader);
+//   part 0 of frame f      waits for the images, part 2 of frame f for the mask.  (Ranks 0 and G-1 run the previous frame's part 2 at the end
+//                          of the iteration just before the context is reused: an upload behind it would stall part 0 for the whole copy —
+//                          measured at c3 on one B200, 19.6 -> 22.4 ms per frame.)
+//   download of frame f    waits for part 2 of frame f, and copies the time-out flag with the rows;
+//   part 2 of frame f + P  waits for that download — not part 0 or 1, for the same reason.
+int check_frame_args(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask);
+
+struct sva_rows_stream {
+    struct Slot {
+        int64_t ticket = -1;
+        bool retired = true;
+        uint16_t* disp = nullptr;  // the caller's buffers of that ticket
+        float* sub = nullptr;
+    };
+    std::vector<sva_ctx*> ctxs;            // borrowed; context j is link j of the chain
+    std::vector<RowsLink*> links;          // the links the stream was created for (a context re-opened since is refused)
+    sva_params p{};
+    int rank = 0, world = 1, P = 2, lag1 = 1, lag2 = 1;
+    size_t disp_bytes = 0, sub_bytes = 0;  // the block's rows of each map (the caller's buffers)
+    size_t sub_at = 0, err_at = 0, slot_bytes = 0;  // layout of a staging slot
+    cudaStream_t compute = nullptr, h2d = nullptr, d2h = nullptr;
+    std::vector<cudaEvent_t> ev_img, ev_mask, ev_p0, ev_p2, ev_out;  // per context: images / mask uploaded, part 0 / part 2 done, download done
+    std::vector<cudaEvent_t> ev_slot;               // per slot: the ticket's rows and flag are in the staging
+    uint8_t* staging = nullptr;                     // pinned, per slot: [disp rows][subpix rows][time-out flag]
+    std::vector<Slot> slots;                        // world + 2: a slot is reused by the ticket world + 2 later, whose part 2 is <= 2 iterations old
+    int64_t next = 0;      // next ticket
+    int64_t fill = 0;      // first ticket since the last flush
+    int64_t finished = 0;  // tickets below this have part 2 and the download enqueued
+    std::set<int64_t> failed;  // retired tickets whose context reported a hand-off time-out
+    int fail(int code, const std::string& msg) { return ctxs[0]->fail(code, "rows_stream: " + msg); }
+    int fwd(int j, int rc) {  // an error of context j, reported through ctxs[0]
+        if (rc != SVA_OK && j != 0) ctxs[0]->err = "rows_stream (context " + std::to_string(j) + "): " + ctxs[j]->err;
+        return rc;
+    }
+};
+
+#define SVA_STREAM_CUDA_OK(s, expr)                                                                           \
+    do {                                                                                                      \
+        cudaError_t e__ = (expr);                                                                             \
+        if (e__ != cudaSuccess) return (s)->fail(SVA_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(e__)); \
+    } while (0)
+
+static void rows_stream_release(sva_rows_stream* s) {
+    for (cudaStream_t st : {s->h2d, s->d2h})
+        if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }
+    for (auto* v : {&s->ev_img, &s->ev_mask, &s->ev_p0, &s->ev_p2, &s->ev_out, &s->ev_slot})
+        for (cudaEvent_t e : *v) if (e) cudaEventDestroy(e);
+    if (s->staging) cudaFreeHost(s->staging);
+    delete s;
+}
+
+// one context through the local stages of its block, so that every device buffer a frame of this geometry needs exists before the stream
+// runs: an allocation inside submit would synchronise the device (a stall, and in a process that plays several ranks a dead-lock)
+static int rows_stream_warm_up(sva_rows_stream* s, int j, const std::vector<uint8_t>& zeros) {
+    sva_ctx* c = s->ctxs[j];
+    RowsLink* l = s->links[j];
+    const sva_image_u8 img{zeros.data(), s->p.height, s->p.width, (size_t)s->p.width};
+    std::vector<sva_image_u8> others(s->p.n_pairs, img);
+    for (const sva_image_u8* mask : {&img, (const sva_image_u8*)nullptr}) {
+        SVA_TRY(sva_frame_upload(c, &s->p, &img, others.data(), mask));
+        SVA_TRY(sva_frame_rows_begin(c, l->y0, l->rows));
+        SVA_TRY(sva_frame_run(c, SVA_STAGE_AD));
+        SVA_TRY(sva_frame_run(c, SVA_STAGE_BOX));
+        SVA_TRY(sva_frame_sgm_rows(c, 2, l->y0, l->rows, nullptr, nullptr));
+        // both sweeps, reading this link's own state buffers and storing nowhere: the paced launches size their pacing buffer here
+        SVA_TRY(sva_frame_sgm_rows(c, 0, l->y0, l->rows, l->d_in(l->mem), nullptr));
+        SVA_TRY(sva_frame_sgm_rows(c, 1, l->y0, l->rows, l->u_in(l->mem), nullptr));
+        SVA_TRY(sva_frame_wta_rows(c, nullptr, l->y0, l->rows));
+    }
+    SVA_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+    return SVA_OK;
+}
+
+// copies a ticket's rows from the staging into the caller's buffers once its download is done
+static int rows_stream_retire(sva_rows_stream* s, int k) {
+    sva_rows_stream::Slot& sl = s->slots[k];
+    SVA_STREAM_CUDA_OK(s, cudaEventSynchronize(s->ev_slot[k]));
+    const uint8_t* st = s->staging + (size_t)k * s->slot_bytes;
+    memcpy(sl.disp, st, s->disp_bytes);
+    if (sl.sub) memcpy(sl.sub, st + s->sub_at, s->sub_bytes);
+    uint32_t err = 0;
+    memcpy(&err, st + s->err_at, sizeof err);
+    if (err) s->failed.insert(sl.ticket);
+    sl.retired = true;
+    return SVA_OK;
+}
+
+// one iteration of the skewed order: part 0 of frame i when `with_part0` (its upload already enqueued by the caller), then part 1 / part 2 of
+// the frames the lags select among the frames of the current fill, [fill, last)
+static int rows_stream_iteration(sva_rows_stream* s, int64_t i, int64_t last, bool with_part0) {
+    if (with_part0) {
+        const int j = (int)(i % s->P);
+        SVA_TRY(s->fwd(j, sva_rows_run_part(s->ctxs[j], 0)));
+        SVA_STREAM_CUDA_OK(s, cudaEventRecord(s->ev_p0[j], s->compute));
+    }
+    const int64_t f1 = i - s->lag1, f2 = i - s->lag2;
+    if (f1 >= s->fill && f1 < last) SVA_TRY(s->fwd((int)(f1 % s->P), sva_rows_run_part(s->ctxs[f1 % s->P], 1)));
+    if (f2 >= s->fill && f2 < last) {
+        const int j = (int)(f2 % s->P), k = (int)(f2 % (int64_t)s->slots.size());
+        sva_ctx* c = s->ctxs[j];
+        RowsLink* l = s->links[j];
+        SVA_STREAM_CUDA_OK(s, cudaStreamWaitEvent(s->compute, s->ev_out[j], 0));   // the context's previous frame is out of disp / subpix
+        SVA_STREAM_CUDA_OK(s, cudaStreamWaitEvent(s->compute, s->ev_mask[j], 0));  // this frame's mask is in
+        SVA_TRY(s->fwd(j, sva_rows_run_part(c, 2)));
+        SVA_STREAM_CUDA_OK(s, cudaEventRecord(s->ev_p2[j], s->compute));
+        SVA_STREAM_CUDA_OK(s, cudaStreamWaitEvent(s->d2h, s->ev_p2[j], 0));
+        uint8_t* st = s->staging + (size_t)k * s->slot_bytes;
+        SVA_STREAM_CUDA_OK(s, cudaMemcpyAsync(st, c->disp.p, s->disp_bytes, cudaMemcpyDeviceToHost, s->d2h));
+        if (s->slots[k].sub) SVA_STREAM_CUDA_OK(s, cudaMemcpyAsync(st + s->sub_at, c->subpix.p, s->sub_bytes, cudaMemcpyDeviceToHost, s->d2h));
+        SVA_STREAM_CUDA_OK(s, cudaMemcpyAsync(st + s->err_at, l->flag(l->mem, F_ERR), sizeof(uint32_t), cudaMemcpyDeviceToHost, s->d2h));
+        SVA_STREAM_CUDA_OK(s, cudaEventRecord(s->ev_out[j], s->d2h));
+        SVA_STREAM_CUDA_OK(s, cudaEventRecord(s->ev_slot[k], s->d2h));
+        s->finished = f2 + 1;
+    }
+    return SVA_OK;
+}
+
+extern "C" {
+
+int sva_rows_stream_create(sva_ctx* const* ctxs, int32_t n_ctxs, const sva_params* p, sva_rows_stream** out) {
+    if (!ctxs || !ctxs[0] || !out) return SVA_ERR_BAD_ARG;
+    *out = nullptr;
+    sva_ctx* c0 = ctxs[0];
+    if (!p) return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: null params");
+    RowsLink* l0 = (RowsLink*)c0->rows_link;
+    if (!l0) return c0->fail(SVA_ERR_STATE, "rows_stream_create: context 0 has no link (sva_rows_open first)");
+    const int G = l0->world, P = G + 1;
+    if (n_ctxs != P) return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: the skewed order keeps world + 1 = " + std::to_string(P) + " frames in flight: pass that many contexts, not " + std::to_string(n_ctxs));
+    if (p->width != l0->W || p->height != l0->H || p->num_disp != l0->D || p->n_paths != 8)
+        return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: the parameters do not match the geometry the links were opened for");
+    for (int j = 0; j < P; j++) {
+        sva_ctx* c = ctxs[j];
+        if (!c) return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: null context");
+        for (int k = 0; k < j; k++) if (ctxs[k] == c) return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: a context is passed twice");
+        const RowsLink* l = (const RowsLink*)c->rows_link;
+        if (!l) return c0->fail(SVA_ERR_STATE, "rows_stream_create: context " + std::to_string(j) + " has no link (sva_rows_open first)");
+        if (l->rank != l0->rank || l->world != G || l->W != l0->W || l->H != l0->H || l->D != l0->D)
+            return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: the links of the contexts were opened for different ranks, worlds or geometries");
+        if (l->part_done != 2) return c0->fail(SVA_ERR_STATE, "rows_stream_create: context " + std::to_string(j) + " is in the middle of a frame (sva_rows_run_part)");
+        if (c->device != c0->device || c->stream != c0->stream)
+            return c0->fail(SVA_ERR_BAD_ARG, "rows_stream_create: every context must run on the same stream (sva_get_stream / sva_set_stream)");
+    }
+    SVA_CUDA_OK(c0, cudaSetDevice(c0->device));
+    sva_rows_stream* s = new sva_rows_stream();
+    s->ctxs.assign(ctxs, ctxs + P);
+    for (int j = 0; j < P; j++) s->links.push_back((RowsLink*)ctxs[j]->rows_link);
+    s->p = *p;
+    s->rank = l0->rank; s->world = G; s->P = P;
+    s->lag1 = 1 + std::min(s->rank, G - 1 - s->rank);
+    s->lag2 = 1 + std::max(s->rank, G - 1 - s->rank);
+    s->compute = c0->stream;
+    auto align = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    s->disp_bytes = (size_t)p->width * l0->rows * sizeof(uint16_t);
+    s->sub_bytes = (size_t)p->width * l0->rows * sizeof(float);
+    s->sub_at = align(s->disp_bytes);
+    s->err_at = s->sub_at + align(s->sub_bytes);
+    s->slot_bytes = s->err_at + 256;
+    s->slots.resize(G + 2);
+    auto setup = [&]() -> int {
+        SVA_STREAM_CUDA_OK(s, cudaStreamCreateWithFlags(&s->h2d, cudaStreamNonBlocking));
+        SVA_STREAM_CUDA_OK(s, cudaStreamCreateWithFlags(&s->d2h, cudaStreamNonBlocking));
+        for (auto* v : {&s->ev_img, &s->ev_mask, &s->ev_p0, &s->ev_p2, &s->ev_out})
+            for (int j = 0; j < P; j++) { v->push_back(nullptr); SVA_STREAM_CUDA_OK(s, cudaEventCreateWithFlags(&v->back(), cudaEventDisableTiming)); }
+        for (size_t k = 0; k < s->slots.size(); k++) { s->ev_slot.push_back(nullptr); SVA_STREAM_CUDA_OK(s, cudaEventCreateWithFlags(&s->ev_slot.back(), cudaEventDisableTiming)); }
+        cudaError_t e = cudaMallocHost(&s->staging, s->slot_bytes * s->slots.size());
+        if (e != cudaSuccess) { s->staging = nullptr; return s->fail(SVA_ERR_NOMEM, std::string("cudaMallocHost: ") + cudaGetErrorString(e)); }
+        const std::vector<uint8_t> zeros((size_t)p->width * p->height, 0);
+        for (int j = 0; j < P; j++) SVA_TRY(s->fwd(j, rows_stream_warm_up(s, j, zeros)));
+        return SVA_OK;
+    };
+    const int rc = setup();
+    if (rc != SVA_OK) { rows_stream_release(s); return rc; }
+    *out = s;
+    return SVA_OK;
+}
+
+int sva_rows_stream_connect_comm(sva_rows_stream* s) {
+    if (!s) return SVA_ERR_BAD_ARG;
+    if (s->next > s->finished) return s->fail(SVA_ERR_STATE, "connect_comm: frames are in flight (flush first)");
+    if (s->world == 1) return SVA_OK;  // no neighbours
+    sva_ctx* c0 = s->ctxs[0];
+    if (!c0->comm) return s->fail(SVA_ERR_STATE, "connect_comm: context 0 has no communicator (sva_comm_init)");
+    if (c0->comm_rank != s->rank || c0->comm_world != s->world) return s->fail(SVA_ERR_BAD_ARG, "connect_comm: the communicator's rank / world differ from the links'");
+    for (int j = 0; j < s->P; j++)
+        if (s->ctxs[j]->rows_link != s->links[j]) return s->fail(SVA_ERR_STATE, "connect_comm: a link was re-opened or closed since create");
+    const int P = s->P, G = s->world;
+    const size_t per_rank = (size_t)P * SVA_IPC_HANDLE_BYTES;
+    std::vector<uint8_t> all((size_t)G * per_rank);
+    for (int j = 0; j < P; j++) SVA_TRY(s->fwd(j, sva_rows_export(s->ctxs[j], all.data() + s->rank * per_rank + (size_t)j * SVA_IPC_HANDLE_BYTES)));
+    SVA_CUDA_OK(c0, cudaSetDevice(c0->device));
+    SVA_TRY(c0->reserve(c0->comm_scratch, std::max<size_t>(256, all.size())));
+    uint8_t* d = c0->comm_scratch.as<uint8_t>();
+    SVA_CUDA_OK(c0, cudaMemcpyAsync(d + s->rank * per_rank, all.data() + s->rank * per_rank, per_rank, cudaMemcpyHostToDevice, c0->stream));
+    SVA_NCCL_OK(c0, nccl()->AllGather(d + s->rank * per_rank, d, per_rank, NCCL_UINT8, (NcclComm)c0->comm, c0->stream));
+    SVA_CUDA_OK(c0, cudaMemcpyAsync(all.data(), d, all.size(), cudaMemcpyDeviceToHost, c0->stream));
+    SVA_CUDA_OK(c0, cudaStreamSynchronize(c0->stream));
+    for (int j = 0; j < P; j++) {
+        auto handle = [&](int r) { return all.data() + (size_t)r * per_rank + (size_t)j * SVA_IPC_HANDLE_BYTES; };
+        SVA_TRY(s->fwd(j, sva_rows_connect(s->ctxs[j], s->rank > 0 ? handle(s->rank - 1) : nullptr, s->rank < G - 1 ? handle(s->rank + 1) : nullptr)));
+    }
+    return sva_comm_barrier(c0);  // nobody runs ahead of a neighbour that has not mapped its side yet
+}
+
+int sva_rows_stream_submit(sva_rows_stream* s, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
+                           uint16_t* out_disp_rows, float* out_subpix_rows, int64_t* out_ticket) {
+    if (!s) return SVA_ERR_BAD_ARG;
+    if (!out_disp_rows || !out_ticket) return s->fail(SVA_ERR_BAD_ARG, "submit: null output");
+    const int G = s->world;
+    for (int j = 0; j < s->P; j++) {
+        const RowsLink* l = s->links[j];
+        if (s->ctxs[j]->rows_link != l) return s->fail(SVA_ERR_STATE, "submit: a link was re-opened or closed since create");
+        if ((s->rank > 0 && !l->prev) || (s->rank < G - 1 && !l->next))
+            return s->fail(SVA_ERR_STATE, "submit: the link of context " + std::to_string(j) + " is not connected (sva_rows_connect*, sva_rows_stream_connect_comm)");
+    }
+    SVA_TRY(check_frame_args(s->ctxs[0], &s->p, ref, others, mask));
+    SVA_CUDA_OK(s->ctxs[0], cudaSetDevice(s->ctxs[0]->device));
+    const int64_t i = s->next;
+    const int j = (int)(i % s->P), k = (int)(i % (int64_t)s->slots.size());
+    sva_rows_stream::Slot& sl = s->slots[k];
+    if (!sl.retired) SVA_TRY(rows_stream_retire(s, k));  // ticket i - (G + 2): its download is at least two iterations old
+    sl.ticket = i; sl.retired = false; sl.disp = out_disp_rows; sl.sub = out_subpix_rows;
+    sva_ctx* c = s->ctxs[j];
+    SVA_STREAM_CUDA_OK(s, cudaStreamWaitEvent(s->h2d, s->ev_p0[j], 0));  // K1a of the context's previous frame has read its images
+    c->stream = s->h2d;
+    const int rc = sva_frame_upload(c, &s->p, ref, others, nullptr);
+    c->stream = s->compute;
+    if (rc != SVA_OK) { sl.retired = true; sl.ticket = -1; return s->fwd(j, rc); }
+    SVA_STREAM_CUDA_OK(s, cudaEventRecord(s->ev_img[j], s->h2d));
+    SVA_STREAM_CUDA_OK(s, cudaStreamWaitEvent(s->compute, s->ev_img[j], 0));
+    if (mask) {  // K3 of the context's previous frame has read its mask (the buffer exists since create: no allocation here)
+        SVA_STREAM_CUDA_OK(s, cudaStreamWaitEvent(s->h2d, s->ev_p2[j], 0));
+        SVA_TRY(s->fwd(j, c->reserve(c->mask, (size_t)s->p.width * s->p.height)));
+        SVA_STREAM_CUDA_OK(s, cudaMemcpy2DAsync(c->mask.p, s->p.width, mask->data, mask->step, s->p.width, s->p.height, cudaMemcpyHostToDevice, s->h2d));
+        c->has_mask = true;
+    }
+    SVA_STREAM_CUDA_OK(s, cudaEventRecord(s->ev_mask[j], s->h2d));  // (without a mask: right after the images, a wait that costs nothing)
+    s->next = i + 1;
+    *out_ticket = i;
+    return rows_stream_iteration(s, i, i + 1, true);
+}
+
+int sva_rows_stream_flush(sva_rows_stream* s) {
+    if (!s) return SVA_ERR_BAD_ARG;
+    SVA_CUDA_OK(s->ctxs[0], cudaSetDevice(s->ctxs[0]->device));
+    for (int64_t i = s->next; s->finished < s->next; i++) SVA_TRY(rows_stream_iteration(s, i, s->next, false));
+    s->fill = s->next;
+    return SVA_OK;
+}
+
+int sva_rows_stream_wait(sva_rows_stream* s, int64_t ticket) {
+    if (!s) return SVA_ERR_BAD_ARG;
+    if (ticket < 0 || ticket >= s->next) return s->fail(SVA_ERR_BAD_ARG, "wait: unknown ticket " + std::to_string(ticket));
+    const int k = (int)(ticket % (int64_t)s->slots.size());
+    if (s->slots[k].ticket == ticket && !s->slots[k].retired) {
+        if (ticket >= s->finished) return s->fail(SVA_ERR_STATE, "wait: the last part of frame " + std::to_string(ticket) + " is not enqueued yet (submit more frames, or flush)");
+        SVA_CUDA_OK(s->ctxs[0], cudaSetDevice(s->ctxs[0]->device));
+        SVA_TRY(rows_stream_retire(s, k));
+    }
+    if (s->failed.count(ticket))
+        return s->fail(SVA_ERR_COMM, "frame " + std::to_string(ticket) + ": a neighbour's path-line state did not arrive within the time-out (SVA_ROWS_TIMEOUT_MS); the block's maps are not valid");
+    return SVA_OK;
+}
+
+int sva_rows_stream_destroy(sva_rows_stream* s) {
+    if (!s) return SVA_ERR_BAD_ARG;
+    cudaSetDevice(s->ctxs[0]->device);
+    cudaStreamSynchronize(s->compute);
+    rows_stream_release(s);
+    return SVA_OK;
+}
+
+}  // extern "C"

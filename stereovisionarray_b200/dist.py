@@ -285,6 +285,23 @@ def rows_direct_connect(ctx, p, rank, world, group=None):
     dist.barrier(group=group)  # nobody runs ahead of a neighbour that has not mapped its side yet
 
 
+def rows_stream_connect(ctxs, p, rank, world, group=None):
+    """rows_direct_connect for the world + 1 contexts of a pipeline.RowsStream (context j of every rank is one chain): opens every link and
+    maps the neighbours' state buffers, with one all-gather of this rank's world + 1 handles.  Collective; create the RowsStream afterwards."""
+    import torch.distributed as dist
+    if len(ctxs) != world + 1:
+        raise ValueError("the skewed order keeps world + 1 = %d frames in flight: that many contexts per GPU" % (world + 1))
+    for c in ctxs:
+        c.rows_open(p, rank, world)
+    if world == 1:
+        return
+    handles = [None] * world
+    dist.all_gather_object(handles, [c.rows_export() for c in ctxs], group=group)
+    for j, c in enumerate(ctxs):
+        c.rows_connect(handles[rank - 1][j] if rank > 0 else None, handles[rank + 1][j] if rank < world - 1 else None)
+    dist.barrier(group=group)
+
+
 def rows_direct_depth(ctx, p, ref, others, mask, rank, world, group=None):
     """One frame through the peer-direct row-block pipeline (sva_rows_*; rows_direct_connect first): the path-line state is stored by the
     neighbour's march kernel straight into this GPU's memory and sequenced by device flags.  Returns (disp, subpix) on rank 0, None elsewhere."""

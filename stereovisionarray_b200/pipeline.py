@@ -308,3 +308,78 @@ class DepthContext:
         ms = C.c_float()
         check(self._h, self._L.sva_stream_elapsed(self._h, C.c_int64(ticket), C.byref(ms)))
         return ms.value
+
+
+class RowsStream:
+    """A stream of frames through the peer-direct row-block pipeline in the order skewed by chain position, one call per frame and rank
+    (sva_rows_stream_*, DESIGN.md §7).  ctxs: this rank's world + 1 DepthContexts, all on one stream, each through rows_open(p, rank, world)
+    (dist.rows_stream_connect opens and connects them; or connect them after creating the stream with connect_comm).  The contexts are
+    borrowed: close the stream before them.
+
+    submit() uploads on a copy stream and returns a ticket; the block's rows (rows_block() of the contexts) reach disp_out / sub_out in
+    wait(ticket) or when the ticket's slot is reused world + 2 frames later, whichever comes first.  Until then the input images and the output
+    arrays must stay untouched (this object keeps them alive); pinned inputs (torch pin_memory tensors viewed as numpy) let the upload overlap
+    the marches.  flush() enqueues the drain: afterwards every submitted frame completes."""
+
+    def __init__(self, ctxs, p):
+        self._L = lib()
+        self._h = None
+        self._ctxs = list(ctxs)  # the stream borrows them: keep them alive as long as it exists
+        self._err = ctxs[0]._h
+        arr = (C.c_void_p * len(ctxs))(*[c._h.value for c in ctxs])
+        h = C.c_void_p()
+        check(self._err, self._L.sva_rows_stream_create(arr, len(ctxs), C.byref(p), C.byref(h)))
+        self._h = h
+        self.params = p
+        self.slots = len(ctxs) + 1  # world + 2
+        self.rows = ctxs[0].rows_block()[1]
+        self._keep = {}
+
+    def connect_comm(self):
+        """collective: connect all world + 1 links over the communicator of ctxs[0] (comm_init)"""
+        check(self._err, self._L.sva_rows_stream_connect_comm(self._h))
+
+    def submit(self, ref, others, mask, disp_out, sub_out=None):
+        """enqueue one iteration of the skewed order for a new frame -> ticket.  disp_out: (rows, width) uint16, sub_out: (rows, width)
+        float32 or None"""
+        p = self.params
+        for a, dt in ((disp_out, np.uint16), (sub_out, np.float32)):
+            if a is not None and (a.dtype != dt or a.shape != (self.rows, p.width) or not a.flags.c_contiguous):
+                raise ValueError("output must be a C-contiguous (%d, %d) %s array" % (self.rows, p.width, np.dtype(dt).name))
+        r, rk = abi.image_u8(ref)
+        o, ok = abi.image_array(others) if not isinstance(others, tuple) else others
+        m = mk = None
+        if mask is not None:
+            m, mk = abi.image_u8(mask)
+        t = C.c_int64()
+        check(self._err, self._L.sva_rows_stream_submit(self._h, C.byref(r), o, C.byref(m) if m is not None else None, _p(disp_out, C.c_uint16),
+                                                         _p(sub_out, C.c_float) if sub_out is not None else None, C.byref(t)))
+        self._keep[t.value] = (rk, ok, mk, disp_out, sub_out)
+        for old in [k for k in self._keep if k <= t.value - self.slots]:  # retired when their slot was reused
+            del self._keep[old]
+        return t.value
+
+    def flush(self):
+        check(self._err, self._L.sva_rows_stream_flush(self._h))
+
+    def wait(self, ticket):
+        """blocks until the ticket's rows are in its output arrays; SvaError with code SVA_ERR_COMM if a hand-off timed out"""
+        try:
+            check(self._err, self._L.sva_rows_stream_wait(self._h, C.c_int64(ticket)))
+        except SvaError as e:
+            if e.code == abi.SVA_ERR_COMM:
+                self._keep.pop(ticket, None)
+            raise
+        self._keep.pop(ticket, None)
+
+    def close(self):
+        if self._h:
+            self._L.sva_rows_stream_destroy(self._h)
+            self._h = None
+            self._keep.clear()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

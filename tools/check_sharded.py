@@ -4,8 +4,9 @@
 
 Schemes: pairs (C: sva_depth_pair_sharded, NCCL reduce from the library), slices and rows (Python + torch.distributed), rows_direct
 (C: sva_rows_*, peer-direct hand-off over CUDA IPC), rows_stream (rows_direct over a stream of distinct frames in the order skewed by chain
-position, dist.rows_direct_stream, every frame checked).  Small frames are checked against a live oracle run; --c3 checks the full
-3840x2160x256 frame against the oracle digests in tests/golden/c3_full_oracle.json (tests/golden/make_c3_hash.py) and the stream on c3's
+position, dist.rows_direct_stream, every frame checked), rows_stream_c (the same stream through the C library's one call per frame,
+sva_rows_stream_* via pipeline.RowsStream, links connected with dist.rows_stream_connect).  Small frames are checked against a live oracle run; --c3 checks the full
+3840x2160x256 frame against the oracle digests in tests/golden/c3_full_oracle.json (tests/golden/make_c3_hash.py) and the streams on c3's
 width, D and pairs at 24 rows per rank (+ the border bands) against a live oracle run, and --time adds device-timed runs of the row pipelines at full size.
 Exit code 1 on any mismatch."""
 import argparse
@@ -26,7 +27,7 @@ from stereovisionarray_b200.pipeline import DepthContext  # noqa: E402
 ap = argparse.ArgumentParser()
 ap.add_argument("--c3", action="store_true", help="the full c3 frame against the committed oracle digests")
 ap.add_argument("--time", action="store_true", help="with --c3: device-timed row pipelines")
-ap.add_argument("--schemes", default="pairs,slices,rows,rows_direct,rows_stream,adapter")
+ap.add_argument("--schemes", default="pairs,slices,rows,rows_direct,rows_stream,rows_stream_c,adapter")
 args = ap.parse_args()
 
 rank, local, world = int(os.environ["RANK"]), int(os.environ["LOCAL_RANK"]), int(os.environ["WORLD_SIZE"])
@@ -149,19 +150,48 @@ def rows_stream(p, scenes):
     return got
 
 
-def check_stream(p, scenes, tag):
+def rows_stream_c(p, scenes):
+    """the frames `scenes` through the C library's stream (pipeline.RowsStream: one sva_rows_stream_submit per frame, uploads and downloads on
+    copy streams), world + 1 contexts on one stream linked with dist.rows_stream_connect; every frame's rows are gathered on rank 0 after a
+    flush.  -> [(frame, (disp, subpix))] on rank 0"""
+    from stereovisionarray_b200.pipeline import RowsStream
+    ctxs, got, s = [], [], None
+    try:
+        for j in range(world + 1):
+            c = DepthContext(local)
+            ctxs.append(c)
+            if j:
+                c.set_stream(ctxs[0].get_stream())
+        sdist.rows_stream_connect(ctxs, p, rank, world)
+        s = RowsStream(ctxs, p)
+        outs = [(np.empty((s.rows, p.width), np.uint16), np.empty((s.rows, p.width), np.float32)) for _ in scenes]
+        tickets = [s.submit(sc["ref"], sc["others"], sc["mask"], *o) for sc, o in zip(scenes, outs)]
+        s.flush()
+        for t in tickets:
+            s.wait(t)
+            got.append((t, sdist.gather_rows(outs[t][0], outs[t][1], p, rank, world)))
+        dist.barrier()  # nobody unmaps a link a neighbour still writes into
+    finally:
+        if s is not None:
+            s.close()
+        for c in reversed(ctxs):  # the borrowers first: ctxs[0] owns the stream
+            c.close()
+    return got
+
+
+def check_stream(p, scenes, tag, name="rows_stream", run=rows_stream):
     global ok
-    got = rows_stream(p, scenes)
+    got = run(p, scenes)
     if rank != 0:
         return
     from oracle.oracle import Oracle
     if [f for f, _ in got] != list(range(len(scenes))):
-        say("rows_stream %s over %d GPUs vs oracle: MISMATCH (frames downloaded: %s)" % (tag, world, [f for f, _ in got]))
+        say("%s %s over %d GPUs vs oracle: MISMATCH (frames downloaded: %s)" % (name, tag, world, [f for f, _ in got]))
         ok = False
     for f, (d, s) in got:
         d0, s0 = Oracle().depth_from_array(p, scenes[f]["ref"], scenes[f]["others"], scenes[f]["mask"])
         same = np.array_equal(d, d0) and np.array_equal(s, s0) and bool((d0 != 0xFFFF).any())  # a frame with no valid pixel checks nothing
-        say("rows_stream %s frame %d over %d GPUs vs oracle: %s (valid %.3f)" % (tag, f, world, "bit-exact" if same else "MISMATCH", float((d0 != 0xFFFF).mean())))
+        say("%s %s frame %d over %d GPUs vs oracle: %s (valid %.3f)" % (name, tag, f, world, "bit-exact" if same else "MISMATCH", float((d0 != 0xFFFF).mean())))
         ok = ok and same
 
 
@@ -186,6 +216,8 @@ if not args.c3:
                 ok = ok and same
         if "rows_stream" in schemes:
             check_stream(p, stream_scenes(h, w, D, off), "%dx%dx%d" % (w, h, D))
+        if "rows_stream_c" in schemes:
+            check_stream(p, stream_scenes(h, w, D, off), "%dx%dx%d" % (w, h, D), "rows_stream_c", rows_stream_c)
 else:
     with open(os.path.join(ROOT, "tests", "golden", "c3_full_oracle.json")) as f:
         gold = json.load(f)
@@ -203,10 +235,13 @@ else:
             say("%s c3 3840x2160x256, 15 pairs, %d GPUs vs oracle digests: integer map %s, sub-pixel map %s (valid pixels %d / %d)"
                 % (name, world, "bit-exact" if same_d else "MISMATCH", "bit-exact" if same_s else "MISMATCH", int((o[0] != 0xFFFF).sum()), gold["valid_pixels"]))
             ok = ok and same_d and same_s
-    if "rows_stream" in schemes:  # distinct full-size c3 frames would cost a minute of oracle time each: c3's width, D and pairs at a
-        ps = configs.params("c3")  # height of 24 rows per rank plus the two border bands of win_half rows, which hold no valid pixel
-        ps.height = 24 * world + 2 * ps.win_half
-        check_stream(ps, stream_scenes(ps.height, ps.width, ps.num_disp, configs.offsets("c3")), "c3 3840x%dx256" % ps.height)
+    # distinct full-size c3 frames would cost a minute of oracle time each: the streams run c3's width, D and pairs at a height of 24 rows per
+    # rank plus the two border bands of win_half rows, which hold no valid pixel
+    ps = configs.params("c3")
+    ps.height = 24 * world + 2 * ps.win_half
+    for name, run in (("rows_stream", rows_stream), ("rows_stream_c", rows_stream_c)):
+        if name in schemes:
+            check_stream(ps, stream_scenes(ps.height, ps.width, ps.num_disp, configs.offsets("c3")), "c3 3840x%dx256" % ps.height, name, run)
     if args.time:
         ctx = DepthContext(local)
         stream = torch.cuda.current_stream()
