@@ -16,6 +16,8 @@ std::array<uint8_t, SVA_COMM_ID_BYTES> svaCommUniqueId();
 void svaCommInit(const std::array<uint8_t, SVA_COMM_ID_BYTES>& id, int rank, int world);
 std::vector<uint16_t> svaDepthPairSharded(const sva_params&, cv::Mat&, std::vector<cv::Mat>&, cv::Mat*, int, std::vector<float>*);
 std::vector<uint16_t> svaDepthRowsSharded(const sva_params&, cv::Mat&, std::vector<cv::Mat>&, cv::Mat*, int, int, int*, int*, std::vector<float>*);
+std::vector<std::vector<uint16_t>> svaDepthGroups(const sva_params&, std::vector<cv::Mat>&, const std::vector<std::vector<std::array<int, 2>>>&, int,
+                                                  const std::vector<cv::Mat>*, std::vector<std::vector<float>>*);
 
 static cv::Mat g_mask;
 cv::Mat getFaceMask(cv::Mat&) { return g_mask.clone(); }
@@ -129,5 +131,34 @@ extern "C" int adapter_rows_stream(int device, const uint8_t* id128, int rank, i
         *out_y0 = s.y0();
         *out_rows = s.rows();
         return 0;
+    } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
+// the 13 CHESS groups of a 5 x 5 frame the way a reference host gets them: getGroups(cameras, "CHESS") straight into svaDepthGroups.  masks13:
+// null, or one pointer per group (null: no mask).  Group g's maps land at out_disp / out_sub + g * w * h.  Returns the number of groups.
+extern "C" int adapter_depth_groups(const sva_params* p, const uint8_t* const* images25, const uint8_t* const* masks13, uint16_t* out_disp, float* out_sub) {
+    try {
+        const int w = p->width, h = p->height;
+        auto mat = [&](const uint8_t* src) { cv::Mat m(h, w, CV_8UC1); std::memcpy(m.data, src, (size_t)w * h); return m; };
+        double f = 0.05, sensor_size = 0.036, pixelSize = sensor_size / w;
+        std::vector<Camera> cameras;
+        std::vector<cv::Mat> images;
+        for (int y = 0; y < 5; y++)
+            for (int x = 0; x < 5; x++) {
+                cameras.push_back(Camera(f, cv::Point3d{-0.1 + x * 0.05, -0.1 + y * 0.05, -0.75}, pixelSize));
+                images.push_back(mat(images25[5 * y + x]));
+            }
+        auto groups = getGroups(cameras, "CHESS");
+        std::vector<cv::Mat> masks;
+        if (masks13)
+            for (size_t g = 0; g < groups.size(); g++) masks.push_back(masks13[g] ? mat(masks13[g]) : cv::Mat());
+        std::vector<std::vector<float>> sub;
+        std::vector<std::vector<uint16_t>> disp = svaDepthGroups(*p, images, groups, 5, masks13 ? &masks : nullptr, &sub);
+        const size_t px = (size_t)w * h;
+        for (size_t g = 0; g < groups.size(); g++) {
+            std::memcpy(out_disp + g * px, disp[g].data(), px * 2);
+            std::memcpy(out_sub + g * px, sub[g].data(), px * 4);
+        }
+        return (int)groups.size();
     } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }

@@ -170,6 +170,32 @@ std::vector<std::vector<std::array<int, 2>>> getGroups(std::vector<Camera>& came
     return groups;
 }
 
+// ---- every reference view of one array frame in one call (sva_depth_groups) ----
+// groups as getGroups returns them (e.g. getGroups(cameras, "CHESS"), quirks included), images on a grid of gridCols columns; masks: null, or one
+// per group (an empty Mat: no mask).  -> one u16 map (rows * cols; SVA_DISP_INVALID where rejected) per group, and the sub-pixel maps in *subpix
+std::vector<std::vector<uint16_t>> svaDepthGroups(const sva_params& p, std::vector<cv::Mat>& images, const std::vector<std::vector<std::array<int, 2>>>& groups,
+                                                  int gridCols, const std::vector<cv::Mat>* masks, std::vector<std::vector<float>>* subpix) {
+    if (masks && masks->size() != groups.size()) throw cv::Exception("svaDepthGroups: one mask (or an empty Mat) per group");
+    std::vector<sva_image_u8> ims, mk;
+    for (auto& m : images) ims.push_back(m.empty() ? sva_image_u8{} : view(m));
+    if (masks) for (auto& m : *masks) mk.push_back(m.empty() ? sva_image_u8{} : view(m));
+    std::vector<int32_t> pairs, sizes;
+    for (auto& g : groups) {
+        sizes.push_back((int32_t)g.size());
+        for (auto& pr : g) { pairs.push_back(pr[0]); pairs.push_back(pr[1]); }
+    }
+    const size_t n = groups.size(), px = (size_t)p.width * p.height;
+    std::vector<std::vector<uint16_t>> disp(n, std::vector<uint16_t>(px));
+    std::vector<std::vector<float>> sub(n, std::vector<float>(px));
+    std::vector<uint16_t*> dp;
+    std::vector<float*> sp;
+    for (size_t g = 0; g < n; g++) { dp.push_back(disp[g].data()); sp.push_back(sub[g].data()); }
+    check(sva_depth_groups(ctx(), &p, gridCols, ims.data(), (int32_t)ims.size(), pairs.data(), sizes.data(), (int32_t)n, 0, (int32_t)n, masks ? mk.data() : nullptr,
+                           dp.data(), sp.data()), "svaDepthGroups");
+    if (subpix) *subpix = std::move(sub);
+    return disp;
+}
+
 // ---- one frame over several GPUs (one process per GPU; any launcher — mpirun, torchrun, a shell loop — provides rank and world) ----
 // No reference counterpart (the reference is one thread): the sharding units are its pair loop (src/CameraStereoVision.cpp:55) and its
 // pixel-row loop (:49).  Rank 0 calls svaCommUniqueId() and hands the 128 bytes to the others by whatever channel the launcher offers;

@@ -183,6 +183,25 @@ int sva_stream_wait(sva_ctx* ctx, int64_t ticket);
 int sva_stream_mark(sva_ctx* ctx);
 int sva_stream_elapsed(sva_ctx* ctx, int64_t ticket, float* out_ms);
 
+/* getGroups — include/functions.h:28, src/functions.cpp:107-116: the depth map of every reference view of ONE array frame, in one call.
+ * images[n_images]: the frame's cameras on a grid of grid_cols columns (camera i at row i / grid_cols, column i % grid_cols).  The groups come in
+ * the layout sva_get_groups writes: pairs[2 * k] = {ref, other} flattened, sizes[g] pairs in group g, every pair of a group with the same
+ * reference (the CHESS list goes in unchanged, its duplicate pairs included).  Pair j of group g gets the grid offsets
+ * gx = col(other) - col(ref), gy = row(other) - row(ref); p is a template whose n_pairs, pair_gx and pair_gy are zero, every other field
+ * applies to every group.  The groups [group_begin, group_end) are computed: out_disp[g - group_begin] (width x height u16) and, when
+ * out_subpix and its entry are not NULL, out_subpix[g - group_begin] (f32) receive exactly what sva_depth_from_array returns for that group's
+ * parameters, reference view, other views and mask.  masks: NULL, or one per group of the range (data == NULL: no mask).  Only the cameras
+ * these groups read need data; the others may have data == NULL, so a rank of a sharded frame passes and uploads only its own cameras.
+ * Each camera read is uploaded once; the groups then run through the capture-stream pipeline of sva_stream_submit (frames in flight there
+ * complete first, and their tickets stay waitable).  Synchronous: returns once every map is in the caller's buffers.
+ * SVA_ERR_BAD_ARG, with nothing enqueued: a group whose pairs do not share one reference, a pair of a camera with itself, an index outside
+ * [0, n_images), n_images not a multiple of grid_cols, a group range outside [0, n_groups], a group whose derived parameters are refused
+ * (e.g. more than 32 pairs, a window sum that overflows), a camera read by the range without data or not width x height, a mask of the
+ * wrong size. */
+int sva_depth_groups(sva_ctx* ctx, const sva_params* p, int32_t grid_cols, const sva_image_u8* images, int32_t n_images, const int32_t* pairs,
+                     const int32_t* sizes, int32_t n_groups, int32_t group_begin, int32_t group_end, const sva_image_u8* masks,
+                     uint16_t* const* out_disp, float* const* out_subpix);
+
 /* ---- staged, device-resident form of the same pipeline (what bench.py times with inputs already in HBM) ------- */
 typedef enum sva_stage {
     SVA_STAGE_AD = 1,        /* K1a: A(y,x,d) = sum_k |R - I_k(shifted)|            -> u16 [H][W][D] */

@@ -27,7 +27,7 @@ EXPORTS = [
     "sva_rows_open", "sva_rows_export", "sva_rows_connect", "sva_rows_connect_comm", "sva_rows_connect_local", "sva_rows_block", "sva_rows_run", "sva_rows_run_phase", "sva_rows_run_part", "sva_get_stream",
     "sva_rows_download", "sva_rows_close", "sva_depth_rows_sharded",
     "sva_rows_stream_create", "sva_rows_stream_connect_comm", "sva_rows_stream_submit", "sva_rows_stream_flush", "sva_rows_stream_wait",
-    "sva_rows_stream_destroy",
+    "sva_rows_stream_destroy", "sva_depth_groups",
 ]
 
 _lib = None
@@ -74,6 +74,8 @@ def lib():
         L.sva_rows_stream_wait.argtypes = [C.c_void_p, C.c_int64]
         for n in ("sva_rows_stream_connect_comm", "sva_rows_stream_flush", "sva_rows_stream_destroy"):
             getattr(L, n).argtypes = [C.c_void_p]
+        L.sva_depth_groups.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                       C.c_void_p, C.c_void_p, C.c_void_p]
         missing = [n for n in EXPORTS if not hasattr(L, n)]
         if missing:
             raise ImportError("libsva_b200.so does not export %s — rebuild it" % missing)

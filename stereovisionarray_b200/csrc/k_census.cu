@@ -13,10 +13,8 @@
 #define CENSUS_RX 4
 #define CENSUS_RY 3
 
-__global__ void __launch_bounds__(128)
-k_census_transform(const uint8_t* __restrict__ img, size_t pitch, int W, int H, uint64_t* __restrict__ out) {
-    const int x = blockIdx.x * 128 + threadIdx.x, y = blockIdx.y;
-    if (x >= W) return;
+// signature of pixel (x, y): shared by the per-view transform and the batched transform of an array frame's camera stack
+__device__ __forceinline__ uint64_t census_signature(const uint8_t* __restrict__ img, size_t pitch, int W, int H, int x, int y) {
     const int c = img[(size_t)y * pitch + x];
     uint64_t t = 0;
     int bit = 0;
@@ -33,7 +31,44 @@ k_census_transform(const uint8_t* __restrict__ img, size_t pitch, int W, int H, 
             bit++;
         }
     }
-    out[(size_t)y * W + x] = t;
+    return t;
+}
+
+__global__ void __launch_bounds__(128)
+k_census_transform(const uint8_t* __restrict__ img, size_t pitch, int W, int H, uint64_t* __restrict__ out) {
+    const int x = blockIdx.x * 128 + threadIdx.x, y = blockIdx.y;
+    if (x >= W) return;
+    out[(size_t)y * W + x] = census_signature(img, pitch, W, H, x, y);
+}
+
+// Cameras of an array frame's stack (tight W x H views, camera i at stack + i * W * H) whose signatures one launch computes.
+struct CensusCams {
+    int n;
+    int cam[SVA_MAX_PAIRS + 1];  // a group reads at most 32 other views and its reference
+};
+
+// the signatures of cameras L.cam[blockIdx.z] of the stack into the same slots of the signature stack
+__global__ void __launch_bounds__(128)
+k_census_transform_stack(const uint8_t* __restrict__ stack, int W, int H, const CensusCams L, uint64_t* __restrict__ sig) {
+    const int x = blockIdx.x * 128 + threadIdx.x, y = blockIdx.y;
+    if (x >= W) return;
+    const size_t off = (size_t)W * H * L.cam[blockIdx.z];
+    sig[off + (size_t)y * W + x] = census_signature(stack + off, (size_t)W, W, H, x, y);
+}
+
+// one launch for up to SVA_MAX_PAIRS + 1 cameras of the stack, on `stream`
+int sva_census_stack(sva_ctx* ctx, const uint8_t* stack, int W, int H, const int* cams, int n, uint64_t* sig, cudaStream_t stream) {
+    if (n <= 0) return SVA_OK;
+    if (n > SVA_MAX_PAIRS + 1) return ctx->fail(SVA_ERR_BAD_ARG, "census_stack: too many cameras in one launch");
+    CensusCams L{};
+    L.n = n;
+    for (int i = 0; i < n; i++) L.cam[i] = cams[i];
+    {
+        LaunchScope ls(ctx, "k_census_transform_stack");
+        k_census_transform_stack<<<dim3(div_up(W, 128), H, n), 128, 0, stream>>>(stack, W, H, L, sig);
+    }
+    SVA_CUDA_OK(ctx, cudaGetLastError());
+    return SVA_OK;
 }
 
 struct CensusPairs {
@@ -71,12 +106,29 @@ k_ad_census(const uint64_t* __restrict__ tr, const uint64_t* __restrict__ to, co
 
 int sva_ap_prepare(sva_ctx* ctx);
 
-// views as uploaded for this mode: ctx->ref_img / ctx->other_imgs, tight pitch W
+// views as uploaded for this mode: ctx->ref_img / ctx->other_imgs, tight pitch W; or, inside sva_depth_groups, the signatures of the
+// array frame's camera stack (ctx->sig_stack), computed once per camera for all groups
 int sva_run_ad_census(sva_ctx* ctx) {
     const sva_params& p = ctx->prm;
     const int W = p.width, H = p.height, D = p.num_disp;
     const size_t px = (size_t)W * H;
     SVA_TRY(sva_ap_prepare(ctx));
+    if (ctx->sig_stack) {
+        CensusPairs P{};
+        P.n = ctx->pair_end - ctx->pair_begin;
+        for (int i = 0; i < P.n; i++) {
+            const int k = ctx->pair_begin + i;
+            P.gx[i] = p.pair_gx[k]; P.gy[i] = p.pair_gy[k]; P.view[i] = ctx->sig_view[k];
+        }
+        {
+            LaunchScope ls(ctx, "k_ad_census");
+            k_ad_census<<<dim3(div_up(W, 128), H, div_up(D, 8)), 128, 0, ctx->stream>>>(ctx->sig_stack + px * ctx->sig_ref, ctx->sig_stack, P, W, H, D, p.min_disp,
+                                                                                        ctx->AP.as<uint32_t>(), ctx->ap.wp, ctx->ap.padl, ctx->ap.padt);
+        }
+        SVA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->have_ad = true;
+        return SVA_OK;
+    }
     SVA_TRY(ctx->reserve(ctx->census, px * sizeof(uint64_t) * (size_t)(p.n_pairs + 1)));
     uint64_t* tr = ctx->census.as<uint64_t>();
     uint64_t* to = tr + px;

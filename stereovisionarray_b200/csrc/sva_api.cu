@@ -27,8 +27,11 @@ int sva_run_sgm_dirs(sva_ctx* ctx, const uint16_t* Cext, int c_ds, uint32_t dir_
 int sva_run_wta_rows(sva_ctx* ctx, const uint16_t* vol, int y0, int rows);
 int sva_run_sgm_rows(sva_ctx* ctx, int group, int y0, int rows, const uint16_t* state_in, uint16_t* state_out);
 int sva_ap_unpack(sva_ctx* ctx);
+int sva_stream_enqueue(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
+                       cudaMemcpyKind view_kind, uint16_t* out_disp, float* out_subpix, int64_t* out_ticket);
 
-static int check_params(sva_ctx* c, const sva_params* p) {
+// (also used by sva_depth_groups, sva_groups.cu: every group's derived parameters are checked before anything is enqueued)
+int check_params(sva_ctx* c, const sva_params* p) {
     if (!p) return c->fail(SVA_ERR_BAD_ARG, "null params");
     if (p->width < 8 || p->height < 8) return c->fail(SVA_ERR_BAD_ARG, "image smaller than 8x8");
     if (p->num_disp < 8 || p->num_disp > 256 || p->num_disp % 8) return c->fail(SVA_ERR_BAD_ARG, "num_disp must be a multiple of 8 in 8..256");
@@ -72,10 +75,10 @@ int check_frame_args(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, c
     return SVA_OK;
 }
 
-extern "C" {
-
-int sva_frame_upload(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask) {
-    if (!c) return SVA_ERR_BAD_ARG;
+// The copy part of an upload: the views into the staging of the kernels that will read them, from host memory (view_kind =
+// cudaMemcpyHostToDevice) or from device memory (cudaMemcpyDeviceToDevice: an array frame's camera stack, sva_depth_groups); the mask is
+// always a host buffer.  In census mode with ctx->sig_stack set, K1a reads the stack's signatures and no view is staged.
+static int stage_frame(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask, cudaMemcpyKind view_kind) {
     NvtxRange range("sva:upload");
     SVA_CUDA_OK(c, cudaSetDevice(c->device));
     SVA_TRY(check_frame_args(c, p, ref, others, mask));
@@ -92,17 +95,17 @@ int sva_frame_upload(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, c
     const bool census = p->reserved[0] == SVA_COST_CENSUS;
     c->use_ad2 = sva_ad2_usable(*p) && !c->tune_ad_gather && !census;
     if (c->use_ad2) {
-        // image-space AD kernel: the views go straight from the host into zero-bordered, 16-byte-pitched device copies
+        // image-space AD kernel: the views go straight into zero-bordered, 16-byte-pitched device copies
         SVA_TRY(sva_ad2_prepare(c));
-        SVA_CUDA_OK(c, cudaMemcpy2DAsync(c->pad_ref.p, c->ad2.rp, ref->data, ref->step, W, H, cudaMemcpyHostToDevice, c->stream));
+        SVA_CUDA_OK(c, cudaMemcpy2DAsync(c->pad_ref.p, c->ad2.rp, ref->data, ref->step, W, H, view_kind, c->stream));
         for (int i = 0; i < p->n_pairs; i++)
-            SVA_CUDA_OK(c, cudaMemcpy2DAsync(sva_ad2_view_origin(c, i), c->ad2.pp, others[i].data, others[i].step, W, H, cudaMemcpyHostToDevice, c->stream));
-    } else {
+            SVA_CUDA_OK(c, cudaMemcpy2DAsync(sva_ad2_view_origin(c, i), c->ad2.pp, others[i].data, others[i].step, W, H, view_kind, c->stream));
+    } else if (!(census && c->sig_stack)) {
         SVA_TRY(c->reserve(c->ref_img, img));
         SVA_TRY(c->reserve(c->other_imgs, img * p->n_pairs));
-        SVA_CUDA_OK(c, cudaMemcpy2DAsync(c->ref_img.p, W, ref->data, ref->step, W, H, cudaMemcpyHostToDevice, c->stream));
+        SVA_CUDA_OK(c, cudaMemcpy2DAsync(c->ref_img.p, W, ref->data, ref->step, W, H, view_kind, c->stream));
         for (int i = 0; i < p->n_pairs; i++)
-            SVA_CUDA_OK(c, cudaMemcpy2DAsync(c->other_imgs.as<uint8_t>() + img * i, W, others[i].data, others[i].step, W, H, cudaMemcpyHostToDevice, c->stream));
+            SVA_CUDA_OK(c, cudaMemcpy2DAsync(c->other_imgs.as<uint8_t>() + img * i, W, others[i].data, others[i].step, W, H, view_kind, c->stream));
     }
     c->has_mask = mask != nullptr;
     if (mask) {
@@ -112,6 +115,13 @@ int sva_frame_upload(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, c
     if (!c->use_ad2 && !census) SVA_TRY(sva_build_line_images(c));
     c->have_frame = true;
     return SVA_OK;
+}
+
+extern "C" {
+
+int sva_frame_upload(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask) {
+    if (!c) return SVA_ERR_BAD_ARG;
+    return stage_frame(c, p, ref, others, mask, cudaMemcpyHostToDevice);
 }
 
 int sva_frame_set_pair_range(sva_ctx* c, int32_t b, int32_t e) {
@@ -438,17 +448,20 @@ int sva_frame_download_disparity_rows(sva_ctx* c, int32_t rows, uint16_t* out_di
     return SVA_OK;
 }
 
+}  // extern "C"
+
 /* ---- streaming form of sva_depth_from_array: a capture stream, two frames in flight ---------------------------------------------
  * submit(t) uploads frame t on a copy stream, runs the stages on the compute stream and downloads the maps on a second copy stream;
  * it returns at once.  Frame t+1's upload overlaps frame t's compute and frame t-1's download (two IoSets, swapped per frame).
  * The host buffers (inputs and outputs) must stay valid until sva_stream_wait(ticket) returns; pin them for real overlap. */
-static void swap_io(sva_ctx* c) {
+void sva_swap_io(sva_ctx* c) {
+    c->io_swapped = !c->io_swapped;
     std::swap(c->pad_ref, c->alt.pad_ref); std::swap(c->pad_imgs, c->alt.pad_imgs); std::swap(c->ref_img, c->alt.ref_img);
     std::swap(c->other_imgs, c->alt.other_imgs); std::swap(c->lines, c->alt.lines); std::swap(c->mask, c->alt.mask);
     std::swap(c->disp, c->alt.disp); std::swap(c->subpix, c->alt.subpix); std::swap(c->ad2_zero_key, c->alt.ad2_zero_key);
 }
 
-static int stream_open(sva_ctx* c) {
+int sva_stream_open(sva_ctx* c) {
     if (c->h2d_stream) return SVA_OK;
     SVA_CUDA_OK(c, cudaStreamCreateWithFlags(&c->h2d_stream, cudaStreamNonBlocking));
     SVA_CUDA_OK(c, cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking));
@@ -461,30 +474,29 @@ static int stream_open(sva_ctx* c) {
     return SVA_OK;
 }
 
-int sva_stream_submit(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
-                      uint16_t* out_disp, float* out_subpix, int64_t* out_ticket) {
-    if (!c || !out_disp || !out_ticket) return SVA_ERR_BAD_ARG;
-    SVA_CUDA_OK(c, cudaSetDevice(c->device));
-    SVA_TRY(stream_open(c));
+// wait for every frame in flight on the capture stream (their tickets stay waitable: their events have completed)
+int sva_stream_drain(sva_ctx* c) {
+    SVA_CUDA_OK(c, cudaStreamSynchronize(c->h2d_stream));
+    if (c->ad_stream) SVA_CUDA_OK(c, cudaStreamSynchronize(c->ad_stream));
+    SVA_CUDA_OK(c, cudaStreamSynchronize(c->stream));
+    SVA_CUDA_OK(c, cudaStreamSynchronize(c->d2h_stream));
+    c->ev_box_valid = false;
+    return SVA_OK;
+}
+
+// The capture-stream pipeline behind sva_stream_submit, for a checked frame whose geometry matches the frames in flight (or with none in
+// flight).  view_kind says where the views live (stage_frame); sva_depth_groups runs its groups through here with the views in its stack.
+int sva_stream_enqueue(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
+                       cudaMemcpyKind view_kind, uint16_t* out_disp, float* out_subpix, int64_t* out_ticket) {
     const int64_t t = c->stream_ticket;
     const int slot = (int)(t & 1);
-    if (t > 0 && p && (p->width != c->prm.width || p->height != c->prm.height || p->num_disp != c->prm.num_disp || p->n_pairs != c->prm.n_pairs ||
-                       p->win_half != c->prm.win_half || p->min_disp != c->prm.min_disp || p->reserved[0] != c->prm.reserved[0])) {
-        // a different geometry re-allocates workspaces: drain the pipeline first so no frame in flight still uses the old ones
-        SVA_CUDA_OK(c, cudaStreamSynchronize(c->h2d_stream));
-        if (c->ad_stream) SVA_CUDA_OK(c, cudaStreamSynchronize(c->ad_stream));
-        SVA_CUDA_OK(c, cudaStreamSynchronize(c->stream));
-        SVA_CUDA_OK(c, cudaStreamSynchronize(c->d2h_stream));
-        c->ev_box_valid = false;
-    }
-    SVA_TRY(check_frame_args(c, p, ref, others, mask));  // a bad frame must not disturb the frames in flight: nothing is touched before this
     if (t >= 2) SVA_CUDA_OK(c, cudaEventSynchronize(c->ev_done[slot]));  // frame t-2 is out: its IoSet is free again
-    swap_io(c);
+    sva_swap_io(c);
     cudaStream_t compute = c->stream;
     c->stream = c->h2d_stream;
-    int rc = sva_frame_upload(c, p, ref, others, mask);
+    int rc = stage_frame(c, p, ref, others, mask, view_kind);
     c->stream = compute;
-    if (rc != SVA_OK) { swap_io(c); return rc; }  // (allocation failure): back onto the IoSet of frame t-1, the ticket is not consumed
+    if (rc != SVA_OK) { sva_swap_io(c); return rc; }  // (allocation failure): back onto the IoSet of frame t-1, the ticket is not consumed
     SVA_CUDA_OK(c, cudaEventRecord(c->ev_h2d[slot], c->h2d_stream));
     // (only where the SGM launches are not paced — c1-sized rows: next to paced launches the intruder costs more than it hides: c2 e2e 1.67 -> 1.76 ms)
     if (c->tune_stream_ad_ahead && c->win_rows == 0 && (c->tune_stream_ad_ahead > 1 || (size_t)p->width * p->num_disp * 4 < 768 * 1024)) {
@@ -531,6 +543,21 @@ int sva_stream_submit(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, 
     return SVA_OK;
 }
 
+extern "C" {
+
+int sva_stream_submit(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
+                      uint16_t* out_disp, float* out_subpix, int64_t* out_ticket) {
+    if (!c || !out_disp || !out_ticket) return SVA_ERR_BAD_ARG;
+    SVA_CUDA_OK(c, cudaSetDevice(c->device));
+    SVA_TRY(sva_stream_open(c));
+    if (c->stream_ticket > 0 && p && (p->width != c->prm.width || p->height != c->prm.height || p->num_disp != c->prm.num_disp || p->n_pairs != c->prm.n_pairs ||
+                       p->win_half != c->prm.win_half || p->min_disp != c->prm.min_disp || p->reserved[0] != c->prm.reserved[0])) {
+        SVA_TRY(sva_stream_drain(c));  // a different geometry re-allocates workspaces: no frame in flight may still use the old ones
+    }
+    SVA_TRY(check_frame_args(c, p, ref, others, mask));  // a bad frame must not disturb the frames in flight: nothing is touched before this
+    return sva_stream_enqueue(c, p, ref, others, mask, cudaMemcpyHostToDevice, out_disp, out_subpix, out_ticket);
+}
+
 int sva_stream_wait(sva_ctx* c, int64_t ticket) {
     if (!c || !c->h2d_stream) return SVA_ERR_BAD_ARG;
     if (ticket < 0 || ticket >= c->stream_ticket) return c->fail(SVA_ERR_BAD_ARG, "unknown ticket");
@@ -545,7 +572,7 @@ int sva_stream_wait(sva_ctx* c, int64_t ticket) {
 int sva_stream_mark(sva_ctx* c) {
     if (!c) return SVA_ERR_BAD_ARG;
     SVA_CUDA_OK(c, cudaSetDevice(c->device));
-    SVA_TRY(stream_open(c));
+    SVA_TRY(sva_stream_open(c));
     SVA_CUDA_OK(c, cudaStreamSynchronize(c->stream));
     SVA_CUDA_OK(c, cudaStreamSynchronize(c->d2h_stream));
     SVA_CUDA_OK(c, cudaEventRecord(c->ev_mark, c->h2d_stream));

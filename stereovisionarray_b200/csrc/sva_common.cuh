@@ -83,6 +83,13 @@ struct sva_ctx {
     int tune_stream_ad_ahead = 1;       // SVA_STREAM_AD_AHEAD
     cudaEvent_t ev_h2d[2] = {nullptr, nullptr}, ev_compute[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr}, ev_mark = nullptr;
     IoSet alt;                 // the set not in use by the frame being submitted
+    bool io_swapped = false;   // toggled by every swap of the two IoSets: which physical set is the current one
+    // ---- array frames (sva_depth_groups, sva_groups.cu) ----
+    cudaStream_t stack_stream = nullptr;  // uploads the frame's cameras into cam_stack (census: and computes their signatures into cam_sig)
+    std::vector<cudaEvent_t> ev_cam;      // one per camera: its view (census: its signatures) is in the stack
+    const uint64_t* sig_stack = nullptr;  // census: K1a reads these signatures instead of transforming the staged views (sva_run_ad_census)
+    int sig_ref = 0;                      //   camera of the reference view in sig_stack
+    int sig_view[SVA_MAX_PAIRS] = {};     //   camera of each pair's other view
     int64_t stream_ticket = 0; // next ticket
     std::string err;
     uint64_t launches = 0;
@@ -121,6 +128,7 @@ struct sva_ctx {
     PairGeom geom[SVA_MAX_PAIRS];
     DevBuf ref_img, other_imgs, lines, mask, A, AP, C, Craw, S, disp, subpix, other_d, scratch, scratch2, pace_buf;
     DevBuf pad_imgs, pad_ref, comm_scratch, census, tex_img, sgm_state;
+    DevBuf cam_stack, cam_sig;   // an array frame's cameras, tight W x H each, and their census signatures (sva_depth_groups)
     unsigned long long tex = 0;  // cudaTextureObject_t over tex_img (K0's source view, k_misc.cu)
     uint64_t tex_key = 0;
     // ---- multi-GPU (sva_dist.cu) ----

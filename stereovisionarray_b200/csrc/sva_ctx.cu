@@ -29,7 +29,7 @@ void sva_ctx::release(DevBuf& b) {
 }
 
 void sva_ctx::device_bufs(std::vector<DevBuf*>& out) {
-    out = {&ref_img, &other_imgs, &lines, &mask, &A, &AP, &pad_imgs, &pad_ref, &C, &Craw, &S, &disp, &subpix, &other_d, &scratch, &scratch2, &pace_buf, &comm_scratch, &census, &tex_img, &sgm_state,
+    out = {&ref_img, &other_imgs, &lines, &mask, &A, &AP, &pad_imgs, &pad_ref, &C, &Craw, &S, &disp, &subpix, &other_d, &scratch, &scratch2, &pace_buf, &comm_scratch, &census, &tex_img, &sgm_state, &cam_stack, &cam_sig,
            &alt.pad_ref, &alt.pad_imgs, &alt.ref_img, &alt.other_imgs, &alt.lines, &alt.mask, &alt.disp, &alt.subpix};
 }
 
@@ -168,6 +168,7 @@ int sva_destroy(sva_ctx* c) {
     if (c->aux_stream) cudaStreamSynchronize(c->aux_stream);
     if (c->h2d_stream) { cudaStreamSynchronize(c->h2d_stream); cudaStreamSynchronize(c->d2h_stream); }
     if (c->ad_stream) cudaStreamSynchronize(c->ad_stream);
+    if (c->stack_stream) cudaStreamSynchronize(c->stack_stream);
     std::vector<DevBuf*> bufs;
     c->device_bufs(bufs);
     for (DevBuf* b : bufs) c->release(*b);
@@ -180,6 +181,8 @@ int sva_destroy(sva_ctx* c) {
     if (c->aux_stream) { cudaStreamDestroy(c->aux_stream); cudaEventDestroy(c->ev_fork); }
     if (c->ev_zero) cudaEventDestroy(c->ev_zero);
     if (c->ad_stream) { cudaStreamDestroy(c->ad_stream); cudaEventDestroy(c->ev_ad); cudaEventDestroy(c->ev_box); }
+    if (c->stack_stream) cudaStreamDestroy(c->stack_stream);
+    for (cudaEvent_t e : c->ev_cam) cudaEventDestroy(e);
     cudaStreamDestroy(c->own_stream);
     delete c;
     return SVA_OK;

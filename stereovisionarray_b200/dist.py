@@ -396,3 +396,39 @@ def rows_direct_stream(ctxs, rank, world, frames, upload=None, download=None):
 def numpy_pack(a_u16):
     """[H][W][D] u16 (D even) -> int32 view, the layout the GPU path reduces"""
     return np.ascontiguousarray(a_u16).view(np.int32)
+
+
+def groups_sharded_depth(ctx, p, images, groups, grid_cols, rank, world, group=None):
+    """Every reference view of one array frame (sva_depth_groups), the groups sharded over `world` GPUs: rank r computes the groups
+    frame_range(n_groups, world, r) (13 CHESS groups on 8 ranks: 2,2,2,2,2,1,1,1) and passes only the cameras they read, so nothing crosses
+    GPUs on the data path.  The maps are gathered on rank 0 -> (disp (G, H, W) uint16, subpix (G, H, W) float32) there, None elsewhere.
+    Collective (the gather)."""
+    from . import groups as _groups
+    groups = _groups.as_groups(groups)
+    b, e = frame_range(len(groups), world, rank)
+    mine = set(_groups.cameras_of(groups[b:e]))
+    d, s = ctx.depth_groups(p, [im if i in mine else None for i, im in enumerate(images)], groups, grid_cols, group_range=(b, e))
+    return gather_groups(d, s, p, len(groups), rank, world, group)
+
+
+def gather_groups(d, s, p, n_groups, rank, world, group=None):
+    """this rank's maps of its groups (frame_range) -> all groups' maps on rank 0, None elsewhere.  Collective."""
+    import torch
+    import torch.distributed as dist
+    if world == 1:
+        return d, s
+    per = frame_range(n_groups, world, 0)[1]  # the largest share
+    d_t = torch.zeros((per, p.height, p.width), dtype=torch.int32)
+    s_t = torch.zeros((per, p.height, p.width), dtype=torch.float32)
+    d_t[:d.shape[0]] = torch.from_numpy(d.astype(np.int32))
+    s_t[:d.shape[0]] = torch.from_numpy(s)
+    d_all = [torch.empty_like(d_t, device="cuda") for _ in range(world)] if rank == 0 else None
+    s_all = [torch.empty_like(s_t, device="cuda") for _ in range(world)] if rank == 0 else None
+    dist.gather(d_t.cuda(), d_all, dst=0, group=group)
+    dist.gather(s_t.cuda(), s_all, dst=0, group=group)
+    if rank != 0:
+        return None
+    counts = [frame_range(n_groups, world, r)[1] - frame_range(n_groups, world, r)[0] for r in range(world)]
+    disp = torch.cat([t[:n] for t, n in zip(d_all, counts)]).cpu().numpy().astype(np.uint16)
+    sub = torch.cat([t[:n] for t, n in zip(s_all, counts)]).cpu().numpy()
+    return disp, sub

@@ -7,6 +7,7 @@ import ctypes as C
 import numpy as np
 
 from . import abi
+from . import groups as _groups
 from ._lib import SvaError, check, lib
 
 
@@ -282,6 +283,48 @@ class DepthContext:
         check(self._h, self._L.sva_depth_from_array(self._h, C.byref(p), C.byref(r), o, C.byref(m) if m is not None else None,
                                                      _p(disp, C.c_uint16), _p(sub, C.c_float)))
         self.params = p
+        return disp, sub
+
+    # ---- every reference view of one array frame (getGroups, SURVEY §8 f3) ----
+    def depth_groups(self, p, images, groups, grid_cols, masks=None, group_range=None, disp=None, sub=None):
+        """The depth maps of the groups [begin, end) = group_range (default: all) of one array frame in one call (sva_depth_groups).
+        images: one 2-D uint8 array per camera of a grid of grid_cols columns, or None for a camera no group of the range reads; groups: what
+        reference_api.getGroups or oracle.get_groups return; p: template parameters with no pairs; masks: None, or one per group of the range
+        (None: no mask).  -> (disp (G, H, W) uint16, subpix (G, H, W) float32), G = end - begin, written into disp / sub when given (C-contiguous;
+        pinned memory lets each map's download overlap the groups after it).  ValueError for what the library refuses."""
+        groups = _groups.as_groups(groups)
+        begin, end = _groups.validate(p, groups, grid_cols, [None if im is None else im.shape for im in images], group_range,
+                                      None if masks is None else [None if m is None else m.shape for m in masks])
+        for a, dt in ((disp, np.uint16), (sub, np.float32)):
+            if a is not None and (a.dtype != dt or a.shape != (end - begin, p.height, p.width) or not a.flags.c_contiguous):
+                raise ValueError("output must be a C-contiguous (%d, %d, %d) %s array" % (end - begin, p.height, p.width, np.dtype(dt).name))
+        return self.depth_groups_unchecked(p, images, groups, grid_cols, masks, (begin, end), disp, sub)
+
+    def depth_groups_unchecked(self, p, images, groups, grid_cols, masks, group_range, disp=None, sub=None):
+        """depth_groups without the Python-side validation: the library's own refusals raise SvaError"""
+        begin, end = group_range
+        n = max(0, end - begin)
+        keep = [None if im is None else np.ascontiguousarray(im, dtype=np.uint8) for im in images]
+        ims = (abi.SvaImageU8 * max(1, len(keep)))()
+        for i, a in enumerate(keep):
+            if a is not None:
+                ims[i] = abi.SvaImageU8(a.ctypes.data, a.shape[0], a.shape[1], a.strides[0])
+        flat = np.array([v for g in groups for pr in g for v in pr] or [0], np.int32)
+        sizes = np.array([len(g) for g in groups] or [0], np.int32)
+        mk, m_arr = [], None
+        if masks is not None:
+            m_arr = (abi.SvaImageU8 * max(1, n))()
+            for i, m in enumerate(masks):
+                if m is not None:
+                    a = np.ascontiguousarray(m, dtype=np.uint8)
+                    mk.append(a)
+                    m_arr[i] = abi.SvaImageU8(a.ctypes.data, a.shape[0], a.shape[1], a.strides[0])
+        disp = np.empty((n, p.height, p.width), np.uint16) if disp is None else disp
+        sub = np.empty((n, p.height, p.width), np.float32) if sub is None else sub
+        d_ptr = (C.c_void_p * max(1, n))(*[disp[i].ctypes.data for i in range(n)])
+        s_ptr = (C.c_void_p * max(1, n))(*[sub[i].ctypes.data for i in range(n)])
+        check(self._h, self._L.sva_depth_groups(self._h, C.byref(p), int(grid_cols), ims, len(keep), flat.ctypes.data, sizes.ctypes.data, len(groups),
+                                                 int(begin), int(end), m_arr, d_ptr, s_ptr))
         return disp, sub
 
     # ---- capture stream: two frames in flight (upload of t+1 | kernels of t | download of t-1) ----

@@ -120,3 +120,38 @@ def make_depth_scene(h, w, seed=0):
     d[rng.random((h, w)) < 0.03] = 0.0
     d[:2, :] = 0.3  # below shiftPerspective2's 0.5 threshold but above DepthMapToPoints3D's 0.1
     return d
+
+
+# ---- one scene seen by every camera of an array (multi-reference groups, sva_depth_groups) ----
+def make_array_scene(h, w, grid_rows, grid_cols, num_disp, seed, min_disp=0):
+    """Fronto-parallel textured layers at integer disparities, rendered consistently into every camera of a grid_rows x grid_cols array.
+    Pixel (x, y) of camera (c, r) (index r * grid_cols + c) shows layer l's texture at (x + c * delta_l, y + r * delta_l) of the layer's
+    reference plane; of the layers whose support covers that point the nearest (largest delta) wins.  So a texture point at (u, v) appears in
+    camera (c, r) at (u - c * delta, v - r * delta): seen from camera i, the match of (x, y) in camera j is (x - gx * delta, y - gy * delta)
+    with (gx, gy) = (col j - col i, row j - row i), the convention of configs.grid_offsets.
+    Layers: a background covering everything at min_disp + D/4 and three rectangles at min_disp + {D/2, 5D/8 + 1, 7D/8 - 2}, placed in the
+    centre camera's image.  -> dict(images[list of u8 (h, w)], gt[list of int32 (h, w)]: each camera's disparity, layers[list of delta])."""
+    D = num_disp
+    deltas = [min_disp + D // 4, min_disp + D // 2, min_disp + (5 * D) // 8 + 1, min_disp + (7 * D) // 8 - 2]
+    cm, rm = (grid_cols - 1) / 2.0, (grid_rows - 1) / 2.0
+    # supports in reference-plane coordinates (u0, v0, u1, v1): rectangles of the centre camera's image, shifted by its delta
+    rects = [None]
+    for (fx, fy, fw, fh), dl in zip([(0.10, 0.12, 0.34, 0.36), (0.52, 0.18, 0.32, 0.30), (0.30, 0.56, 0.30, 0.30)], deltas[1:]):
+        rects.append((fx * w + cm * dl, fy * h + rm * dl, (fx + fw) * w + cm * dl, (fy + fh) * h + rm * dl))
+    texs = []
+    for i, dl in enumerate(deltas):
+        texs.append(texture(h + (grid_rows - 1) * dl + 1, w + (grid_cols - 1) * dl + 1, seed * 16 + i))
+    yy, xx = np.mgrid[0:h, 0:w]
+    images, gts = [], []
+    for r in range(grid_rows):
+        for c in range(grid_cols):
+            img = np.zeros((h, w), np.uint8)
+            gt = np.zeros((h, w), np.int32)
+            for tex, dl, rc in zip(texs, deltas, rects):  # ascending delta: nearer layers overwrite
+                u, v = xx + c * dl, yy + r * dl
+                inside = np.ones((h, w), bool) if rc is None else (u >= rc[0]) & (u < rc[2]) & (v >= rc[1]) & (v < rc[3])
+                img[inside] = tex[v[inside], u[inside]]
+                gt[inside] = dl
+            images.append(img)
+            gts.append(gt)
+    return {"images": images, "gt": gts, "layers": deltas}
