@@ -18,6 +18,10 @@ std::vector<uint16_t> svaDepthPairSharded(const sva_params&, cv::Mat&, std::vect
 std::vector<uint16_t> svaDepthRowsSharded(const sva_params&, cv::Mat&, std::vector<cv::Mat>&, cv::Mat*, int, int, int*, int*, std::vector<float>*);
 std::vector<std::vector<uint16_t>> svaDepthGroups(const sva_params&, std::vector<cv::Mat>&, const std::vector<std::vector<std::array<int, 2>>>&, int,
                                                   const std::vector<cv::Mat>*, std::vector<std::vector<float>>*);
+std::vector<uint16_t> svaFuseMaps(int, int, int, int, const std::vector<int>&, const std::vector<std::vector<uint16_t>>&, const std::vector<std::vector<float>>*,
+                                  int, const sva_fuse_params&, const cv::Mat*, std::vector<float>*, std::vector<uint8_t>*);
+std::vector<uint16_t> svaDepthGroupsFused(const sva_params&, std::vector<cv::Mat>&, const std::vector<std::vector<std::array<int, 2>>>&, int, int,
+                                          const sva_fuse_params&, std::vector<float>*, std::vector<uint8_t>*, const std::vector<cv::Mat>*, const cv::Mat*);
 
 static cv::Mat g_mask;
 cv::Mat getFaceMask(cv::Mat&) { return g_mask.clone(); }
@@ -159,6 +163,46 @@ extern "C" int adapter_depth_groups(const sva_params* p, const uint8_t* const* i
             std::memcpy(out_disp + g * px, disp[g].data(), px * 2);
             std::memcpy(out_sub + g * px, sub[g].data(), px * 4);
         }
+        return (int)groups.size();
+    } catch (const std::exception& e) { g_err = e.what(); return -1; }
+}
+
+// the CHESS groups of a 5 x 5 frame fused into camera target's view, twice: svaDepthGroupsFused(p, images, getGroups(cameras, "CHESS"), 5,
+// target, f, &subpix, &support) into out_*[0 .. w * h), and svaDepthGroups followed by svaFuseMaps (sub-pixel maps iff p->subpixel) into
+// out_*[w * h .. 2 w * h).  target_mask: null or w x h.  Returns the number of groups.
+extern "C" int adapter_depth_groups_fused(const sva_params* p, const uint8_t* const* images25, int target, int tol_16, int min_support,
+                                          const uint8_t* target_mask, uint16_t* out_disp, float* out_sub, uint8_t* out_support) {
+    try {
+        const int w = p->width, h = p->height;
+        const size_t px = (size_t)w * h;
+        auto mat = [&](const uint8_t* src) { cv::Mat m(h, w, CV_8UC1); std::memcpy(m.data, src, px); return m; };
+        double f = 0.05, sensor_size = 0.036, pixelSize = sensor_size / w;
+        std::vector<Camera> cameras;
+        std::vector<cv::Mat> images;
+        for (int y = 0; y < 5; y++)
+            for (int x = 0; x < 5; x++) {
+                cameras.push_back(Camera(f, cv::Point3d{-0.1 + x * 0.05, -0.1 + y * 0.05, -0.75}, pixelSize));
+                images.push_back(mat(images25[5 * y + x]));
+            }
+        auto groups = getGroups(cameras, "CHESS");
+        sva_fuse_params fp{};
+        fp.tol_16 = tol_16;
+        fp.min_support = min_support;
+        cv::Mat tm = target_mask ? mat(target_mask) : cv::Mat();
+        std::vector<float> sub;
+        std::vector<uint8_t> sup;
+        std::vector<uint16_t> d = svaDepthGroupsFused(*p, images, groups, 5, target, fp, &sub, &sup, nullptr, &tm);
+        std::memcpy(out_disp, d.data(), px * 2);
+        std::memcpy(out_sub, sub.data(), px * 4);
+        std::memcpy(out_support, sup.data(), px);
+        std::vector<std::vector<float>> gsub;
+        std::vector<std::vector<uint16_t>> gdisp = svaDepthGroups(*p, images, groups, 5, nullptr, &gsub);
+        std::vector<int> refs;
+        for (auto& g : groups) refs.push_back(g[0][0]);
+        d = svaFuseMaps(w, h, 5, 25, refs, gdisp, p->subpixel == 1 ? &gsub : nullptr, target, fp, &tm, &sub, &sup);
+        std::memcpy(out_disp + px, d.data(), px * 2);
+        std::memcpy(out_sub + px, sub.data(), px * 4);
+        std::memcpy(out_support + px, sup.data(), px);
         return (int)groups.size();
     } catch (const std::exception& e) { g_err = e.what(); return -1; }
 }

@@ -196,6 +196,64 @@ std::vector<std::vector<uint16_t>> svaDepthGroups(const sva_params& p, std::vect
     return disp;
 }
 
+// ---- multi-view depth fusion (sva_fuse_maps, sva_depth_groups_fused; DESIGN §3 item 6; no reference counterpart) ----
+// The maps of views whose reference cameras are viewRefs (e.g. svaDepthGroups' outputs with each group's reference camera) fused into camera
+// target's view on a grid of gridCols columns and nCameras cameras; subpix: null (fuse the integer maps) or one per view; targetMask: null or
+// an empty Mat (no mask), or width x height.  -> the fused u16 map (SVA_DISP_INVALID where rejected); the sub-pixel map in *outSubpix and the
+// number of agreeing views per pixel in *outSupport when given.
+std::vector<uint16_t> svaFuseMaps(int width, int height, int gridCols, int nCameras, const std::vector<int>& viewRefs,
+                                  const std::vector<std::vector<uint16_t>>& disp, const std::vector<std::vector<float>>* subpix, int target,
+                                  const sva_fuse_params& f, const cv::Mat* targetMask, std::vector<float>* outSubpix, std::vector<uint8_t>* outSupport) {
+    const size_t px = (size_t)width * height;
+    if (viewRefs.size() != disp.size() || (subpix && subpix->size() != disp.size())) throw cv::Exception("svaFuseMaps: one reference (and map) per view");
+    std::vector<const uint16_t*> dp;
+    std::vector<const float*> sp;
+    for (size_t g = 0; g < disp.size(); g++) {
+        if (disp[g].size() != px || (subpix && (*subpix)[g].size() != px)) throw cv::Exception("svaFuseMaps: a map is not width x height");
+        dp.push_back(disp[g].data());
+        if (subpix) sp.push_back((*subpix)[g].data());
+    }
+    std::vector<int32_t> refs(viewRefs.begin(), viewRefs.end());
+    std::vector<uint16_t> out(px);
+    std::vector<float> sub(px);
+    std::vector<uint8_t> sup(px);
+    const bool masked = targetMask && !targetMask->empty();
+    const sva_image_u8 mk = masked ? view(*targetMask) : sva_image_u8{};
+    check(sva_fuse_maps(ctx(), width, height, gridCols, nCameras, refs.data(), (int32_t)refs.size(), dp.data(), subpix ? sp.data() : nullptr, target, &f,
+                        masked ? &mk : nullptr, out.data(), sub.data(), sup.data()), "svaFuseMaps");
+    if (outSubpix) *outSubpix = std::move(sub);
+    if (outSupport) *outSupport = std::move(sup);
+    return out;
+}
+
+// Every group of one array frame (as svaDepthGroups computes them), fused into camera target's view in one call: the group maps never leave
+// the GPU.  The sub-pixel maps are fused iff p.subpixel == 1.  Equal to svaDepthGroups followed by svaFuseMaps with each group's reference.
+std::vector<uint16_t> svaDepthGroupsFused(const sva_params& p, std::vector<cv::Mat>& images, const std::vector<std::vector<std::array<int, 2>>>& groups,
+                                          int gridCols, int target, const sva_fuse_params& f, std::vector<float>* subpix, std::vector<uint8_t>* support,
+                                          const std::vector<cv::Mat>* masks, const cv::Mat* targetMask) {
+    if (masks && masks->size() != groups.size()) throw cv::Exception("svaDepthGroupsFused: one mask (or an empty Mat) per group");
+    std::vector<sva_image_u8> ims, mk;
+    for (auto& m : images) ims.push_back(m.empty() ? sva_image_u8{} : view(m));
+    if (masks) for (auto& m : *masks) mk.push_back(m.empty() ? sva_image_u8{} : view(m));
+    std::vector<int32_t> pairs, sizes;
+    for (auto& g : groups) {
+        sizes.push_back((int32_t)g.size());
+        for (auto& pr : g) { pairs.push_back(pr[0]); pairs.push_back(pr[1]); }
+    }
+    const size_t px = (size_t)p.width * p.height;
+    std::vector<uint16_t> out(px);
+    std::vector<float> sub(px);
+    std::vector<uint8_t> sup(px);
+    const bool masked = targetMask && !targetMask->empty();
+    const sva_image_u8 tm = masked ? view(*targetMask) : sva_image_u8{};
+    check(sva_depth_groups_fused(ctx(), &p, gridCols, ims.data(), (int32_t)ims.size(), pairs.data(), sizes.data(), (int32_t)groups.size(),
+                                 masks ? mk.data() : nullptr, target, &f, masked ? &tm : nullptr, out.data(), sub.data(), sup.data()),
+          "svaDepthGroupsFused");
+    if (subpix) *subpix = std::move(sub);
+    if (support) *support = std::move(sup);
+    return out;
+}
+
 // ---- one frame over several GPUs (one process per GPU; any launcher — mpirun, torchrun, a shell loop — provides rank and world) ----
 // No reference counterpart (the reference is one thread): the sharding units are its pair loop (src/CameraStereoVision.cpp:55) and its
 // pixel-row loop (:49).  Rank 0 calls svaCommUniqueId() and hands the 128 bytes to the others by whatever channel the launcher offers;

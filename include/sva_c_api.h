@@ -202,6 +202,43 @@ int sva_depth_groups(sva_ctx* ctx, const sva_params* p, int32_t grid_cols, const
                      const int32_t* sizes, int32_t n_groups, int32_t group_begin, int32_t group_end, const sva_image_u8* masks,
                      uint16_t* const* out_disp, float* const* out_subpix);
 
+/* ---- multi-view depth fusion (DESIGN.md §3 item 6): the maps of several reference views of one array frame merged into one camera's view ----
+ * No reference counterpart (shiftPerspective2 warps f64 metric depth with "last writer wins"); spec frozen in tests/fuse_oracle.c
+ * (orc_fuse_views), parity unpinned by the reference.  Everything after the fixed-point step is integer: the result is bit-exact and does not
+ * depend on the order of the views.
+ *  1. pixel (x, y) of view g is used iff disp != SVA_DISP_INVALID and, with sub-pixel maps, 0 <= subpix < 4352; q = 16 * disp, or with
+ *     sub-pixel maps q = rint(16 * subpix) (ties to even), in 1/16 px;
+ *  2. it lands on x' = x - ((gx * q + 8) >> 4), y' = y - ((gy * q + 8) >> 4) of the target, (gx, gy) = (col t - col r_g, row t - row r_g),
+ *     >> an arithmetic (floor) shift; outside the image it is dropped;
+ *  3. per view and target pixel the largest q that lands there wins (the nearest surface);
+ *  4. among the views' candidates c_h at a pixel, c* has the largest support #{h : |c_h - c*| <= tol_16} (ties: the larger value);
+ *     M = {h : |c_h - c*| <= tol_16}, n* = |M|, q^ = (sum_M c_h + n* / 2) / n*;
+ *  5. rejected (no candidate, n* < min_support, or target mask 0): disp = SVA_DISP_INVALID, subpix = -1; accepted: disp = (q^ + 8) >> 4,
+ *     subpix = q^ / 16.  support = n* everywhere (0 without a candidate). */
+typedef struct sva_fuse_params {
+    int32_t tol_16;       /* candidates within tol_16 / 16 px agree; 0..4095 */
+    int32_t min_support;  /* views that must agree for a pixel to be accepted; 1..n_views */
+    int32_t reserved[6];  /* must be 0 */
+} sva_fuse_params;
+/* The maps in host memory (e.g. sva_depth_groups' outputs, or maps gathered from the ranks of a sharded frame): disp[g] (and subpix[g] when
+ * subpix is not NULL) width x height of the view whose reference camera is view_refs[g], on a grid of grid_cols columns; target: the camera
+ * whose view the result is in; target_mask: NULL or width x height (0 = reject).  out_subpix and out_support (u8) may be NULL.  Synchronous.
+ * SVA_ERR_BAD_ARG, with nothing enqueued: n_views outside 1..32, a reference or the target outside [0, n_cameras), n_cameras not a positive
+ * multiple of grid_cols, tol_16 outside 0..4095, min_support outside 1..n_views, non-zero reserved fields, a null map or output, a size below
+ * 1 x 1, a mask of the wrong size. */
+int sva_fuse_maps(sva_ctx* ctx, int32_t width, int32_t height, int32_t grid_cols, int32_t n_cameras, const int32_t* view_refs, int32_t n_views,
+                  const uint16_t* const* disp, const float* const* subpix, int32_t target, const sva_fuse_params* f,
+                  const sva_image_u8* target_mask, uint16_t* out_disp, float* out_subpix, uint8_t* out_support);
+/* Every group of the frame (sva_depth_groups over [0, n_groups)), then their fusion into camera target, in one call: each group's maps are
+ * warped into the target's view on the device right after its K3 and never leave it; the fused maps are the only download.  The views are the
+ * groups (view_refs = each group's reference camera, n_cameras = n_images); the sub-pixel maps are used iff p->subpixel == 1.  The result
+ * equals sva_depth_groups followed by sva_fuse_maps on its outputs bit for bit.  SVA_ERR_BAD_ARG, with nothing enqueued: every refusal of
+ * both calls. */
+int sva_depth_groups_fused(sva_ctx* ctx, const sva_params* p, int32_t grid_cols, const sva_image_u8* images, int32_t n_images,
+                           const int32_t* pairs, const int32_t* sizes, int32_t n_groups, const sva_image_u8* masks, int32_t target,
+                           const sva_fuse_params* f, const sva_image_u8* target_mask, uint16_t* out_disp, float* out_subpix,
+                           uint8_t* out_support);
+
 /* ---- staged, device-resident form of the same pipeline (what bench.py times with inputs already in HBM) ------- */
 typedef enum sva_stage {
     SVA_STAGE_AD = 1,        /* K1a: A(y,x,d) = sum_k |R - I_k(shifted)|            -> u16 [H][W][D] */

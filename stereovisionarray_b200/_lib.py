@@ -27,7 +27,7 @@ EXPORTS = [
     "sva_rows_open", "sva_rows_export", "sva_rows_connect", "sva_rows_connect_comm", "sva_rows_connect_local", "sva_rows_block", "sva_rows_run", "sva_rows_run_phase", "sva_rows_run_part", "sva_get_stream",
     "sva_rows_download", "sva_rows_close", "sva_depth_rows_sharded",
     "sva_rows_stream_create", "sva_rows_stream_connect_comm", "sva_rows_stream_submit", "sva_rows_stream_flush", "sva_rows_stream_wait",
-    "sva_rows_stream_destroy", "sva_depth_groups",
+    "sva_rows_stream_destroy", "sva_depth_groups", "sva_fuse_maps", "sva_depth_groups_fused",
 ]
 
 _lib = None
@@ -76,6 +76,10 @@ def lib():
             getattr(L, n).argtypes = [C.c_void_p]
         L.sva_depth_groups.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                        C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sva_fuse_maps.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sva_depth_groups_fused.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                             C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         missing = [n for n in EXPORTS if not hasattr(L, n)]
         if missing:
             raise ImportError("libsva_b200.so does not export %s — rebuild it" % missing)

@@ -47,6 +47,11 @@ class SvaParams(C.Structure):
     ]
 
 
+class SvaFuseParams(C.Structure):
+    """sva_fuse_params: candidates within tol_16 / 16 px agree; min_support views must agree (DESIGN §3 item 6)"""
+    _fields_ = [("tol_16", C.c_int32), ("min_support", C.c_int32), ("reserved", C.c_int32 * 6)]
+
+
 def make_params(width, height, num_disp, pairs, win_half=20, min_disp=0, cost_shift=None, cost_cap=SVA_COST_CAP_MAX,
                 p1=None, p2=None, n_paths=8, lr_gx=0, lr_max_diff=1, subpixel=1, cost_mode=COST_SAD):
     """pairs: list of (gx, gy) grid offsets of the other cameras.  Defaults follow SURVEY §8(d):

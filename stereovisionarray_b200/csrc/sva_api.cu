@@ -486,6 +486,7 @@ int sva_stream_drain(sva_ctx* c) {
 
 // The capture-stream pipeline behind sva_stream_submit, for a checked frame whose geometry matches the frames in flight (or with none in
 // flight).  view_kind says where the views live (stage_frame); sva_depth_groups runs its groups through here with the views in its stack.
+// out_disp may be NULL only here, not in sva_stream_submit: the maps are then not downloaded (see below).
 int sva_stream_enqueue(sva_ctx* c, const sva_params* p, const sva_image_u8* ref, const sva_image_u8* others, const sva_image_u8* mask,
                        cudaMemcpyKind view_kind, uint16_t* out_disp, float* out_subpix, int64_t* out_ticket) {
     const int64_t t = c->stream_ticket;
@@ -535,8 +536,10 @@ int sva_stream_enqueue(sva_ctx* c, const sva_params* p, const sva_image_u8* ref,
     SVA_CUDA_OK(c, cudaEventRecord(c->ev_compute[slot], compute));
     SVA_CUDA_OK(c, cudaStreamWaitEvent(c->d2h_stream, c->ev_compute[slot], 0));
     const size_t px = (size_t)p->width * p->height;
-    SVA_CUDA_OK(c, cudaMemcpyAsync(out_disp, c->disp.p, px * 2, cudaMemcpyDeviceToHost, c->d2h_stream));
-    if (out_subpix) SVA_CUDA_OK(c, cudaMemcpyAsync(out_subpix, c->subpix.p, px * 4, cudaMemcpyDeviceToHost, c->d2h_stream));
+    // out_disp == NULL (sva_depth_groups_fused): no download.  The maps stay in this frame's IoSet; work the caller enqueues on the compute
+    // stream after this call reads them before K3 of frame t + 2, the next writer of that IoSet's maps.
+    if (out_disp) SVA_CUDA_OK(c, cudaMemcpyAsync(out_disp, c->disp.p, px * 2, cudaMemcpyDeviceToHost, c->d2h_stream));
+    if (out_disp && out_subpix) SVA_CUDA_OK(c, cudaMemcpyAsync(out_subpix, c->subpix.p, px * 4, cudaMemcpyDeviceToHost, c->d2h_stream));
     SVA_CUDA_OK(c, cudaEventRecord(c->ev_done[slot], c->d2h_stream));
     c->stream_ticket = t + 1;
     *out_ticket = t;

@@ -129,6 +129,7 @@ struct sva_ctx {
     DevBuf ref_img, other_imgs, lines, mask, A, AP, C, Craw, S, disp, subpix, other_d, scratch, scratch2, pace_buf;
     DevBuf pad_imgs, pad_ref, comm_scratch, census, tex_img, sgm_state;
     DevBuf cam_stack, cam_sig;   // an array frame's cameras, tight W x H each, and their census signatures (sva_depth_groups)
+    DevBuf fuse_planes, fuse_in, fuse_mask, fuse_out;  // depth fusion (k_fuse.cu): per-view z-buffers, host maps, target mask, outputs
     unsigned long long tex = 0;  // cudaTextureObject_t over tex_img (K0's source view, k_misc.cu)
     uint64_t tex_key = 0;
     // ---- multi-GPU (sva_dist.cu) ----

@@ -30,6 +30,7 @@ void sva_ctx::release(DevBuf& b) {
 
 void sva_ctx::device_bufs(std::vector<DevBuf*>& out) {
     out = {&ref_img, &other_imgs, &lines, &mask, &A, &AP, &pad_imgs, &pad_ref, &C, &Craw, &S, &disp, &subpix, &other_d, &scratch, &scratch2, &pace_buf, &comm_scratch, &census, &tex_img, &sgm_state, &cam_stack, &cam_sig,
+           &fuse_planes, &fuse_in, &fuse_mask, &fuse_out,
            &alt.pad_ref, &alt.pad_imgs, &alt.ref_img, &alt.other_imgs, &alt.lines, &alt.mask, &alt.disp, &alt.subpix};
 }
 

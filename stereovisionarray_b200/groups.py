@@ -1,6 +1,6 @@
-"""Host logic of the multi-reference call sva_depth_groups (getGroups, SURVEY §8 f3): grid offsets of a group's pairs, the flattened layout
-the C ABI takes, and the refusal rules, checked here before the library is called so that a caller gets a ValueError naming the problem.
-Pure Python: no library, no GPU."""
+"""Host logic of the multi-reference calls sva_depth_groups (getGroups, SURVEY §8 f3) and of the depth fusion (sva_fuse_maps,
+sva_depth_groups_fused): grid offsets of a group's pairs, the flattened layout the C ABI takes, and the refusal rules, checked here before the
+library is called so that a caller gets a ValueError naming the problem.  Pure Python: no library, no GPU."""
 from . import abi
 
 
@@ -101,3 +101,27 @@ def validate(p, groups, grid_cols, shapes, group_range=None, mask_shapes=None):
             if m is not None and tuple(m) != (p.height, p.width):
                 raise ValueError("mask of group %d is %r, not %dx%d" % (begin + i, tuple(m), p.height, p.width))
     return begin, end
+
+
+def validate_fuse(n_views, refs, grid_cols, n_cameras, target, tol_16, min_support, shape, mask_shape=None):
+    """Raise ValueError where sva_fuse_maps (and the fusion part of sva_depth_groups_fused) would return SVA_ERR_BAD_ARG.  shape: (rows, cols)
+    of the maps; mask_shape: None or the target mask's (rows, cols)."""
+    if not 1 <= n_views <= 32:
+        raise ValueError("%d views: fusion takes 1..32" % n_views)
+    if len(refs) != n_views:
+        raise ValueError("one reference camera per view")
+    if grid_cols < 1 or n_cameras < 1 or n_cameras % grid_cols:
+        raise ValueError("%d cameras are not a positive multiple of grid_cols = %d" % (n_cameras, grid_cols))
+    for g, r in enumerate(refs):
+        if not 0 <= r < n_cameras:
+            raise ValueError("reference %d of view %d outside [0, %d)" % (r, g, n_cameras))
+    if not 0 <= target < n_cameras:
+        raise ValueError("target %d outside [0, %d)" % (target, n_cameras))
+    if not 0 <= tol_16 <= 4095:
+        raise ValueError("tol_16 must be in 0..4095")
+    if not 1 <= min_support <= n_views:
+        raise ValueError("min_support must be in 1..%d" % n_views)
+    if min(shape) < 1:
+        raise ValueError("empty maps")
+    if mask_shape is not None and tuple(mask_shape) != tuple(shape):
+        raise ValueError("target mask is %r, not %r" % (tuple(mask_shape), tuple(shape)))

@@ -15,6 +15,32 @@ def _p(a, t):
     return a.ctypes.data_as(C.POINTER(t))
 
 
+def _groups_args(images, groups, masks, n_masks):
+    """the C layout of sva_depth_groups' frame arguments -> (images, flat pairs, sizes, masks or None, keepalive)"""
+    keep = [None if im is None else np.ascontiguousarray(im, dtype=np.uint8) for im in images]
+    ims = (abi.SvaImageU8 * max(1, len(keep)))()
+    for i, a in enumerate(keep):
+        if a is not None:
+            ims[i] = abi.SvaImageU8(a.ctypes.data, a.shape[0], a.shape[1], a.strides[0])
+    flat = np.array([v for g in groups for pr in g for v in pr] or [0], np.int32)
+    sizes = np.array([len(g) for g in groups] or [0], np.int32)
+    m_arr = None
+    if masks is not None:
+        m_arr = (abi.SvaImageU8 * max(1, n_masks))()
+        for i, m in enumerate(masks):
+            if m is not None:
+                a = np.ascontiguousarray(m, dtype=np.uint8)
+                keep.append(a)
+                m_arr[i] = abi.SvaImageU8(a.ctypes.data, a.shape[0], a.shape[1], a.strides[0])
+    return ims, flat, sizes, m_arr, keep
+
+
+def fuse_params(tol_16=16, min_support=2):
+    f = abi.SvaFuseParams()
+    f.tol_16, f.min_support = int(tol_16), int(min_support)
+    return f
+
+
 class DepthContext:
     def __init__(self, device=0):
         self._L = lib()
@@ -304,28 +330,66 @@ class DepthContext:
         """depth_groups without the Python-side validation: the library's own refusals raise SvaError"""
         begin, end = group_range
         n = max(0, end - begin)
-        keep = [None if im is None else np.ascontiguousarray(im, dtype=np.uint8) for im in images]
-        ims = (abi.SvaImageU8 * max(1, len(keep)))()
-        for i, a in enumerate(keep):
-            if a is not None:
-                ims[i] = abi.SvaImageU8(a.ctypes.data, a.shape[0], a.shape[1], a.strides[0])
-        flat = np.array([v for g in groups for pr in g for v in pr] or [0], np.int32)
-        sizes = np.array([len(g) for g in groups] or [0], np.int32)
-        mk, m_arr = [], None
-        if masks is not None:
-            m_arr = (abi.SvaImageU8 * max(1, n))()
-            for i, m in enumerate(masks):
-                if m is not None:
-                    a = np.ascontiguousarray(m, dtype=np.uint8)
-                    mk.append(a)
-                    m_arr[i] = abi.SvaImageU8(a.ctypes.data, a.shape[0], a.shape[1], a.strides[0])
+        ims, flat, sizes, m_arr, keep = _groups_args(images, groups, masks, n)
         disp = np.empty((n, p.height, p.width), np.uint16) if disp is None else disp
         sub = np.empty((n, p.height, p.width), np.float32) if sub is None else sub
         d_ptr = (C.c_void_p * max(1, n))(*[disp[i].ctypes.data for i in range(n)])
         s_ptr = (C.c_void_p * max(1, n))(*[sub[i].ctypes.data for i in range(n)])
-        check(self._h, self._L.sva_depth_groups(self._h, C.byref(p), int(grid_cols), ims, len(keep), flat.ctypes.data, sizes.ctypes.data, len(groups),
+        check(self._h, self._L.sva_depth_groups(self._h, C.byref(p), int(grid_cols), ims, len(images), flat.ctypes.data, sizes.ctypes.data, len(groups),
                                                  int(begin), int(end), m_arr, d_ptr, s_ptr))
         return disp, sub
+
+    # ---- multi-view depth fusion (DESIGN §3 item 6) ----
+    def fuse_maps(self, disp, sub, refs, grid_cols, n_cameras, target, tol_16=16, min_support=2, mask=None):
+        """The maps of several reference views of one array frame fused into camera target's view (sva_fuse_maps).  disp: (G, H, W) uint16
+        (e.g. depth_groups' output); sub: (G, H, W) float32, or None to fuse the integer maps; refs[g]: view g's reference camera on a grid of
+        grid_cols columns and n_cameras cameras; mask: None or (H, W) uint8 of the target (0 = reject).  -> (disp (H, W) uint16,
+        subpix (H, W) float32, support (H, W) uint8: how many views agree).  ValueError for what the library refuses."""
+        disp = np.asarray(disp)
+        if disp.ndim != 3 or disp.dtype != np.uint16:
+            raise ValueError("disp must be a (G, H, W) uint16 array")
+        if sub is not None and (np.shape(sub) != disp.shape or np.asarray(sub).dtype != np.float32):
+            raise ValueError("sub must be None or a float32 array of disp's shape")
+        _groups.validate_fuse(disp.shape[0], refs, grid_cols, n_cameras, target, tol_16, min_support, disp.shape[1:],
+                              None if mask is None else np.shape(mask))
+        return self.fuse_maps_unchecked(list(disp), None if sub is None else list(sub), refs, grid_cols, n_cameras, target,
+                                        fuse_params(tol_16, min_support), mask)
+
+    def fuse_maps_unchecked(self, disp, sub, refs, grid_cols, n_cameras, target, f, mask=None):
+        """fuse_maps without the Python-side validation: disp / sub are lists of (H, W) maps (None: a null pointer), f an abi.SvaFuseParams;
+        the library's own refusals raise SvaError"""
+        H, W = next(d.shape for d in disp if d is not None)
+        keep = [None if d is None else np.ascontiguousarray(d, dtype=np.uint16) for d in disp]
+        d_ptr = (C.c_void_p * max(1, len(keep)))(*[None if d is None else d.ctypes.data for d in keep])
+        s_keep = None if sub is None else [None if s is None else np.ascontiguousarray(s, dtype=np.float32) for s in sub]
+        s_ptr = None if sub is None else (C.c_void_p * max(1, len(s_keep)))(*[None if s is None else s.ctypes.data for s in s_keep])
+        refs = np.array(list(refs) or [0], np.int32)
+        m, mk = (None, None) if mask is None else abi.image_u8(np.ascontiguousarray(mask, dtype=np.uint8))
+        out = (np.empty((H, W), np.uint16), np.empty((H, W), np.float32), np.empty((H, W), np.uint8))
+        check(self._h, self._L.sva_fuse_maps(self._h, W, H, int(grid_cols), int(n_cameras), refs.ctypes.data, len(keep), d_ptr, s_ptr, int(target),
+                                              C.byref(f), None if m is None else C.byref(m), *[a.ctypes.data for a in out]))
+        return out
+
+    def depth_groups_fused(self, p, images, groups, grid_cols, target, tol_16=16, min_support=2, masks=None, target_mask=None):
+        """Every group of one array frame (as depth_groups computes them, masks one per group or None) fused into camera target's view in one
+        call (sva_depth_groups_fused): the group maps never leave the device.  The sub-pixel maps are fused iff p.subpixel == 1.  Equal to
+        fuse_maps(*depth_groups(...), refs=[g[0][0] for g in groups], ...) bit for bit.  -> (disp, subpix, support) as fuse_maps returns."""
+        groups = _groups.as_groups(groups)
+        _groups.validate(p, groups, grid_cols, [None if im is None else im.shape for im in images], None,
+                         None if masks is None else [None if m is None else m.shape for m in masks])
+        _groups.validate_fuse(len(groups), [g[0][0] for g in groups], grid_cols, len(images), target, tol_16, min_support, (p.height, p.width),
+                              None if target_mask is None else np.shape(target_mask))
+        return self.depth_groups_fused_unchecked(p, images, groups, grid_cols, target, fuse_params(tol_16, min_support), masks, target_mask)
+
+    def depth_groups_fused_unchecked(self, p, images, groups, grid_cols, target, f, masks=None, target_mask=None):
+        """depth_groups_fused without the Python-side validation (f: abi.SvaFuseParams): the library's own refusals raise SvaError"""
+        ims, flat, sizes, m_arr, keep = _groups_args(images, groups, masks, len(groups))
+        m, mk = (None, None) if target_mask is None else abi.image_u8(np.ascontiguousarray(target_mask, dtype=np.uint8))
+        out = (np.empty((p.height, p.width), np.uint16), np.empty((p.height, p.width), np.float32), np.empty((p.height, p.width), np.uint8))
+        check(self._h, self._L.sva_depth_groups_fused(self._h, C.byref(p), int(grid_cols), ims, len(images), flat.ctypes.data, sizes.ctypes.data,
+                                                       len(groups), m_arr, int(target), C.byref(f), None if m is None else C.byref(m),
+                                                       *[a.ctypes.data for a in out]))
+        return out
 
     # ---- capture stream: two frames in flight (upload of t+1 | kernels of t | download of t-1) ----
     def stream_submit(self, p, ref, others, mask, disp, sub):

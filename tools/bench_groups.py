@@ -4,10 +4,14 @@
     python tools/bench_groups.py [--steps K] [--warmup W] [--out FILE]
     python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_groups.py [--steps K] [--out FILE]
 
-One GPU: three arms in the same process, alternating round by round (so clock and thermal drift hit them alike):
+One GPU: five arms in the same process, alternating round by round (so clock and thermal drift hit them alike):
   (a) groups:   one sva_depth_groups call — 25 uploads, each group staged from the device stack, the groups pipelined;
   (b) separate: 13 synchronous sva_depth_from_array calls — 55 uploads;
-  (c) stream:   13 sva_stream_submit calls with host views, then waits for the last two tickets — 55 uploads, frames pipelined.
+  (c) stream:   13 sva_stream_submit calls with host views, then waits for the last two tickets — 55 uploads, frames pipelined;
+  (d) fused:    one sva_depth_groups_fused call into camera 12's view (tol 1 px, min_support 2): the group maps never leave the device;
+  (e) groups_then_fuse: (a), then sva_fuse_maps on its 13 host maps into the same view.
+After the timed rounds, the two fusion kernels (k_fuse_splat, k_fuse_consensus) are timed alone with torch.profiler over --steps
+sva_fuse_maps calls: the device time of each launch, from the CUDA activity trace.
 Several ranks: groups_sharded_depth, rank r computing the groups frame_range(13, N, r) from only the cameras they read; the slowest rank's
 compute and the gather of the maps to rank 0 are reported separately.
 Each figure is the median over --steps rounds of a host clock around work that ends with every map in host memory.  Rates: groups/s, and
@@ -79,6 +83,33 @@ params = [G.group_params(p, g, 5) for g in groups]
 gmde = NG * W * H * D / 1e9
 
 
+TARGET = 12  # the centre camera
+
+
+def fuse_kernel_times(fn, n):
+    """device time of the fusion kernels over n calls of fn, from torch.profiler's CUDA activity trace -> {kernel: {mean_us, launches}}"""
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(n):
+            fn()
+        torch.cuda.synchronize()
+    out = {}
+    for ev in prof.events():
+        for k in ("k_fuse_splat", "k_fuse_consensus"):
+            if k in ev.name and ev.device_type.name == "CUDA":
+                e = out.setdefault(k, {"total_us": 0.0, "launches": 0})
+                e["total_us"] += ev.device_time
+                e["launches"] += 1
+    for e in out.values():
+        e["mean_us"] = round(e["total_us"] / max(1, e["launches"]), 2)
+        e["total_us"] = round(e["total_us"], 1)
+    if set(out) != {"k_fuse_splat", "k_fuse_consensus"}:
+        return {"not_measured": "the profiler trace holds only %r of the two fusion kernels" % sorted(out)}
+    return out
+
+
 def timed(fn):
     barrier()
     t0 = time.perf_counter()
@@ -110,7 +141,16 @@ try:
             ctx.stream_wait(t[-2])
             ctx.stream_wait(t[-1])
 
-        arms = {"groups": arm_groups, "separate": arm_separate, "stream": arm_stream}
+        refs = [g[0][0] for g in groups]
+
+        def arm_fused():
+            ctx.depth_groups_fused(p, images, groups, 5, TARGET, 16, 2)
+
+        def arm_groups_then_fuse():
+            ctx.depth_groups(p, images, groups, 5, disp=g_disp, sub=g_sub)
+            ctx.fuse_maps(g_disp, g_sub, refs, 5, 25, TARGET, 16, 2)
+
+        arms = {"groups": arm_groups, "separate": arm_separate, "stream": arm_stream, "fused": arm_fused, "groups_then_fuse": arm_groups_then_fuse}
         for _ in range(args.warmup):
             for fn in arms.values():
                 fn()
@@ -124,9 +164,14 @@ try:
                       "ms_all_rounds": [round(t, 3) for t in times[k]]}
         res["arms"] = {"groups": "sva_depth_groups: 25 uploads, groups staged from the device stack and pipelined",
                        "separate": "13 synchronous sva_depth_from_array calls (55 uploads)",
-                       "stream": "13 sva_stream_submit calls with host views (55 uploads), then waits for the last two tickets"}
+                       "stream": "13 sva_stream_submit calls with host views (55 uploads), then waits for the last two tickets",
+                       "fused": "sva_depth_groups_fused into camera %d (tol_16 16, min_support 2): one fused map downloaded" % TARGET,
+                       "groups_then_fuse": "sva_depth_groups (13 maps downloaded), then sva_fuse_maps on them (13 maps uploaded again)"}
         res["groups_speedup_vs_stream"] = round(res["stream"]["ms_per_frame"] / res["groups"]["ms_per_frame"], 3)
         res["groups_speedup_vs_separate"] = round(res["separate"]["ms_per_frame"] / res["groups"]["ms_per_frame"], 3)
+        res["fused_minus_groups_ms"] = round(res["fused"]["ms_per_frame"] - res["groups"]["ms_per_frame"], 3)
+        res["fused_speedup_vs_groups_then_fuse"] = round(res["groups_then_fuse"]["ms_per_frame"] / res["fused"]["ms_per_frame"], 3)
+        res["fuse_kernels"] = fuse_kernel_times(lambda: ctx.fuse_maps(g_disp, g_sub, refs, 5, 25, TARGET, 16, 2), args.steps)
     else:
         b, e = sdist.frame_range(NG, world, rank)
         mine = set(G.cameras_of(groups[b:e]))
