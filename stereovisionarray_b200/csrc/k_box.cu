@@ -218,7 +218,6 @@ struct BoxPParams {
     int W, H, D, k, kk, dmin, shift, cap;
     int gxp, gxn, gyp, gyn;
     int band_rows, txo, wp;
-    int l2hint; // k_box_planar_shfl: 1 = entering rows evict_last, leaving rows and C evict_first
     int chunk;  // k_box_planar_shfl: warm-up rows summed per horizontal pass (chunk x the largest A keeps a 16-bit field below 32768)
     long long row_words;
     int ry0, ry1;  // output rows [ry0, ry1) (the whole image, or a row block)
@@ -429,10 +428,9 @@ k_box_planar_shfl(BoxPParams q) {
     }
     __syncthreads();
 
-    // L2 policies: a row of A is read twice by this warp, 2K rows apart — entering (keep it: evict_last) and leaving (done: evict_first);
-    // C is written once and read by the next kernel only after the whole volume went by (evict_first)
-    const unsigned long long pol_enter = q.l2hint ? l2_policy_evict_last() : l2_policy_evict_normal();
-    const unsigned long long pol_leave = q.l2hint ? l2_policy_evict_first() : l2_policy_evict_normal();
+    // L2 policy of the loads of A and the stores of C: evict_normal (entering rows evict_last, leaving rows and C evict_first measured no
+    // gain: DESIGN.md §4)
+    const unsigned long long pol = l2_policy_evict_normal();
     const uint32_t* pe = q.AP + (size_t)dpc * q.wp + (size_t)blockIdx.x * q.txo + lane * 8 + (size_t)y0 * q.row_words;  // update n adds physical row y0 + n (image row y0 - K + n)
     const long long back = 2LL * K * q.row_words;
     const int N = (y1 - y0) + 2 * K - 1;
@@ -462,8 +460,8 @@ k_box_planar_shfl(BoxPParams q) {
             "BOXSDONE_%=:\n"
             "}" ::"r"(bar), "r"(parity) : "memory");
         const uint32_t* src = &s_out[r & 1][4 * hf][xl0];
-        if (st0) stg_u128_hint(po, make_uint4(src[0], src[BXP_OPITCH], src[2 * BXP_OPITCH], src[3 * BXP_OPITCH]), pol_leave);
-        if (st1) stg_u128_hint(po + 128 * D, make_uint4(src[128], src[BXP_OPITCH + 128], src[2 * BXP_OPITCH + 128], src[3 * BXP_OPITCH + 128]), pol_leave);
+        if (st0) stg_u128_hint(po, make_uint4(src[0], src[BXP_OPITCH], src[2 * BXP_OPITCH], src[3 * BXP_OPITCH]), pol);
+        if (st1) stg_u128_hint(po + 128 * D, make_uint4(src[128], src[BXP_OPITCH + 128], src[2 * BXP_OPITCH + 128], src[3 * BXP_OPITCH + 128]), pol);
         po += orow;
     };
     // horizontal pass: the window sums of every column take in one row's (or one warm-up chunk's) packed differences u
@@ -536,10 +534,10 @@ k_box_planar_shfl(BoxPParams q) {
 #pragma unroll
         for (int j = 0; j < 8; j++) acc[j] = 0x80008000u;
         int cnt = 0;
-        U32x8 a = ldg_stream_u256(pe, pol_enter);
+        U32x8 a = ldg_stream_u256(pe, pol);
         for (int n = 0; n < 2 * K - 1; n++) {
             U32x8 b = a;
-            if (n + 1 < 2 * K - 1) { pe += q.row_words; b = ldg_stream_u256(pe, pol_enter); }
+            if (n + 1 < 2 * K - 1) { pe += q.row_words; b = ldg_stream_u256(pe, pol); }
 #pragma unroll
             for (int j = 0; j < 8; j++) acc[j] += a.v[j];
             if (++cnt == q.chunk || n + 1 == 2 * K - 1) {
@@ -557,8 +555,8 @@ k_box_planar_shfl(BoxPParams q) {
         auto fetch = [&](const int it, U32x8& e, U32x8& l) {
             if (it < R) {
                 pe += q.row_words;
-                e = ldg_stream_u256(pe, pol_enter);
-                if (it > 0) l = ldg_stream_u256(pe - back, pol_leave);
+                e = ldg_stream_u256(pe, pol);
+                if (it > 0) l = ldg_stream_u256(pe - back, pol);
             }
         };
         auto row = [&](const int it, const U32x8& e, const U32x8& l) {
@@ -621,10 +619,7 @@ static int sva_launch_box_planar(sva_ctx* ctx) {
             default: return occ == 3 ? k_box_planar_shfl<52, 1, 3> : k_box_planar_shfl<52, 1, 2>;
         }
     };
-    if (shfl) {
-        q.chunk = std::max(1, 32767 / (255 * p.n_pairs));
-        q.l2hint = ctx->tune_box_l2 ? 1 : 0;
-    }
+    if (shfl) q.chunk = std::max(1, 32767 / (255 * p.n_pairs));
     q.ry0 = 0; q.ry1 = H;
     if (ctx->win_rows > 0) { q.ry0 = ctx->win_y0; q.ry1 = ctx->win_y0 + ctx->win_rows; }
     const int Hw = q.ry1 - q.ry0;

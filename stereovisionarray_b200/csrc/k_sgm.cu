@@ -33,7 +33,6 @@ constexpr size_t SGM_SMEM_PER_SM = 218 * 1024;  // ring space a resident wave ma
 constexpr int SGM_WARPS_PER_SM = 46;            // marching warps per SM at 40 registers: two CTAs of 23 + 1 helper warp (warps are allocated in fours:
                                                 // 2 x 24 x 32 x 40 registers fit the 64 K file, 2 x 28 do not)
 constexpr int SGM_PF = 8;  // steps of prefetch in flight per warp; the ring has PF + 1 stages (the slot refilled at step s was last read at step s-1)
-constexpr int SGM_PF_BULK = 7;  // bulk-copy form: PF + 2 stages (the same 9 as above, so the resident-wave arithmetic is unchanged)
 
 struct SgmParams {
     const uint16_t* C;
@@ -46,7 +45,7 @@ struct SgmParams {
     unsigned int* pace_arrive;  // [pace_rounds] CTAs that finished round r (nullptr = no global pacing)
     unsigned int* pace_min;     // rounds finished by every CTA
     int pace_rounds, pace_window, march_warps;
-    int diag_split;     // diagonals run the event-split march (SVA_SGM_DIAG_SPLIT, default on)
+    int diag_split;     // diagonals run the event-split march (launches that are not paced)
     int c_ds;           // 0: C is [H][W][D]; > 0: C is slice-major [D / c_ds][H][W][c_ds] (disparity slices gathered from several GPUs)
     int balanced;       // grid = m * SM count; warp w of CTA b handles direction w % ndirs, line b + grid * (w / ndirs)
     int ranged;         // 1: direction i contributes only its lines [line_lo[i], line_lo[i] + line_cnt[i]); warp w of CTA b takes the
@@ -113,20 +112,9 @@ __device__ __forceinline__ void sgm_step(uint32_t (&L)[NR], const uint32_t (&Cc)
 
 int sva_run_wta(sva_ctx* ctx, const uint16_t* vol);
 
-// ---- how a warp moves its cells: the ring of shared-memory stages C streams through, and the way L reaches S ------------------------
-// BULK = false: per-lane cp.async (LDGSTS) into a ring of PF + 1 stages, S accumulated by per-lane 64-bit REDs (Ampere-style; every lane
-//               issues its own 4..16-byte piece through the L1TEX data path).
-// BULK = true:  the TMA engine's bulk copies (SASS UBLKCP / UBLKRED): ONE elected lane starts the copy of a whole cell (2 * D contiguous
-//               bytes) into a stage and arms that stage's mbarrier with the byte count; the warp waits on the barrier's phase parity.  L
-//               goes back through the consumed stage: every lane stores its registers into the slot, a proxy fence orders those writes
-//               before the async proxy, and the elected lane issues one cp.reduce.async.bulk (.add.u32 — packed u16x2 sums are carry-free by
-//               DESIGN.md §3.3) of the whole cell into S.  The ring has PF + 2 stages: the slot consumed at step s is refilled at step
-//               s + 2, after a bulk wait_group.read has confirmed that the reduce issued from it has read it.
-// BULK as a template argument: 0 = per-lane form, 1 = bulk loads of C with per-lane REDs into S, 2 = bulk loads and bulk reduces.
-template <int PF, int BULK> __host__ __device__ constexpr int sgm_ns() { return BULK == 2 ? PF + 2 : PF + 1; }
-template <int NR, int PF, int BULK> __host__ __device__ constexpr int sgm_warp_smem() {  // bytes per warp: the ring (+ one mbarrier per stage)
-    return sgm_ns<PF, BULK>() * 32 * 2 * NR * 2 + (BULK ? ((sgm_ns<PF, BULK>() * 8 + 15) & ~15) : 0);
-}
+// ---- how a warp moves its cells: per-lane cp.async (LDGSTS) into a ring of PF + 1 shared-memory stages, S accumulated by per-lane
+// 64-bit REDs (every lane issues its own 4..16-byte piece; the TMA engine's bulk copies measured slower: DESIGN.md §4) -----------------
+__host__ __device__ constexpr int sgm_warp_smem(const int nr, const int pf) { return (pf + 1) * 32 * 2 * nr * 2; }  // bytes per warp: the ring
 
 // base + 2 * idx as ONE IMAD.WIDE on the (idle) FMA pipe.  Left to itself the compiler builds the 64-bit address of a u16 element from a
 // 32-bit index with integer-ALU instructions (IADD3 / IADD3.X carry chains, or LEA + LEA.HI.X when it sees the constant 2) — on the pipe that
@@ -137,84 +125,56 @@ __device__ __forceinline__ const uint16_t* sgm_elem(const uint16_t* base, const 
     return (const uint16_t*)(uintptr_t)a;
 }
 
-template <int NR, int PF, bool FULL, bool STORE, int BL, int BULK>
+template <int NR, int PF, bool FULL, bool STORE, int BL>
 struct SgmPipe {
-    static constexpr int NS = sgm_ns<PF, BULK>(), NV = 2 * NR, STAGE = 32 * NV * 2;
+    static constexpr int NS = PF + 1, NV = 2 * NR, STAGE = 32 * NV * 2;
     using V = typename VecSel<NR, BL>::type;
     // Cursors are CELL indices times D, the same in every lane (warp-uniform: the compiler keeps them on the uniform datapath); what differs per
-    // lane is folded into the base pointers (per-lane form) or does not exist at all (bulk form: one lane addresses whole cells).
-    const uint16_t* C;  // cost volume (+ this lane's offset in the per-lane form)
-    uint16_t* S;        // aggregation volume (ditto)
+    // lane is folded into the base pointers.
+    const uint16_t* C;  // cost volume + this lane's offset
+    uint16_t* S;        // aggregation volume + this lane's offset
     uint32_t ring;      // this lane's bytes inside stage 0
-    uint32_t cell0;     // stage 0 (BULK)
-    uint32_t bars;      // the stages' mbarriers (BULK)
-    uint32_t cell_bytes, two;
-    bool active, elect;
+    uint32_t two;
+    bool active;
     __device__ __forceinline__ void init(const SgmParams& q, const uint32_t warp_base, const int lane, const bool active_) {
         constexpr int LANE_ELEMS = BL ? 4 : NV;
-        const int D = q.D, le = lane * LANE_ELEMS;
-        // slice-major cost volume (per-lane form only): a lane's cells never straddle a slice (c_ds % NV == 0)
+        const int le = lane * LANE_ELEMS;
+        // slice-major cost volume: a lane's cells never straddle a slice (c_ds % NV == 0)
         const size_t lane_c = q.c_ds > 0 ? (size_t)(le / q.c_ds) * q.H * q.W * q.c_ds + le % q.c_ds : (size_t)le;
-        C = BULK ? q.C : q.C + lane_c;
-        S = BULK == 2 ? q.S : q.S + le;
+        C = q.C + lane_c;
+        S = q.S + le;
         ring = warp_base + lane * (BL ? 8 : 4 * NR);
-        cell0 = warp_base; bars = warp_base + NS * STAGE; cell_bytes = 2u * D; two = q.elem_bytes;
-        active = active_; elect = lane == 0;
-        if (BULK) {
-            if (elect) {
-#pragma unroll
-                for (int i = 0; i < NS; i++) mbar_init(bars + 8 * i, 1);
-                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            }
-            fence_proxy_async_smem();
-            __syncwarp();
-        }
+        two = q.elem_bytes;
+        active = active_;
     }
     // start the copy of the cell at element index `ic` of C into stage `slot`
     __device__ __forceinline__ void fill(const int slot, const uint32_t ic) const {
-        if (BULK) {
-            if (elect) {
-                if (BULK == 2) bulk_wait_read<NS - PF - 1>();  // the reduce that was issued from this slot NS - PF steps ago has read it
-                mbar_expect_tx(bars + 8 * slot, cell_bytes);
-                bulk_g2s(cell0 + slot * STAGE, C + ic, cell_bytes, bars + 8 * slot);
-            }
-        } else if (active) V::cp_async(ring + slot * STAGE, sgm_elem(C, ic, two));
+        if (active) V::cp_async(ring + slot * STAGE, sgm_elem(C, ic, two));
     }
-    __device__ __forceinline__ void fill_end() const { if (!BULK) cp_async_commit(); }
-    // the cell of step t (stage t % NS, used for the (t / NS)-th time) -> registers
-    __device__ __forceinline__ void take(const int slot, const uint32_t parity, uint32_t (&Cc)[NR]) const {
-        if (BULK) mbar_wait(bars + 8 * slot, parity); else cp_async_wait<PF - 1>();
+    __device__ __forceinline__ void fill_end() const { cp_async_commit(); }
+    // the cell of step t (stage t % NS) -> registers
+    __device__ __forceinline__ void take(const int slot, uint32_t (&Cc)[NR]) const {
+        cp_async_wait<PF - 1>();
 #pragma unroll
         for (int j = 0; j < NR; j++) Cc[j] = SGM_INF2;
         if (active) V::lds(ring + slot * STAGE, Cc);
     }
-    // L of the cell just computed -> the cell at element index `is` of S; `slot` = the stage its C came from
-    __device__ __forceinline__ void emit(const int slot, const uint32_t is, const uint32_t (&L)[NR]) const {
-        uint16_t* dst = BULK == 2 ? S + is : const_cast<uint16_t*>(sgm_elem(S, is, two));
-        if (BULK == 2) {
-            if (active) V::sts(ring + slot * STAGE, L);
-            fence_proxy_async_smem();
-            __syncwarp();
-            if (elect) {
-                if (STORE) bulk_s2g(dst, cell0 + slot * STAGE, cell_bytes); else bulk_red_add_u32(dst, cell0 + slot * STAGE, cell_bytes);
-                bulk_commit();
-            }
-        } else if (active) {
+    // L of the cell just computed -> the cell at element index `is` of S
+    __device__ __forceinline__ void emit(const uint32_t is, const uint32_t (&L)[NR]) const {
+        uint16_t* dst = const_cast<uint16_t*>(sgm_elem(S, is, two));
+        if (active) {
             if (STORE) V::store(dst, L); else V::red(dst, L);
         }
-    }
-    __device__ __forceinline__ void drain() const {  // shared memory must outlive the bulk reads
-        if (BULK == 2) { if (elect) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); __syncwarp(); }
     }
 };
 
 // ---- the accumulate march: specialised at compile time on DIAG (wrap / restart logic only for diagonals), FULL (all 32 lanes
 // active: no predicates) and STORE (plain store vs RED), running 32-bit element cursors instead of recomputed cell indices.
-template <int NR, int PF, bool FULL, bool DIAG, bool STORE, int BL, int BULK>
+template <int NR, int PF, bool FULL, bool DIAG, bool STORE, int BL>
 __device__ __forceinline__ void sgm_acc_march(const SgmParams& q, const int dx, const int dy, const int line, const int lane, const uint32_t warp_smem,
                                               const int bar_threads, volatile int* s_pace /* [0] rounds finished by this CTA, [1] rounds finished by every CTA */,
                                               const bool leader) {
-    using Pipe = SgmPipe<NR, PF, FULL, STORE, BL, BULK>;
+    using Pipe = SgmPipe<NR, PF, FULL, STORE, BL>;
     constexpr int NS = Pipe::NS, NV = 2 * NR, LANE_ELEMS = BL ? 4 : NV;
     const int W = q.W, H = q.H, D = q.D;
     const int len = dy == 0 ? W : H;
@@ -252,9 +212,9 @@ __device__ __forceinline__ void sgm_acc_march(const SgmParams& q, const int dx, 
     for (int j = 0; j < NR; j++) L[j] = 0;
     uint32_t mm = 0, mp2 = q.p2p2;
     bool restart = false;  // step 0 starts from L = 0, mm = 0, which yields L = C
-    auto step = [&](const int slot, const uint32_t parity, const int refill_slot, const bool refill) {
+    auto step = [&](const int slot, const int refill_slot, const bool refill) {
         uint32_t Cc[NR];
-        pipe.take(slot, parity, Cc);
+        pipe.take(slot, Cc);
         if (refill) { pipe.fill(refill_slot, ic); adv(ic, cc, dstep_c, wrapfix_c); }
         pipe.fill_end();
         if (DIAG && restart) {
@@ -263,12 +223,11 @@ __device__ __forceinline__ void sgm_acc_march(const SgmParams& q, const int dx, 
             mm = 0; mp2 = q.p2p2;
         }
         sgm_step<NR, FULL, BL>(L, Cc, mm, mp2, q.p1p1, q.p2p2, first_lane, last_lane, p1_up, p1_dn);
-        pipe.emit(slot, is, L);
+        pipe.emit(is, L);
         restart = adv(is, cs, dstep, wrapfix);
     };
     int s0 = 0;
-    uint32_t par = 0;
-    for (; s0 + NS + PF <= len; s0 += NS, par ^= 1u) {
+    for (; s0 + NS + PF <= len; s0 += NS) {
         // keep the row-sweeping warps of this CTA in step (one named barrier per ring round): directions that sweep the rows in the
         // same order then touch the C and S lines they share within microseconds of each other, i.e. while they are in L2
         if (bar_threads) {
@@ -282,11 +241,10 @@ __device__ __forceinline__ void sgm_acc_march(const SgmParams& q, const int dx, 
             }
         }
 #pragma unroll
-        for (int u = 0; u < NS; u++) step(u, par, (u + PF) % NS, true);
+        for (int u = 0; u < NS; u++) step(u, (u + PF) % NS, true);
     }
     if (s_pace && leader && lane == 0) s_pace[0] = s0 / NS;  // all paced rounds done (lets the helper warp finish)
-    for (int s = s0; s < len; s++) step(s % NS, (uint32_t)(s / NS) & 1u, (s + PF) % NS, s + PF < len);
-    pipe.drain();
+    for (int s = s0; s < len; s++) step(s % NS, (s + PF) % NS, s + PF < len);
 }
 
 // Diagonal march for ONE line per warp, split at the wrap events.  A diagonal leaves the image sideways once every W steps; the
@@ -295,10 +253,10 @@ __device__ __forceinline__ void sgm_acc_march(const SgmParams& q, const int dx, 
 // bound by the integer pipe): whole ring rounds of NS steps run unrolled, the few steps around an event run one at a time.  The wrap
 // step is a per-line constant, i.e. warp-uniform here.  The CTA barrier / pacing rhythm (every NS steps, same step indices in every
 // warp) is kept, so the warps of a CTA still meet the same number of times.
-template <int NR, int PF, bool FULL, bool STORE, int BL, int BULK>
+template <int NR, int PF, bool FULL, bool STORE, int BL>
 __device__ __forceinline__ void sgm_acc_march_diag32(const SgmParams& q, const int dx, const int dy, const int line, const int lane,
                                                      const uint32_t warp_smem, const int bar_threads, volatile int* s_pace, const bool leader) {
-    using Pipe = SgmPipe<NR, PF, FULL, STORE, BL, BULK>;
+    using Pipe = SgmPipe<NR, PF, FULL, STORE, BL>;
     constexpr int NS = Pipe::NS, NV = 2 * NR, LANE_ELEMS = BL ? 4 : NV;
     const int W = q.W, H = q.H, D = q.D;
     const int len = H;
@@ -330,16 +288,16 @@ __device__ __forceinline__ void sgm_acc_march_diag32(const SgmParams& q, const i
 #pragma unroll
     for (int j = 0; j < NR; j++) L[j] = 0;
     uint32_t mm = 0, mp2 = q.p2p2;
-    auto step = [&](const int slot, const uint32_t parity, const int refill_slot, const bool refill) {
+    auto step = [&](const int slot, const int refill_slot, const bool refill) {
         uint32_t Cc[NR];
-        pipe.take(slot, parity, Cc);
+        pipe.take(slot, Cc);
         if (refill) { pipe.fill(refill_slot, ic); ic += dstep_c; }
         pipe.fill_end();
         sgm_step<NR, FULL, BL>(L, Cc, mm, mp2, q.p1p1, q.p2p2, first_lane, last_lane, p1_up, p1_dn);
-        pipe.emit(slot, is, L);
+        pipe.emit(is, L);
         is += dstep;
     };
-    int s = 0, slot = 0, round = 0;  // slot == s % NS throughout: a stage's parity is (s / NS) & 1
+    int s = 0, slot = 0, round = 0;  // slot == s % NS throughout
     while (s < len) {
         // last step before the next event: the prefetch cursor has advanced PF + s + 1 times after step s (while it refills)
         const int e_c = wc - PF - 1, e_s = ws - 1;
@@ -354,14 +312,13 @@ __device__ __forceinline__ void sgm_acc_march_diag32(const SgmParams& q, const i
                 }
             }
             if (paced) round++;
-            const uint32_t par = (uint32_t)(s / NS) & 1u;
             if (paced && s + NS - 1 <= e) {  // a whole ring round without an event: every step refills
 #pragma unroll
-                for (int u = 0; u < NS; u++) step(u, par, (u + PF) % NS, true);
+                for (int u = 0; u < NS; u++) step(u, (u + PF) % NS, true);
                 s += NS;
             } else {
                 const int rs = slot + PF >= NS ? slot + PF - NS : slot + PF;
-                step(slot, par, rs, s + PF < len);
+                step(slot, rs, s + PF < len);
                 s++;
                 slot = slot + 1 == NS ? 0 : slot + 1;
             }
@@ -375,17 +332,16 @@ __device__ __forceinline__ void sgm_acc_march_diag32(const SgmParams& q, const i
         }
     }
     if (s_pace && leader && lane == 0) s_pace[0] = round;  // all paced rounds done (lets the helper warp finish)
-    pipe.drain();
 }
 
 // Row-block march (dy != 0): the generic march over image rows [row_y0, row_y0 + row_cnt) only.  A line that was already under way
 // above (below) the block continues from the L its previous owner stored; its minimum is recomputed from that L.  A line whose
 // predecessor cell lies outside the image at the block's first row (the sweep's first row, or a diagonal that has just wrapped) starts
 // fresh exactly as in the whole-frame march.  Column of line x0 after t rows: (x0 + dx * t) mod W.
-template <int NR, int PF, bool FULL, bool STORE, int BL, int BULK>
+template <int NR, int PF, bool FULL, bool STORE, int BL>
 __device__ __forceinline__ void sgm_rows_march(const SgmParams& q, const int dx, const int dy, const int slot_of_dir, const int line, const int lane,
                                                const uint32_t warp_smem, const int bar_threads, volatile int* s_pace, const bool leader) {
-    using Pipe = SgmPipe<NR, PF, FULL, STORE, BL, BULK>;
+    using Pipe = SgmPipe<NR, PF, FULL, STORE, BL>;
     using V = typename VecSel<NR, BL>::type;
     constexpr int NS = Pipe::NS, NV = 2 * NR, LANE_ELEMS = BL ? 4 : NV;
     const int W = q.W, H = q.H, D = q.D;
@@ -430,9 +386,9 @@ __device__ __forceinline__ void sgm_rows_march(const SgmParams& q, const int dx,
         mp2 = mm + q.p2p2;
     }
     bool restart = false;
-    auto step = [&](const int slot, const uint32_t parity, const int refill_slot, const bool refill) {
+    auto step = [&](const int slot, const int refill_slot, const bool refill) {
         uint32_t Cc[NR];
-        pipe.take(slot, parity, Cc);
+        pipe.take(slot, Cc);
         if (refill) { pipe.fill(refill_slot, ic); adv(ic, cc); }
         pipe.fill_end();
         if (restart) {
@@ -441,12 +397,11 @@ __device__ __forceinline__ void sgm_rows_march(const SgmParams& q, const int dx,
             mm = 0; mp2 = q.p2p2;
         }
         sgm_step<NR, FULL, BL>(L, Cc, mm, mp2, q.p1p1, q.p2p2, first_lane, last_lane, p1_up, p1_dn);
-        pipe.emit(slot, is, L);
+        pipe.emit(is, L);
         restart = adv(is, cs);
     };
     int s0 = 0;
-    uint32_t par = 0;
-    for (; s0 + NS + PF <= len; s0 += NS, par ^= 1u) {
+    for (; s0 + NS + PF <= len; s0 += NS) {
         if (bar_threads) {  // same CTA rhythm and global pacing as the whole-frame march
             asm volatile("bar.sync 1, %0;" ::"r"(bar_threads) : "memory");
             if (s_pace) {
@@ -456,11 +411,10 @@ __device__ __forceinline__ void sgm_rows_march(const SgmParams& q, const int dx,
             }
         }
 #pragma unroll
-        for (int u = 0; u < NS; u++) step(u, par, (u + PF) % NS, true);
+        for (int u = 0; u < NS; u++) step(u, (u + PF) % NS, true);
     }
     if (s_pace && leader && lane == 0) s_pace[0] = s0 / NS;
-    for (int s = s0; s < len; s++) step(s % NS, (uint32_t)(s / NS) & 1u, (s + PF) % NS, s + PF < len);
-    pipe.drain();
+    for (int s = s0; s < len; s++) step(s % NS, (s + PF) % NS, s + PF < len);
     if (q.state_out && active) V::store(q.state_out + state_at, L);
 }
 
@@ -474,10 +428,10 @@ __device__ __forceinline__ bool sgm_ranged_line(const SgmParams& q, int g, int& 
 }
 
 // 40 registers: 48 resident warps per SM (e.g. two 22-warp CTAs of a paced c4 launch) must fit the 64 K register file
-template <int NR, int PF, bool FULL, bool STORE, int BL, bool ROWS, int BULK>
+template <int NR, int PF, bool FULL, bool STORE, int BL, bool ROWS>
 __global__ void __maxnreg__(40)
 k_sgm_acc(SgmParams q) {
-    constexpr int RING_BYTES = sgm_warp_smem<NR, PF, BULK>();
+    constexpr int RING_BYTES = sgm_warp_smem(NR, PF);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);  // the same value, marked warp-uniform for the compiler: line, direction and
@@ -518,7 +472,7 @@ k_sgm_acc(SgmParams q) {
     const int dx = q.dxs[dir], dy = q.dys[dir];
     const int nlines = dy == 0 ? q.H : q.W;
     if (line >= nlines) return;
-    const uint32_t ring = smem_u32(smem_raw) + warp * RING_BYTES;  // this warp's stages (+ mbarriers)
+    const uint32_t ring = smem_u32(smem_raw) + warp * RING_BYTES;  // this warp's stages
     int bar_threads = 0;
     bool leader = false;
     if (q.balanced && dy != 0) {  // threads of this CTA that march down/up the rows (all do the same number of rounds)
@@ -535,25 +489,34 @@ k_sgm_acc(SgmParams q) {
     }
     volatile int* pace = (q.pace_arrive && bar_threads) ? s_pace : nullptr;
     if (ROWS) {  // row-sweeping directions only (the host never puts a horizontal one into a ROWS launch)
-        sgm_rows_march<NR, PF, FULL, STORE, BL, BULK>(q, dx, dy, q.state_slot[dir], line, lane, ring, bar_threads, pace, leader);
+        sgm_rows_march<NR, PF, FULL, STORE, BL>(q, dx, dy, q.state_slot[dir], line, lane, ring, bar_threads, pace, leader);
         return;
     }
     if (dx != 0 && dy != 0) {
-        if (q.diag_split) sgm_acc_march_diag32<NR, PF, FULL, STORE, BL, BULK>(q, dx, dy, line, lane, ring, bar_threads, pace, leader);
-        else sgm_acc_march<NR, PF, FULL, true, STORE, BL, BULK>(q, dx, dy, line, lane, ring, bar_threads, pace, leader);
-    } else sgm_acc_march<NR, PF, FULL, false, STORE, BL, BULK>(q, dx, dy, line, lane, ring, bar_threads, pace, leader);
+        if (q.diag_split) sgm_acc_march_diag32<NR, PF, FULL, STORE, BL>(q, dx, dy, line, lane, ring, bar_threads, pace, leader);
+        else sgm_acc_march<NR, PF, FULL, true, STORE, BL>(q, dx, dy, line, lane, ring, bar_threads, pace, leader);
+    } else sgm_acc_march<NR, PF, FULL, false, STORE, BL>(q, dx, dy, line, lane, ring, bar_threads, pace, leader);
 }
 
-template <int NR, int PF, bool FULL, bool STORE, int BL, bool ROWS, int BULK>
-static int launch_acc_impl(sva_ctx* ctx, const SgmParams& q, const char* name) {
-    constexpr size_t RING_BYTES = sgm_warp_smem<NR, PF, BULK>();  // per warp
+// Row-sweeping launches are paced when one image row of C + S is 768 KB or more (SVA_SGM_PACE pins the choice).
+static bool sgm_paced(const sva_ctx* ctx, const SgmParams& q) {
+    return ctx->tune_sgm_pace < 0 ? (size_t)q.W * q.D * 4 >= 768 * 1024 : ctx->tune_sgm_pace != 0;
+}
+
+// path lines one launch can keep resident at once: the marching warps per SM, or the rings that fit its shared memory
+static int sgm_resident_lines(const sva_ctx* ctx, int nr) {
+    return ctx->sm_count * std::min(SGM_WARPS_PER_SM, (int)(SGM_SMEM_PER_SM / sgm_warp_smem(nr, SGM_PF)));
+}
+
+template <int NR, int PF, bool FULL, bool STORE, int BL, bool ROWS = false>
+static int launch_acc(sva_ctx* ctx, const SgmParams& q, const char* name) {
+    constexpr size_t RING_BYTES = sgm_warp_smem(NR, PF);  // per warp
     constexpr int FALLBACK_WARPS = 8;
     int nlines = 0;
     for (int i = 0; i < q.ndirs; i++) nlines = std::max(nlines, q.dys[i] == 0 ? q.H : q.W);
     int warps = FALLBACK_WARPS, grid = div_up(nlines, FALLBACK_WARPS) * q.ndirs;
     SgmParams qq = q;
     qq.balanced = 0;
-    qq.diag_split = ctx->tune_sgm_diag_split;
     // one wave of identical CTAs: m CTAs per SM, as few warps per CTA as cover all lines (every CTA the same mix of directions, every SM
     // the same number of CTAs, so all lines advance at the same rate); launches too large for one wave fall back to 8-warp CTAs
     int total = 0;
@@ -567,21 +530,20 @@ static int launch_acc_impl(sva_ctx* ctx, const SgmParams& q, const char* name) {
     }
     if (q.ranged && !qq.balanced) grid = div_up(total, FALLBACK_WARPS);
     const size_t smem = (size_t)warps * RING_BYTES;
-    SVA_CUDA_OK(ctx, cudaFuncSetAttribute(k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    SVA_CUDA_OK(ctx, cudaFuncSetAttribute(k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS, BULK>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    SVA_CUDA_OK(ctx, cudaFuncSetAttribute(k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    SVA_CUDA_OK(ctx, cudaFuncSetAttribute(k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     qq.march_warps = warps;
     qq.pace_arrive = nullptr;
     int threads = warps * 32;
     bool n_vert = false;
     for (int i = 0; i < q.ndirs; i++) n_vert = n_vert || q.dys[i] != 0;
-    const bool pace = ctx->tune_sgm_pace < 0 ? (size_t)q.W * q.D * 4 >= 768 * 1024 : ctx->tune_sgm_pace != 0;
-    if (qq.balanced && pace && q.ndirs > 1 && n_vert && q.W >= grid && warps < 32) {
+    if (qq.balanced && sgm_paced(ctx, q) && q.ndirs > 1 && n_vert && q.W >= grid && warps < 32) {
         // global pacing needs every CTA resident (the grid is one balanced wave by construction; check the occupancy anyway)
         int per_sm = 0;
-        SVA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS, BULK>, threads + 32, smem));
+        SVA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS>, threads + 32, smem));
         if (getenv("SVA_DEBUG")) fprintf(stderr, "[sva] sgm_acc NR=%d ndirs=%d grid=%d threads=%d smem=%zu per_sm=%d\n", NR, q.ndirs, grid, threads + 32, smem, per_sm);
         if ((long long)per_sm * ctx->sm_count >= grid) {
-            const int rounds = ((ROWS ? q.row_cnt : q.H) - PF) / sgm_ns<PF, BULK>();
+            const int rounds = ((ROWS ? q.row_cnt : q.H) - PF) / (PF + 1);
             if (rounds > ctx->tune_sgm_pace_window) {
                 SVA_TRY(ctx->reserve(ctx->pace_buf, ((size_t)rounds + 16) * sizeof(unsigned int)));
                 SVA_CUDA_OK(ctx, cudaMemsetAsync(ctx->pace_buf.p, 0, ((size_t)rounds + 16) * sizeof(unsigned int), ctx->stream));
@@ -595,26 +557,16 @@ static int launch_acc_impl(sva_ctx* ctx, const SgmParams& q, const char* name) {
     }
     // measured: the event-split diagonal march gains 6.6 % on unpaced launches (c1: 0.279 -> 0.261 ms) and nothing on paced ones (c2 / c4
     // move at the pace of the grid-wide minimum), where the generic march is kept
-    if (qq.pace_arrive && ctx->tune_sgm_diag_split < 2) qq.diag_split = 0;
+    qq.diag_split = qq.pace_arrive == nullptr;
     {
         // timing label = the kernel's symbol as ncu prints it + "/" + what this launch carries
         char sym[96];
-        snprintf(sym, sizeof sym, "k_sgm_acc<%d, %d, %d, %d, %d, %d, %d>/%s%s", NR, PF, (int)FULL, (int)STORE, BL, (int)ROWS, (int)BULK, name, q.ranged && q.dys[0] != 0 ? "_ranged" : "");
+        snprintf(sym, sizeof sym, "k_sgm_acc<%d, %d, %d, %d, %d, %d>/%s%s", NR, PF, (int)FULL, (int)STORE, BL, (int)ROWS, name, q.ranged && q.dys[0] != 0 ? "_ranged" : "");
         LaunchScope ls(ctx, ctx->intern(sym));
-        k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS, BULK><<<grid, threads, smem, ctx->stream>>>(qq);
+        k_sgm_acc<NR, PF, FULL, STORE, BL, ROWS><<<grid, threads, smem, ctx->stream>>>(qq);
     }
     SVA_CUDA_OK(ctx, cudaGetLastError());
     return SVA_OK;
-}
-
-// The bulk forms (the TMA engine's 1-D copies) need a cell to be one contiguous run: every layout except the slice-major volumes of the
-// sliced multi-GPU scheme.  SVA_SGM_BULK = 1 (bulk loads + per-lane REDs) or 2 (bulk loads + bulk reduces); the default, 0, is the per-lane
-// cp.async / RED form, which measured fastest on B200 (profiles/r02_sgm_bulk_ab.txt).
-template <int NR, int PF, bool FULL, bool STORE, int BL, bool ROWS = false>
-static int launch_acc(sva_ctx* ctx, const SgmParams& q, const char* name) {
-    if (ctx->tune_sgm_bulk == 2 && q.c_ds == 0) return launch_acc_impl<NR, SGM_PF_BULK, FULL, STORE, BL, ROWS, 2>(ctx, q, name);
-    if (ctx->tune_sgm_bulk == 1 && q.c_ds == 0) return launch_acc_impl<NR, PF, FULL, STORE, BL, ROWS, 1>(ctx, q, name);
-    return launch_acc_impl<NR, PF, FULL, STORE, BL, ROWS, 0>(ctx, q, name);
 }
 
 // the directions q.dxs / q.dys in ONE launch; store = plain stores (a single direction that initialises S) instead of REDs
@@ -622,7 +574,7 @@ template <int NR>
 static int launch_dirs_nr(sva_ctx* ctx, const SgmParams& q, bool store) {
     const bool full = q.lanes == 32;
     // what the launch carries: row-sweeping directions (they share C and S lines in L2: the launch streams C once and read-modify-writes S
-    // once), horizontal directions (-> and <- cannot share: each streams C and S), or a mix (4 paths / SVA_SGM_SPLIT=0)
+    // once), horizontal directions (-> and <- cannot share: each streams C and S), or a mix (4 paths)
     bool any_v = false, any_h = false;
     for (int i = 0; i < q.ndirs; i++) { any_v = any_v || q.dys[i] != 0; any_h = any_h || q.dys[i] == 0; }
     static const char* const cnt[9] = {"0", "1", "2", "3", "4", "5", "6", "7", "8"};
@@ -637,7 +589,7 @@ static int launch_dirs_nr(sva_ctx* ctx, const SgmParams& q, bool store) {
         return full ? launch_acc<NR, SGM_PF, true, false, 0, true>(ctx, q, nm) : launch_acc<NR, SGM_PF, false, false, 0, true>(ctx, q, nm);
     }
     if constexpr (NR == 4) {  // D = 256 / 192 on a contiguous volume: the block layout (whole-sector copies and REDs)
-        if (q.c_ds == 0 && !getenv("SVA_SGM_NO_BLK")) {
+        if (q.c_ds == 0) {
             if (q.lanes == 32) return store ? launch_acc<NR, SGM_PF, true, true, 32>(ctx, q, nm) : launch_acc<NR, SGM_PF, true, false, 32>(ctx, q, nm);
             if (q.lanes == 24) return store ? launch_acc<NR, SGM_PF, false, true, 24>(ctx, q, nm) : launch_acc<NR, SGM_PF, false, false, 24>(ctx, q, nm);
         }
@@ -670,51 +622,33 @@ static void set_dirs(SgmParams& q, const int* idx, int n) {
 }
 
 // One group of directions that sweep the rows the same way.  They share a row's C and S lines in L2 only while ALL their lines are
-// resident and paced; a group with more lines than fit one resident wave (3 x 3840 at c3) is therefore cut into launches that do fit —
-// whole directions first, one direction split by line range — instead of running in unsynchronised waves that share nothing.
+// resident and paced; a group with more lines than fit one resident wave (3 x 3840 at c3) is therefore cut into launches that do fit
+// instead of running in unsynchronised waves that share nothing.  Such a group is always a ROW BLOCK (a whole frame that needs the cut is
+// marched in row blocks: run_group_in_blocks), and it is cut by COLUMNS.
 static int launch_row_group(sva_ctx* ctx, SgmParams& q, int nr, const int* idx, int n) {
     set_dirs(q, idx, n);
     q.ranged = 0;
-    const size_t ring = (size_t)(SGM_PF + 1) * 32 * 2 * nr * 2 + (ctx->tune_sgm_bulk ? 80 : 0);  // (+ the stages' mbarriers)
-    const int cap = ctx->sm_count * std::min(SGM_WARPS_PER_SM, (int)(SGM_SMEM_PER_SM / ring));
-    const bool pace = ctx->tune_sgm_pace < 0 ? (size_t)q.W * q.D * 4 >= 768 * 1024 : ctx->tune_sgm_pace != 0;
-    if (!pace || n * q.W <= cap || q.W > cap || getenv("SVA_SGM_NO_RANGED")) return launch_dirs(ctx, q, nr, false);
-    const int launches = div_up(n * q.W, cap), per_launch = div_up(n * q.W, launches);  // equal shares: every launch streams the whole volume once
-    if (q.row_cnt > 0 && !getenv("SVA_SGM_NO_COLSPLIT")) {
-        // A ROW BLOCK is cut by COLUMNS instead: launch j takes, of every direction, the lines that enter the block inside column range j.
-        // A diagonal drifts one column per row, so over a block of B rows the lines of a launch stay within their column range + B columns:
-        // each launch streams ITS columns of C and S once for all three directions, and only the B-column fringe is streamed by two
-        // launches — (1 + B / range) volumes of traffic per group instead of one per launch (c3, 270-row blocks: 1.14 instead of 2).
-        const int W = q.W;
-        const long long t = q.dys[0] > 0 ? q.row_y0 : q.H - 1 - (q.row_y0 + q.row_cnt - 1);  // rows the sweep has crossed before this block
-        for (int j = 0; j < launches; j++) {
-            const int c0 = (int)((long long)W * j / launches), c1 = (int)((long long)W * (j + 1) / launches);
-            SgmParams s = q;
-            s.ranged = 1; s.ndirs = 0;
-            for (int dir = 0; dir < n; dir++) {
-                // column of line x0 after t rows is (x0 + dx * t) mod W, so the lines entering in [c0, c1) are the range starting at (c0 - dx * t) mod W
-                const int lo = (int)((((long long)c0 - (long long)q.dxs[dir] * t) % W + W) % W), len = c1 - c0, first = std::min(len, W - lo);
-                for (int part = 0; part < 2; part++) {
-                    const int a = part == 0 ? lo : 0, cnt = part == 0 ? first : len - first;
-                    if (cnt <= 0) continue;
-                    s.dxs[s.ndirs] = q.dxs[dir]; s.dys[s.ndirs] = q.dys[dir]; s.state_slot[s.ndirs] = q.state_slot[dir];
-                    s.line_lo[s.ndirs] = a; s.line_cnt[s.ndirs] = cnt; s.ndirs++;
-                }
-            }
-            SVA_TRY(launch_dirs(ctx, s, nr, false));
-        }
-        return SVA_OK;
-    }
-    int dir = 0, lo = 0;
-    while (dir < n) {
+    const int cap = sgm_resident_lines(ctx, nr);
+    if (!sgm_paced(ctx, q) || n * q.W <= cap || q.W > cap) return launch_dirs(ctx, q, nr, false);
+    // Launch j takes, of every direction, the lines that enter the block inside column range j.  A diagonal drifts one column per row, so
+    // over a block of B rows the lines of a launch stay within their column range + B columns: each launch streams ITS columns of C and S
+    // once for all three directions, and only the B-column fringe is streamed by two launches — (1 + B / range) volumes of traffic per group
+    // instead of one per launch (c3, 270-row blocks: 1.14 instead of 2).
+    const int W = q.W, launches = div_up(n * W, cap);
+    const long long t = q.dys[0] > 0 ? q.row_y0 : q.H - 1 - (q.row_y0 + q.row_cnt - 1);  // rows the sweep has crossed before this block
+    for (int j = 0; j < launches; j++) {
+        const int c0 = (int)((long long)W * j / launches), c1 = (int)((long long)W * (j + 1) / launches);
         SgmParams s = q;
         s.ranged = 1; s.ndirs = 0;
-        for (int room = per_launch; dir < n && room > 0;) {
-            const int take = std::min(room, q.W - lo);
-            s.dxs[s.ndirs] = q.dxs[dir]; s.dys[s.ndirs] = q.dys[dir]; s.state_slot[s.ndirs] = q.state_slot[dir];
-            s.line_lo[s.ndirs] = lo; s.line_cnt[s.ndirs] = take; s.ndirs++;
-            room -= take; lo += take;
-            if (lo == q.W) { dir++; lo = 0; }
+        for (int dir = 0; dir < n; dir++) {
+            // column of line x0 after t rows is (x0 + dx * t) mod W, so the lines entering in [c0, c1) are the range starting at (c0 - dx * t) mod W
+            const int lo = (int)((((long long)c0 - (long long)q.dxs[dir] * t) % W + W) % W), len = c1 - c0, first = std::min(len, W - lo);
+            for (int part = 0; part < 2; part++) {
+                const int a = part == 0 ? lo : 0, cnt = part == 0 ? first : len - first;
+                if (cnt <= 0) continue;
+                s.dxs[s.ndirs] = q.dxs[dir]; s.dys[s.ndirs] = q.dys[dir]; s.state_slot[s.ndirs] = q.state_slot[dir];
+                s.line_lo[s.ndirs] = a; s.line_cnt[s.ndirs] = cnt; s.ndirs++;
+            }
         }
         SVA_TRY(launch_dirs(ctx, s, nr, false));
     }
@@ -745,10 +679,8 @@ static int run_group_in_blocks(sva_ctx* ctx, SgmParams& q, int nr, const int* id
 }
 
 static bool group_needs_blocks(sva_ctx* ctx, const SgmParams& q, int nr, int n) {
-    const size_t ring = (size_t)(SGM_PF + 1) * 32 * 2 * nr * 2 + (ctx->tune_sgm_bulk ? 80 : 0);
-    const int cap = ctx->sm_count * std::min(SGM_WARPS_PER_SM, (int)(SGM_SMEM_PER_SM / ring));
-    const bool pace = ctx->tune_sgm_pace < 0 ? (size_t)q.W * q.D * 4 >= 768 * 1024 : ctx->tune_sgm_pace != 0;
-    return pace && n * q.W > cap && q.W <= cap && !getenv("SVA_SGM_NO_RANGED") && !getenv("SVA_SGM_NO_COLSPLIT") && q.c_ds == 0;
+    const int cap = sgm_resident_lines(ctx, nr);
+    return sgm_paced(ctx, q) && n * q.W > cap && q.W <= cap && q.c_ds == 0;
 }
 
 // exactly the directions of dir_mask, one launch each: the first stores, the others RED, so S ends up as their sum
@@ -862,16 +794,19 @@ int sva_run_sgm(sva_ctx* ctx) {
             beg = nullptr;
         }
     } wall(ctx);
-    if (n == 8 && ctx->tune_sgm_split && ctx->tune_sgm_hstore && !ctx->s_prezeroed) {
-        // S is never zeroed: the first horizontal direction WRITES it (plain stores: C in, S out = 4 B/DE), the second accumulates (6 B/DE), then
-        // the row-sweeping groups — 10 B/DE for the horizontal pair instead of 12 plus the 2 B/DE of the memset that ran next to K1
-        static const int grp[3][3] = {{0, 4, 5}, {1, 6, 7}, {2, 3, -1}};
+    if (n == 8) {
+        // A row-sweeping launch holds only lines that advance one row per step, so (paced where a row is large) all of them touch a
+        // row's C and S lines while these are in L2.  The horizontal lines (W steps each, every row in flight at once) cannot share
+        // and get launches of their own.  S is never zeroed: the first horizontal direction WRITES it (plain stores: C in, S out = 4 B/DE),
+        // the second accumulates (6 B/DE), then the row-sweeping groups — 10 B/DE for the horizontal pair instead of 12 plus the 2 B/DE of a memset
+        static const int grp[2][3] = {{0, 4, 5}, {1, 6, 7}};
         const int h0 = 2, h1 = 3;
         set_dirs(q, &h0, 1);
         SVA_TRY(launch_dirs(ctx, q, nr, true));
         // The second horizontal direction is a launch of H warps bound by the latency of its own recurrence (~200 clocks per step): with
-        // SVA_SGM_HSTORE = 2 it runs on the second stream NEXT TO the first row-sweeping group (REDs commute; both start after the stores).
-        const bool side = ctx->tune_sgm_hstore == 3 || (ctx->tune_sgm_hstore == 2 && q.W * (size_t)q.D * 4 < 768 * 1024);  // not next to paced launches: they want the SM to themselves
+        // SVA_SGM_HSTORE = 2 (the default) it runs on the second stream NEXT TO the first row-sweeping group (REDs commute; both start after
+        // the stores); 1 keeps the launches one after the other.
+        const bool side = ctx->tune_sgm_hstore == 2 && q.W * (size_t)q.D * 4 < 768 * 1024;  // not next to paced launches: they want the SM to themselves
         cudaStream_t main_stream = ctx->stream;
         if (side) {
             if (!ctx->aux_stream) {
@@ -900,26 +835,13 @@ int sva_run_sgm(sva_ctx* ctx) {
         ctx->have_sgm = true; ctx->have_disp = true;
         return SVA_OK;
     }
-    // S = 0 (zeroed next to K1a / K1b when the caller got that far ahead: sva_api.cu), every path accumulates with REDs, K3 reads S_total
+    // 4 paths: S = 0 (zeroed next to K1a / K1b when the caller got that far ahead: sva_api.cu), one launch accumulating with REDs, K3 reads S_total
     if (ctx->s_prezeroed) SVA_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_zero, 0));
     else SVA_CUDA_OK(ctx, cudaMemsetAsync(ctx->S.p, 0, cells * sizeof(uint16_t), ctx->stream));
     ctx->s_prezeroed = false;
-    if (n == 8 && ctx->tune_sgm_split) {
-        // A row-sweeping launch holds only lines that advance one row per step, so (paced where a row is large) all of them touch a
-        // row's C and S lines while these are in L2.  The horizontal lines (W steps each, every row in flight at once) cannot share
-        // and get their own launch.
-        static const int grp[3][3] = {{0, 4, 5}, {1, 6, 7}, {2, 3, -1}};
-        for (int g = 0; g < 2; g++) {
-            if (group_needs_blocks(ctx, q, nr, 3)) SVA_TRY(run_group_in_blocks(ctx, q, nr, grp[g], 3));
-            else SVA_TRY(launch_row_group(ctx, q, nr, grp[g], 3));
-        }
-        set_dirs(q, grp[2], 2);
-        SVA_TRY(launch_dirs(ctx, q, nr, false));
-    } else {  // 4 paths (or SVA_SGM_SPLIT=0): one launch, directions that sweep the same rows next to each other
-        static const int all8[8] = {0, 4, 5, 1, 6, 7, 2, 3}, all4[4] = {0, 1, 2, 3};
-        set_dirs(q, n == 8 ? all8 : all4, n);
-        SVA_TRY(launch_dirs(ctx, q, nr, false));
-    }
+    static const int all4[4] = {0, 1, 2, 3};
+    set_dirs(q, all4, 4);
+    SVA_TRY(launch_dirs(ctx, q, nr, false));
     wall.stop();
     SVA_TRY(sva_run_wta(ctx, ctx->S.as<uint16_t>()));
     ctx->have_sgm = true; ctx->have_disp = true;

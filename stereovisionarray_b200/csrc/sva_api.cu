@@ -144,7 +144,7 @@ static int prezero_s(sva_ctx* c) {
     const sva_params& p = c->prm;
     c->s_prezeroed = false;
     if (p.n_paths == 0 || c->sgm_dir_mask_override || !c->tune_prezero) return SVA_OK;
-    if (p.n_paths == 8 && c->tune_sgm_split && c->tune_sgm_hstore) return SVA_OK;  // S is written, not accumulated, by the first SGM launch
+    if (p.n_paths == 8) return SVA_OK;  // S is written, not accumulated, by the first SGM launch
     const size_t bytes = (size_t)p.width * p.height * p.num_disp * sizeof(uint16_t);
     SVA_TRY(c->reserve(c->S, bytes + 64));
     if (!c->aux_stream) {

@@ -103,22 +103,17 @@ struct sva_ctx {
     int pair_begin = 0, pair_end = 0;
     bool has_mask = false;
     bool debug_store_full_s = false;
-    int tune_sgm_split = 1;       // SVA_SGM_SPLIT: 8 paths as three launches (down-sweeping, up-sweeping, horizontal; default) or, 0, as one
-    int tune_sgm_hstore = 2;      // SVA_SGM_HSTORE: 1 = the first horizontal direction initialises S with plain stores (no memset) and the second accumulates;
-                                  // 2 (default) = and the second runs on the second stream next to the first row-sweeping group where the launches are not
-                                  // paced; 3 = always next to it; 0 = S zeroed by a memset next to K1, both horizontal directions in one launch
+    int tune_sgm_hstore = 2;      // SVA_SGM_HSTORE: 8 paths: the first horizontal direction initialises S with plain stores (no memset), the second
+                                  // accumulates; 2 (default) = on the second stream next to the first row-sweeping group where the launches are not paced;
+                                  // 1 = one launch after the other (bench.py's kernel-table pass)
     int tune_sgm_pace = -1;       // SVA_SGM_PACE: keep all CTAs of a row-sweeping launch within pace_window rounds (of 9 rows) of each other.
                                   // -1 = automatic: on when one image row of C + S (W*D*4 bytes) is 768 KB or more.  The three directions of such a
                                   // launch share C and S lines in L2 only while their rows stay within the L2-resident window; unpaced drift is harmless
                                   // at c1 (0.66 MB per row: 0.277 ms unpaced, 0.283 paced) and costly at c4 (1.47 MB per row: 1.355 -> 0.925 ms paced).
     int tune_sgm_pace_window = 2; // SVA_SGM_PACE_WINDOW: rounds of 9 rows
-    int tune_sgm_bulk = 0;        // SVA_SGM_BULK: 1 = C streams in by the TMA engine's bulk copies + mbarriers, 2 = and S is accumulated by bulk reduces;
-                                  // 0 (default, fastest measured) = per-lane cp.async / RED
-    int tune_sgm_diag_split = 1;  // SVA_SGM_DIAG_SPLIT: diagonal lines run the march that is split at the wrap events (no per-step wrap logic)
     int tune_ad_gather = 0;       // SVA_AD_GATHER=1: force the line-image gather AD kernel (k_ad.cu) even where the image-space kernel applies
     int tune_ad_set = 1;          // SVA_AD_SET: use the AD kernel compiled for the frame's pair set where one exists (0 = always the generic kernel)
     int tune_ad_th = 0;           // SVA_AD_TH: rows per tile of the image-space AD kernel (0 = chosen per launch, k_ad2.cu)
-    int tune_box_l2 = 0;          // SVA_BOX_L2: K1b's entering rows stay in L2 (evict_last) for their second read as leaving rows (evict_first, like the C stores)
     int tune_box_occ = 0;         // SVA_BOX_OCC: CTAs per SM K1b is compiled for (2: up to 128 registers, 3: 80; 0 = chosen per launch)
     int tune_box_bands = 0;       // SVA_BOX_BANDS: row bands of K1b (0 = chosen per launch)
     int tune_box_shfl = 1;        // SVA_BOX_SHFL: K1b's horizontal window sums by warp shuffles where win_half % 8 == 4 (0 = the shared-memory prefix table)
@@ -200,7 +195,7 @@ __device__ __forceinline__ uint4 ldg_stream_u128(const void* p) {
     return v;
 }
 // 32 bytes per lane in ONE instruction (LDG.E.256, sm_100): a warp-load covers 1 KB of whole sectors.  `policy` is an L2 eviction
-// policy word from l2_policy_* below.  The address must be 32-byte aligned.
+// policy word from l2_policy_evict_normal below.  The address must be 32-byte aligned.
 struct U32x8 { uint32_t v[8]; };
 __device__ __forceinline__ U32x8 ldg_stream_u256(const void* p, const unsigned long long policy) {
     U32x8 r;
@@ -208,16 +203,6 @@ __device__ __forceinline__ U32x8 ldg_stream_u256(const void* p, const unsigned l
                  : "=r"(r.v[0]), "=r"(r.v[1]), "=r"(r.v[2]), "=r"(r.v[3]), "=r"(r.v[4]), "=r"(r.v[5]), "=r"(r.v[6]), "=r"(r.v[7])
                  : "l"(p), "l"(policy));
     return r;
-}
-__device__ __forceinline__ unsigned long long l2_policy_evict_last() {
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-__device__ __forceinline__ unsigned long long l2_policy_evict_first() {
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
 }
 __device__ __forceinline__ unsigned long long l2_policy_evict_normal() {
     unsigned long long pol;

@@ -3,7 +3,6 @@
 #include <climits>
 #include <cstdio>
 #include <cstdlib>
-#include <cstring>
 
 #include "sva_common.cuh"
 
@@ -111,12 +110,9 @@ static bool read_switch(const char* name, int& field, int lo, int hi, const char
 }
 
 static bool read_switches(sva_ctx* c) {
-    bool ok = read_switch("SVA_SGM_SPLIT", c->tune_sgm_split, 0, 1, "0, 1")
-           && read_switch("SVA_SGM_PACE", c->tune_sgm_pace, -1, 1, "-1, 0, 1")
+    return read_switch("SVA_SGM_PACE", c->tune_sgm_pace, -1, 1, "-1, 0, 1")
            && read_switch("SVA_SGM_PACE_WINDOW", c->tune_sgm_pace_window, 1, 1 << 20, "1 or more")
-           && read_switch("SVA_SGM_HSTORE", c->tune_sgm_hstore, 0, 3, "0, 1, 2, 3")
-           && read_switch("SVA_SGM_BULK", c->tune_sgm_bulk, 0, 2, "0, 1, 2")
-           && read_switch("SVA_SGM_DIAG_SPLIT", c->tune_sgm_diag_split, 0, 2, "0, 1, 2")
+           && read_switch("SVA_SGM_HSTORE", c->tune_sgm_hstore, 1, 2, "1, 2")
            && read_switch("SVA_STREAM_AD_AHEAD", c->tune_stream_ad_ahead, 0, 2, "0, 1, 2")
            && read_switch("SVA_PREZERO", c->tune_prezero, 0, 1, "0, 1")
            && read_switch("SVA_WTA_SEG", c->tune_wta_seg, -1, 1 << 16, "-1, 0, or a segment length up to 65536")
@@ -124,15 +120,8 @@ static bool read_switches(sva_ctx* c) {
            && read_switch("SVA_AD_SET", c->tune_ad_set, 0, 1, "0, 1")
            && read_switch("SVA_AD_TH", c->tune_ad_th, 0, 1 << 16, "0, or rows per tile up to 65536")
            && read_switch("SVA_BOX_SHFL", c->tune_box_shfl, 0, 1, "0, 1")
-           && read_switch("SVA_BOX_L2", c->tune_box_l2, 0, 1, "0, 1")
            && read_switch("SVA_BOX_BANDS", c->tune_box_bands, 0, 1 << 20, "0, or a band count")
            && read_switch("SVA_BOX_OCC", c->tune_box_occ, 0, 3, "0, 2, 3", 1);  // K1b exists for 2 and 3 CTAs per SM
-    // read where the SGM launches are planned (k_sgm.cu), by presence; "1" is the one documented value, anything else is a mistake
-    for (const char* name : {"SVA_SGM_NO_BLK", "SVA_SGM_NO_RANGED", "SVA_SGM_NO_COLSPLIT"}) {
-        const char* e = getenv(name);
-        if (ok && e && strcmp(e, "1") != 0) { create_err = std::string(name) + "=" + e + " is not valid (allowed: 1, or unset)"; ok = false; }
-    }
-    return ok;
 }
 
 extern "C" {

@@ -7,38 +7,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// ---- bulk asynchronous copies (the TMA engine's 1-D form, SASS UBLKCP / UBLKRED) and their mbarriers: one elected lane moves a whole
-// cell (2 * D contiguous bytes) per instruction instead of 32 lanes moving 4-16 bytes each through the L1TEX data path ----
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}" ::"r"(bar), "r"(parity) : "memory");
-}
-// global -> shared, completion counted in bytes on an mbarrier (a CTA's own shared window is a valid shared::cluster address)
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-// shared -> global as an element-wise u32 ADD performed at L2 (packed u16x2 sums are carry-free here) / as a plain store
-__device__ __forceinline__ void bulk_red_add_u32(void* dst, uint32_t src, uint32_t bytes) {
-    asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.u32 [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_s2g(void* dst, uint32_t src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 template <int NR> struct Vec;
 template <> struct Vec<1> {
     static __device__ __forceinline__ void load(const uint16_t* p, uint32_t (&r)[1]) { r[0] = ldg_stream_u32(p); }
@@ -47,7 +15,6 @@ template <> struct Vec<1> {
     }
     static __device__ __forceinline__ void cp_async(uint32_t dst, const uint16_t* p) { asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(p) : "memory"); }
     static __device__ __forceinline__ void lds(uint32_t src, uint32_t (&r)[1]) { asm volatile("ld.shared.u32 %0, [%1];" : "=r"(r[0]) : "r"(src)); }
-    static __device__ __forceinline__ void sts(uint32_t dst, const uint32_t (&r)[1]) { asm volatile("st.shared.u32 [%0], %1;" ::"r"(dst), "r"(r[0]) : "memory"); }
     static __device__ __forceinline__ void store(uint16_t* p, const uint32_t (&r)[1]) { *reinterpret_cast<uint32_t*>(p) = r[0]; }
     static __device__ __forceinline__ void red(uint16_t* p, const uint32_t (&r)[1]) {
         asm volatile("red.global.add.u32 [%0], %1;" ::"l"(p), "r"(r[0]) : "memory");
@@ -60,7 +27,6 @@ template <> struct Vec<2> {
     }
     static __device__ __forceinline__ void cp_async(uint32_t dst, const uint16_t* p) { asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(p) : "memory"); }
     static __device__ __forceinline__ void lds(uint32_t src, uint32_t (&r)[2]) { asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(r[0]), "=r"(r[1]) : "r"(src)); }
-    static __device__ __forceinline__ void sts(uint32_t dst, const uint32_t (&r)[2]) { asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(dst), "r"(r[0]), "r"(r[1]) : "memory"); }
     static __device__ __forceinline__ void store(uint16_t* p, const uint32_t (&r)[2]) { *reinterpret_cast<uint2*>(p) = make_uint2(r[0], r[1]); }
     static __device__ __forceinline__ void red(uint16_t* p, const uint32_t (&r)[2]) {
         unsigned long long v = ((unsigned long long)r[1] << 32) | r[0];
@@ -74,9 +40,6 @@ template <> struct Vec<4> {
     }
     static __device__ __forceinline__ void cp_async(uint32_t dst, const uint16_t* p) { asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(p) : "memory"); }
     static __device__ __forceinline__ void lds(uint32_t src, uint32_t (&r)[4]) { asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(src)); }
-    static __device__ __forceinline__ void sts(uint32_t dst, const uint32_t (&r)[4]) {
-        asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]) : "memory");
-    }
     static __device__ __forceinline__ void store(uint16_t* p, const uint32_t (&r)[4]) { *reinterpret_cast<uint4*>(p) = make_uint4(r[0], r[1], r[2], r[3]); }
     static __device__ __forceinline__ void red(uint16_t* p, const uint32_t (&r)[4]) {
         unsigned long long v0 = ((unsigned long long)r[1] << 32) | r[0], v1 = ((unsigned long long)r[3] << 32) | r[2];
@@ -141,10 +104,6 @@ template <int BL> struct VecBlk4 {
     static __device__ __forceinline__ void lds(uint32_t src, uint32_t (&r)[4]) {
         asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(r[0]), "=r"(r[1]) : "r"(src));
         asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(r[2]), "=r"(r[3]) : "r"(src + 8 * BL));
-    }
-    static __device__ __forceinline__ void sts(uint32_t dst, const uint32_t (&r)[4]) {
-        asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(dst), "r"(r[0]), "r"(r[1]) : "memory");
-        asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(dst + 8 * BL), "r"(r[2]), "r"(r[3]) : "memory");
     }
     static __device__ __forceinline__ void store(uint16_t* p, const uint32_t (&r)[4]) {
         *reinterpret_cast<uint2*>(p) = make_uint2(r[0], r[1]);

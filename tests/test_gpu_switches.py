@@ -1,7 +1,7 @@
 """Every kernel variant the A/B switches of DESIGN §8a select, against the oracle, on guarded contexts.  Needs a B200: -m gpu.
 
-The switches are environment variables read at sva_create (SVA_SGM_NO_* also where the SGM launches are planned), so each check sets its
-variables for the whole test and creates a fresh context.  SWITCHES has one entry per variant: the variables, the cases that reach the
+The switches are environment variables read at sva_create, so each check sets its variables for the whole test and creates a fresh
+context.  SWITCHES has one entry per variant: the variables, the cases that reach the
 variant, the stages it can change and a witness — what the timing labels of one production run must show for the switch to have taken
 effect — where the library exposes one.  tests/test_switch_inventory.py checks that every switch the library reads has an entry here."""
 import re
@@ -58,16 +58,12 @@ class Sw(NamedTuple):
 
 
 def _sgm_args(labels):
-    """template arguments <NR, PF, FULL, STORE, BL, ROWS, BULK> of every k_sgm_acc launch"""
+    """template arguments <NR, PF, FULL, STORE, BL, ROWS> of every k_sgm_acc launch"""
     return [[int(a) for a in re.match(r"k_sgm_acc<([^>]*)>", l).group(1).split(",")] for l in labels if l.startswith("k_sgm_acc<")]
 
 
 def _ranged(labels, group):
     return sum(1 for l in labels if re.search(r"/red_%s\d_ranged$" % group, l))
-
-
-def _bulk(v):
-    return lambda L, p: bool(_sgm_args(L)) and all(a[6] == v for a in _sgm_args(L))
 
 
 def _stores(L):
@@ -78,7 +74,6 @@ _one_hstore = lambda L, p: len(_stores(L)) == 1 and _stores(L)[0].endswith("/sto
 _no_ranged = lambda L, p: bool(_sgm_args(L)) and not any("_ranged" in l for l in L)
 
 BOX4 = ("c0", "c11", "c13", "c12")  # win_half 4, 12, 20, 28: the register form of K1b (win_half % 8 == 4) with 1, 3, 5, 7 lanes per window
-BULK_D = ("c5", "c0", "c1", "d160", "c2", "c3")  # D = 16 (NR 1, 8 lanes, 4 paths), 64 (NR 1, full warp, 4 paths), 128 (NR 2), 160 (NR 4, 20 lanes), 192 / 256 (block layout, 24 / 32 lanes)
 PACE_D = ("pace64", "pace128", "pace192", "pace256")
 
 SWITCHES = [
@@ -96,25 +91,13 @@ SWITCHES = [
     # 4096 bands: one row per band, shorter than any window (a band the cost model never picks)
     *[Sw({"SVA_BOX_BANDS": v}, ("c0", "c13", "c7", "rows0"), "K1b", None, "the band count is otherwise the cost model's (c7: the prefix-table kernel, k = 7)")
       for v in ("1", "2", "5", "4096")],
-    Sw({"SVA_BOX_L2": "1"}, ("c0", "c13"), "K1b", None, "the eviction hints are compiled into the register form, which c0 (k = 4) and c13 (k = 20) run"),
     # K2 (k_sgm.cu)
-    *[Sw({"SVA_SGM_BULK": v}, BULK_D + tuple(ROWS) + ("mblk",), "K2", _bulk(int(v)), dirs=BULK_D) for v in ("1", "2")],
     *[Sw({"SVA_SGM_PACE": "1", "SVA_SGM_PACE_WINDOW": wnd}, PACE_D, "K2", None, "frames this small are not paced by default; their rounds exceed the window")
       for wnd in ("1", "2", "4")],
     Sw({"SVA_SGM_PACE": "0"}, ("wide1", "mblk"), "K2", _no_ranged),
-    Sw({"SVA_SGM_DIAG_SPLIT": "0"}, ("c1", "c2", "wide0"), "K2", None, "unpaced 8-path frames run the split diagonal march by default"),
-    Sw({"SVA_SGM_DIAG_SPLIT": "2"}, ("wide1",), "K2", None, "wide1 is paced: by default its diagonals take the generic march"),
-    Sw({"SVA_SGM_DIAG_SPLIT": "2", "SVA_SGM_PACE": "1"}, ("pace64", "pace192"), "K2", None, "forced pacing with the split diagonal march"),
-    *[Sw({"SVA_SGM_HSTORE": "0", "SVA_PREZERO": z}, ("c1", "c2", "wide1"), "K2", lambda L, p: not _stores(L)) for z in ("0", "1")],
-    *[Sw({"SVA_SGM_HSTORE": v}, ("c1", "wide1"), "K2", _one_hstore) for v in ("1", "3")],
+    Sw({"SVA_SGM_HSTORE": "1"}, ("c1", "wide1"), "K2", _one_hstore),
     Sw({"SVA_PREZERO": "0"}, ("c0", "c5"), "K2", None, "4-path frames zero S next to K1 by default; 0 = a memset in line"),
-    Sw({"SVA_SGM_SPLIT": "0"}, ("c1", "c2", "wide1"), "K2", lambda L, p: any(l.endswith("/red_mixed8") for l in L)),
-    Sw({"SVA_SGM_NO_BLK": "1"}, ("c2", "c3", "pace256"), "K2",
-       lambda L, p: any(a[0] == 4 for a in _sgm_args(L)) and all(a[4] == 0 for a in _sgm_args(L))),
-    Sw({"SVA_SGM_NO_RANGED": "1"}, ("mblk",), "K2", _no_ranged),
-    # without the column cut the group is one set of ranged launches for the whole frame: 3 W lines in launches of at least W lines = 1 to
-    # 3 per group, against one such set per row block (two blocks here) by default
-    Sw({"SVA_SGM_NO_COLSPLIT": "1"}, ("mblk",), "K2", lambda L, p: 1 <= _ranged(L, "down") <= 3 and 1 <= _ranged(L, "up") <= 3),
+    # the default schedule: one set of column-cut ranged launches per row block (two blocks here) and sweep
     Sw({}, ("mblk",), "K2", lambda L, p: _ranged(L, "down") >= 4 and _ranged(L, "up") >= 4),
     # K3 (k_wta.cu): 0 = the shared-memory tile kernel (+ the LR check where lr_gx != 0); the segment lengths the frame-size rule never picks
     # at these sizes (160 with D = 192 leaves a partial rotation in every segment; 4096 = one segment per row)
@@ -167,7 +150,7 @@ def _clean(c):
 def _new_ctx(monkeypatch, env):
     from stereovisionarray_b200.pipeline import DepthContext
     for k, v in env.items():
-        monkeypatch.setenv(k, v)  # kept for the whole test: SVA_SGM_NO_* are read at launch time
+        monkeypatch.setenv(k, v)
     c = DepthContext(0)
     c.set_guard(True)
     return c
@@ -260,10 +243,9 @@ def test_switch_capture_stream_matches_oracle(monkeypatch, oracle, e, case):
         ctx.close()
 
 
-@pytest.mark.parametrize("var,value", [("SVA_BOX_OCC", "1"), ("SVA_SGM_SPLIT", "off"), ("SVA_SGM_PACE_WINDOW", "0"), ("SVA_SGM_BULK", "3"),
-                                       ("SVA_SGM_HSTORE", "4"), ("SVA_SGM_DIAG_SPLIT", "-1"), ("SVA_SGM_PACE", "2"), ("SVA_WTA_SEG", "-2"),
-                                       ("SVA_AD_TH", "-8"), ("SVA_BOX_BANDS", "2x"), ("SVA_AD_SET", ""), ("SVA_STREAM_AD_AHEAD", "3"),
-                                       ("SVA_SGM_NO_BLK", "0")])
+@pytest.mark.parametrize("var,value", [("SVA_BOX_OCC", "1"), ("SVA_SGM_PACE_WINDOW", "0"), ("SVA_SGM_HSTORE", "0"), ("SVA_SGM_HSTORE", "3"),
+                                       ("SVA_SGM_HSTORE", "4"), ("SVA_SGM_PACE", "2"), ("SVA_WTA_SEG", "-2"), ("SVA_AD_TH", "-8"),
+                                       ("SVA_BOX_BANDS", "2x"), ("SVA_AD_SET", ""), ("SVA_STREAM_AD_AHEAD", "3")])
 def test_bad_switch_value_is_refused(monkeypatch, var, value):
     """a value outside the documented set fails sva_create, naming the variable, instead of running some other schedule (SVA_BOX_OCC=1
     used to leave K1b without a launch shape: no cost volume written, and the stale one used).  No kernel runs here."""
